@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: batched IK solves/s of the B200 engine (FABRIK + ANN) beside the CPU restatement.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Under torchrun (N > 1) every rank solves its own contiguous shard of the trajectory (weak scaling:
 `--rows` FABRIK targets per GPU); rank 0 prints ONE JSON line.  A "step" is one pass of the hot path
@@ -35,7 +35,9 @@ INTERIOR_BOX = ((2.0, 4.0, 3.0), (1.0, -2.0, 1.0))      # SURVEY 8d cfg 3 (R)
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline FABRIK loop (`value`); the secondary legs time "
+                         "between 2 and 5 steps, or half of this")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--rows", type=int, default=100_000_000, help="FABRIK targets per GPU (config 3)")
@@ -45,7 +47,24 @@ def parse_args():
                     help="ANN targets per GPU for the config-4 leg (1e9 over 8 GPUs); 0 skips it")
     ap.add_argument("--skip-ann", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0; a fixed, seeded sample "
+                         f"of at most {DUMP_ROWS} rows per array) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ROWS = 1_500_000   # 24 MB of float32 [*, 4] angles per dumped array, 48 MB for both
+
+
+def dump_rows(n):
+    """The rows of an n-row output that --dump-outputs writes: all of them up to DUMP_ROWS, else the same seeded sample
+    in every run, in ascending order."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
 
 
 # ---- clocks -----------------------------------------------------------------------------------------
@@ -252,6 +271,13 @@ def main():
         w1 = time.perf_counter()
         return max_over_ranks(e0.elapsed_time(e1) * 1e-3), w0, w1
 
+    def dump(name, t):
+        """--dump-outputs: the dump_rows sample of rank 0's device output t, as DIR/<name>.npy"""
+        if args.dump_outputs and rank == 0:
+            rows = torch.from_numpy(dump_rows(t.shape[0])).to(t.device)
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.index_select(0, rows).cpu().numpy())
+
     PARITY_ROWS = 100_000
 
     def reduce_parity(block):
@@ -323,6 +349,7 @@ def main():
     one = eng.stats_fetch_torch()                               # per-launch iteration count (deterministic)
     launches0 = eng.launch_count
     secs, w0, w1 = timed_device_loop(lambda: eng.fabrik_solve_device(xyz, angles), args.steps, args.warmup)
+    dump("fabrik_angles", angles)   # before the legs below overwrite `angles`
     gpu_launches = (eng.launch_count - launches0 - args.warmup) * world
     value = n * world * args.steps / secs
     total = reduce_stats(one)
@@ -553,6 +580,8 @@ def main():
             a_secs, _, _ = timed_device_loop(lambda: aeng.ann_solve_device(axyz, aout, mode=mode), a_steps, 3)
             gpu_launches += (aeng.launch_count - a_launch0 - 3) * world
             modes[mode] = a_secs / a_steps
+            if mode == "fp16x3_ts":     # the default mode, the one `ann.value` reports
+                dump("ann_angles", aout)
         # parity of the default mode's launch on the bench's own rows: NumPy fp32 / fp64 restatements of ann.py:70-76
         # and an independent torch-CPU fp32 evaluation (oracle/torch_oracle.py); FK error with the oracle's FK
         aeng.ann_solve_device(axyz, aout, mode="fp16x3_ts")

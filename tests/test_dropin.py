@@ -3,9 +3,10 @@
 CPU: with dropin/ ahead of the reference tree every `kinematics.*` / `robot.*` import of cli.py, rpc_broker.py and
 the reference's tests resolves to the shims while the reference's own `tests`, `plot`, `cli`, `rpc_broker` stay its
 own, and `cli.CLI()` constructs.  GPU: the reference's unit suites, cli.py and the broker callback run unmodified
-(tools/run_reference_suite.py).  Both need a checkout of the reference (IK_REFERENCE_ROOT, /root/reference, or
-an untracked .refscratch/ copy placed there for one run on the GPU box, which has no /root/reference: that run's log is
-profiles/r02_dropin_suite.log); without one the tests skip."""
+(tools/run_reference_suite.py).  Both run the reference's own code, which is not part of this repository, so they need
+a checkout of it (IK_REFERENCE_ROOT, or a .refscratch/ copy in the repository root) and skip without one; the log of
+one such run is profiles/r02_dropin_suite.log.  test_plain_pythonpath_is_not_enough needs only the reference's package
+layout and builds a stand-in tree for it."""
 import os
 import subprocess
 import sys
@@ -38,12 +39,14 @@ def test_reference_imports_resolve_to_the_dropin():
     assert "ok  kinematics.inverse" in out and "ok  cli" in out and "LAUNCH" in out
 
 
-def test_plain_pythonpath_is_not_enough():
+def test_plain_pythonpath_is_not_enough(tmp_path):
     """Why INTEGRATION.md prescribes the launcher (or PYTHONSAFEPATH): `python cli.py` puts the script directory at
-    sys.path[0], ahead of PYTHONPATH, so the reference's own packages would win."""
-    ref = _reference_root()
-    if ref is None:
-        pytest.skip("no checkout of the reference available")
+    sys.path[0], ahead of PYTHONPATH, so the reference's own packages would win.  Only the reference's package layout
+    matters here, so a stand-in tree with its `kinematics` package and a `cli.py` takes its place."""
+    ref = str(tmp_path)
+    os.makedirs(os.path.join(ref, "kinematics"))
+    for name in ("cli.py", os.path.join("kinematics", "__init__.py"), os.path.join("kinematics", "point.py")):
+        open(os.path.join(ref, name), "w").close()
     env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "dropin"), PYTHONDONTWRITEBYTECODE="1")
     env.pop("PYTHONSAFEPATH", None)
     probe = "import sys; sys.path.insert(0, sys.argv[1]); import kinematics.point as m; print(m.__file__)"

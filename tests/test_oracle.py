@@ -141,7 +141,16 @@ def test_shipped_scalers_match_constants():
     np.testing.assert_array_equal(sx.scale_, np_oracle.SHIPPED_SCALE_X)
     np.testing.assert_array_equal(sy.mean_, np_oracle.SHIPPED_MEAN_Y)
     np.testing.assert_array_equal(sy.scale_, np_oracle.SHIPPED_SCALE_Y)
-    # and the oracle's scaler arithmetic equals sklearn's on both sides
+
+
+def test_oracle_scaler_arithmetic_matches_sklearn():
+    """The oracle's scaler arithmetic equals sklearn's StandardScaler on both sides, with the shipped scalers' values."""
+    pytest.importorskip("sklearn")
+    from sklearn.preprocessing import StandardScaler
+    sx, sy = StandardScaler(), StandardScaler()
+    sx.mean_, sx.scale_ = np_oracle.SHIPPED_MEAN_X.copy(), np_oracle.SHIPPED_SCALE_X.copy()
+    sy.mean_, sy.scale_ = np_oracle.SHIPPED_MEAN_Y.copy(), np_oracle.SHIPPED_SCALE_Y.copy()
+    sx.n_features_in_, sy.n_features_in_ = 3, 4
     x = np.random.default_rng(1).uniform(-3, 6, size=(50, 3))
     np.testing.assert_array_equal(sx.transform(x), (x - sx.mean_) / sx.scale_)
     y = np.random.default_rng(2).normal(size=(50, 4)).astype(np.float32)
