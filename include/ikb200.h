@@ -127,9 +127,23 @@ int ikb_fabrik_solve_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t
                           int precision, ikb_stats *stats);
 
 /* ---- Fabrik.calculate with explicit initial chains (fabrik.py:44-67) -------------------------
- * init: n_init x 4 x 3 doubles (n_init == 1 broadcasts one chain to all goals, or n_init == n);
- * goals: n x 3 doubles; chain_out: n x 4 x 3 doubles.  3-D, IEEE fp64 with the reference's
- * operation order (sqrt and division correctly rounded, no FMA contraction).  HOST pointers.   */
+ * A chain of n_points = J points (1 <= J <= IKB_CHAIN_MAX_POINTS, else IKB_ERR_UNSUPPORTED) with one link length per
+ * point (links: J doubles in HOST memory; the backward pass uses links[J-2..0], the forward pass links[1..J-1]).
+ * init: n_init x J x 3 doubles (n_init == 1 broadcasts one chain to all goals, or n_init == n);
+ * goals: n x 3 doubles; chain_out: n x J x 3 doubles; iters_out: n passes per row.  3-D, IEEE fp64 with the
+ * reference's operation order (sqrt and division correctly rounded, no FMA contraction): the result of a row does not
+ * depend on the batch it is in.  tol and max_iter are the reference's err_margin and max_iter_num: tol >= 1 or
+ * max_iter <= 0 returns the initial chains.  A zero-length segment leaves a non-finite chain and sets
+ * stats.first_zero_division (ZeroDivisionError upstream).  Row counts are 64-bit, without a per-call limit.
+ * _device: DEVICE pointers, enqueued on `stream`; _host: HOST pointers, staged through the engine's pipeline. */
+#define IKB_CHAIN_MAX_POINTS 256
+int ikb_fabrik_chain_device(ikb_engine *e, int32_t n_points, const double *links, double tol, int32_t max_iter,
+                            const double *init, int64_t n_init, const double *goals, int64_t n, double *chain_out,
+                            int32_t *iters_out /* nullable */, void *stream);
+int ikb_fabrik_chain_host(ikb_engine *e, int32_t n_points, const double *links, double tol, int32_t max_iter,
+                          const double *init, int64_t n_init, const double *goals, int64_t n, double *chain_out,
+                          int32_t *iters_out /* nullable */, ikb_stats *stats);
+/* the 4-point chain with the engine's own links, tol and max_iter (ikb_config) */
 int ikb_fabrik_calculate_host(ikb_engine *e, const double *init, int64_t n_init,
                               const double *goals, int64_t n, double *chain_out,
                               int32_t *iters_out /* nullable */, ikb_stats *stats);

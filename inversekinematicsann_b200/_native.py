@@ -14,6 +14,7 @@ IKB_ERR_INVALID, IKB_ERR_CUDA, IKB_ERR_NO_MODEL, IKB_ERR_UNSUPPORTED = -1, -2, -
 IKB_F32, IKB_F64 = 0, 1
 IKB_FABRIK_F64, IKB_FABRIK_F32 = 0, 1
 IKB_MLP_FP32_SIMT, IKB_MLP_FP16X3_TC, IKB_MLP_FP16X3_TS = 0, 1, 2
+IKB_CHAIN_MAX_POINTS = 256
 
 # every symbol include/ikb200.h declares (tests check that the built library exports them all)
 EXPORTED_SYMBOLS = [
@@ -21,6 +22,7 @@ EXPORTED_SYMBOLS = [
     "ikb_stats_reset", "ikb_stats_fetch",
     "ikb_check_limits_device", "ikb_check_limits_host",
     "ikb_fabrik_solve_device", "ikb_fabrik_solve_host", "ikb_fabrik_calculate_host",
+    "ikb_fabrik_chain_device", "ikb_fabrik_chain_host",
     "ikb_fk_device", "ikb_fk_host", "ikb_fk_chain_host",
     "ikb_mlp_load", "ikb_ann_solve_device", "ikb_ann_solve_host",
     "ikb_generate_device", "ikb_microbench_fma", "ikb_launch_count",
@@ -79,6 +81,10 @@ def load():
         "ikb_fabrik_solve_device": (i32, [engine, vp, i32, i64, vp, i32, vp, vp, i32, i32, vp]),
         "ikb_fabrik_solve_host": (i32, [engine, vp, i32, i64, vp, i32, vp, vp, i32, i32, stats_p]),
         "ikb_fabrik_calculate_host": (i32, [engine, vp, i64, vp, i64, vp, vp, stats_p]),
+        "ikb_fabrik_chain_device": (i32, [engine, ctypes.c_int32, vp, dbl, ctypes.c_int32, vp, i64, vp, i64, vp, vp,
+                                          vp]),
+        "ikb_fabrik_chain_host": (i32, [engine, ctypes.c_int32, vp, dbl, ctypes.c_int32, vp, i64, vp, i64, vp, vp,
+                                        stats_p]),
         "ikb_fk_device": (i32, [engine, vp, i32, i64, vp, vp, i32, vp, vp]),
         "ikb_fk_host": (i32, [engine, vp, i32, i64, vp, vp, i32, vp, stats_p]),
         "ikb_fk_chain_host": (i32, [engine, vp, vp, ctypes.POINTER(i32)]),

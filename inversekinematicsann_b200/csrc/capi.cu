@@ -3,6 +3,7 @@
 // needs a CUDA device.
 #include <cmath>
 #include <cstdio>
+#include <algorithm>
 #include <cstring>
 #include <new>
 #include <string>
@@ -16,9 +17,10 @@ cudaError_t ikb_launch_fabrik_planar(const void *xyz, int xyz_f64, long long n, 
                                      void *angles, int angles_f64, int *iters, void *fk_err, int fk_stats,
                                      int precision, IkbDeviceStats *stats, unsigned long long *work_counter,
                                      const IkbRobot &rc, int num_sms, cudaStream_t stream);
-cudaError_t ikb_launch_fabrik_generic(const double *init, long long n_init, const double *goals,
-                                      long long n, double *chain_out, int *iters,
-                                      IkbDeviceStats *stats, const IkbRobot &rc, cudaStream_t stream);
+cudaError_t ikb_launch_fabrik_chain(int n_points, const double *links, double tol, int max_iter, const double *init,
+                                    long long n_init, const double *goals, long long n, long long index_base,
+                                    double *chain_out, int *iters, IkbDeviceStats *stats,
+                                    unsigned long long *work_counter, int num_sms, cudaStream_t stream);
 cudaError_t ikb_launch_fabrik_generic_ikine(const void *xyz, int xyz_f64, long long n, long long index_base,
                                             void *angles, int angles_f64, int *iters, IkbDeviceStats *stats,
                                             const IkbRobot &rc, cudaStream_t stream);
@@ -485,33 +487,82 @@ int ikb_fabrik_solve_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t
     return host_end(e, stats);
 }
 
+// ---- Fabrik.calculate on J-point chains (fabrik.py:44-67) ----------------------------------------
+static int chain_args_error(ikb_engine *e, const char *what, int32_t n_points, const double *links, const double *init,
+                            int64_t n_init, const double *goals, int64_t n, const double *chain_out)
+{
+    if (!e)
+        return IKB_ERR_INVALID;
+    if (n_points < 1 || n_points > IKB_CHAIN_MAX_POINTS)
+        return fail(e, IKB_ERR_UNSUPPORTED, std::string(what) + ": n_points must be 1.." +
+                                                std::to_string(IKB_CHAIN_MAX_POINTS) + ", got " + std::to_string(n_points));
+    if (!links || n < 0 || (n_init != 1 && n_init != n) || (n > 0 && (!init || !goals || !chain_out)))
+        return fail(e, IKB_ERR_INVALID, std::string(what) + ": bad argument (n_init must be 1 or n)");
+    return IKB_OK;
+}
+
+int ikb_fabrik_chain_device(ikb_engine *e, int32_t n_points, const double *links, double tol, int32_t max_iter,
+                            const double *init, int64_t n_init, const double *goals, int64_t n, double *chain_out,
+                            int32_t *iters_out, void *stream)
+{
+    int rc = chain_args_error(e, "ikb_fabrik_chain_device", n_points, links, init, n_init, goals, n, chain_out);
+    if (rc)
+        return rc;
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    IKB_CUDA(e, ikb_launch_fabrik_chain(n_points, links, tol, max_iter, init, n_init, goals, n, 0, chain_out, iters_out,
+                                        e->d_stats, next_counter(e), e->num_sms, (cudaStream_t)stream));
+    e->launches += (n > 0);
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline: goals in d_in2 (3 doubles per slot row), chains in d_out and per-row initial chains in
+// d_in (4 doubles per slot row each), iterations in d_aux.  A single initial chain (n_init == 1) is copied to d_in of
+// every slot once.
+int ikb_fabrik_chain_host(ikb_engine *e, int32_t n_points, const double *links, double tol, int32_t max_iter,
+                          const double *init, int64_t n_init, const double *goals, int64_t n, double *chain_out,
+                          int32_t *iters_out, ikb_stats *stats)
+{
+    int rc = chain_args_error(e, "ikb_fabrik_chain_host", n_points, links, init, n_init, goals, n, chain_out);
+    if (rc)
+        return rc;
+    const long long row_doubles = 3LL * n_points;
+    rc = host_begin(e, std::max<long long>(n, (n * row_doubles + 3) / 4));
+    if (rc)
+        return rc;
+    const long long m_max = std::max(1LL, std::min(e->slot_rows, 4 * e->slot_rows / row_doubles));
+    const bool per_row_init = n_init != 1;
+    if (n > 0 && !per_row_init)
+        for (int i = 0; i < kSlots; ++i)
+            IKB_CUDA(e, cudaMemcpyAsync(e->slots[i].d_in, init, row_doubles * sizeof(double), cudaMemcpyHostToDevice,
+                                        e->slots[i].stream));
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        double *d_init = (double *)s.d_in, *d_goals = (double *)s.d_in2, *d_chain = (double *)s.d_out;
+        if (per_row_init)
+            IKB_CUDA(e, cudaMemcpyAsync(d_init, init + lo * row_doubles, m * row_doubles * sizeof(double),
+                                        cudaMemcpyHostToDevice, s.stream));
+        IKB_CUDA(e, cudaMemcpyAsync(d_goals, goals + 3 * lo, m * 3 * sizeof(double), cudaMemcpyHostToDevice, s.stream));
+        IKB_CUDA(e, ikb_launch_fabrik_chain(n_points, links, tol, max_iter, d_init, per_row_init ? m : 1, d_goals, m, lo,
+                                            d_chain, iters_out ? s.d_aux : nullptr, e->d_stats, next_counter(e),
+                                            e->num_sms, s.stream));
+        e->launches++;
+        IKB_CUDA(e, cudaMemcpyAsync(chain_out + lo * row_doubles, d_chain, m * row_doubles * sizeof(double),
+                                    cudaMemcpyDeviceToHost, s.stream));
+        if (iters_out)
+            IKB_CUDA(e, cudaMemcpyAsync(iters_out + lo, s.d_aux, m * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+    }
+    return host_end(e, stats);
+}
+
 int ikb_fabrik_calculate_host(ikb_engine *e, const double *init, int64_t n_init, const double *goals,
                               int64_t n, double *chain_out, int32_t *iters_out, ikb_stats *stats)
 {
-    if (!e || n < 0 || (n > 0 && (!init || !goals || !chain_out)) || (n_init != 1 && n_init != n))
-        return fail(e, IKB_ERR_INVALID, "ikb_fabrik_calculate_host: bad argument (n_init must be 1 or n)");
-    int rc = host_begin(e, n);
-    if (rc)
-        return rc;
-    if (n > 0) {
-        double *d_init = nullptr, *d_goals = nullptr, *d_chain = nullptr;
-        int *d_it = nullptr;
-        cudaStream_t st = e->slots[0].stream;
-        IKB_CUDA(e, cudaMalloc(&d_init, n_init * 12 * sizeof(double)));
-        IKB_CUDA(e, cudaMalloc(&d_goals, n * 3 * sizeof(double)));
-        IKB_CUDA(e, cudaMalloc(&d_chain, n * 12 * sizeof(double)));
-        IKB_CUDA(e, cudaMalloc(&d_it, n * sizeof(int)));
-        IKB_CUDA(e, cudaMemcpyAsync(d_init, init, n_init * 12 * sizeof(double), cudaMemcpyHostToDevice, st));
-        IKB_CUDA(e, cudaMemcpyAsync(d_goals, goals, n * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-        IKB_CUDA(e, ikb_launch_fabrik_generic(d_init, n_init, d_goals, n, d_chain, d_it, e->d_stats, e->rc, st));
-        e->launches++;
-        IKB_CUDA(e, cudaMemcpyAsync(chain_out, d_chain, n * 12 * sizeof(double), cudaMemcpyDeviceToHost, st));
-        if (iters_out)
-            IKB_CUDA(e, cudaMemcpyAsync(iters_out, d_it, n * sizeof(int), cudaMemcpyDeviceToHost, st));
-        IKB_CUDA(e, cudaStreamSynchronize(st));
-        cudaFree(d_init); cudaFree(d_goals); cudaFree(d_chain); cudaFree(d_it);
-    }
-    return host_end(e, stats);
+    if (!e)
+        return IKB_ERR_INVALID;
+    return ikb_fabrik_chain_host(e, 4, e->rc.links, e->cfg.tol, e->cfg.max_iter, init, n_init, goals, n, chain_out,
+                                 iters_out, stats);
 }
 
 // ---- forward kinematics ---------------------------------------------------------------------------

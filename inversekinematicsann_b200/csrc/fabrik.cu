@@ -25,6 +25,7 @@
 #include <cstdlib>
 
 #include "fk_device.cuh"
+#include "vec3.cuh"
 
 // -DIKB_FABRIK_CHECK: trap when a shared-memory queue would be indexed outside its capacity (the pool's
 // compute-sanitizer is closed, so the debug variant of tools/build_variant.sh carries its own bounds checks)
@@ -808,84 +809,6 @@ __global__ void __launch_bounds__(IKB_FABRIK_WARPS * 32, IKB_FABRIK_MIN_CTAS) fa
     fabrik_warp_loop<Real, FUSE_FK, OUT32, ZERO_ITER>(a, reinterpret_cast<WarpQueues<Real, typename TailType<OUT32>::type> *>(s_raw));
 }
 
-// ---- generic 3-D path ---------------------------------------------------------------------------
-// IEEE fp64 with the reference's operation order (point.py:25-45): correctly rounded sqrt and
-// division, explicit _rn intrinsics so nothing is contracted into FMAs.  One chain per thread.
-struct Vec3 {
-    double x, y, z;
-};
-
-__device__ __forceinline__ double dist3(const Vec3 &a, const Vec3 &b)
-{
-    const double dx = __dsub_rn(a.x, b.x), dy = __dsub_rn(a.y, b.y), dz = __dsub_rn(a.z, b.z);
-    return __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
-}
-
-// get_point_between(s, e, L) = s + (L / |s - e|) * (e - s); NaN when the distance is 0
-__device__ __forceinline__ Vec3 point_between3(const Vec3 &s, const Vec3 &e, double L)
-{
-    const double t = __ddiv_rn(L, dist3(s, e));
-    Vec3 o;
-    o.x = __dadd_rn(s.x, __dmul_rn(t, __dsub_rn(e.x, s.x)));
-    o.y = __dadd_rn(s.y, __dmul_rn(t, __dsub_rn(e.y, s.y)));
-    o.z = __dadd_rn(s.z, __dmul_rn(t, __dsub_rn(e.z, s.z)));
-    return o;
-}
-
-struct FabrikGenericArgs {
-    const double *init;  // n_init x 4 x 3
-    long long n_init;
-    const double *goals;  // n x 3
-    long long n;
-    double *chain_out;  // n x 4 x 3
-    int *iters;         // nullable
-    IkbDeviceStats *stats;
-    IkbRobot rc;
-};
-
-__global__ void __launch_bounds__(128) fabrik_generic_kernel(const FabrikGenericArgs a)
-{
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.n)
-        return;
-    const double *ip = a.init + (a.n_init == 1 ? 0 : 12 * i);
-    Vec3 P[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-        P[j] = Vec3{ip[3 * j], ip[3 * j + 1], ip[3 * j + 2]};
-    const Vec3 S = P[0];
-    const Vec3 T{a.goals[3 * i], a.goals[3 * i + 1], a.goals[3 * i + 2]};
-    const double *d = a.rc.links;
-    const double tol = a.rc.tol;
-    double se = 1.0, ge = 1.0;
-    int step = 0;
-    while ((se > tol || ge > tol) && a.rc.max_iter > step) {  // fabrik.py:57-59
-        const Vec3 b2 = point_between3(T, P[2], d[2]);
-        const Vec3 b1 = point_between3(b2, P[1], d[1]);
-        const Vec3 b0 = point_between3(b1, P[0], d[0]);
-        se = dist3(b0, S);
-        P[0] = S;
-        P[1] = point_between3(P[0], b1, d[1]);
-        P[2] = point_between3(P[1], b2, d[2]);
-        P[3] = point_between3(P[2], T, d[3]);
-        ge = dist3(P[3], T);
-        ++step;
-    }
-    bool nan_out = false;
-    double *o = a.chain_out + 12 * i;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        o[3 * j] = P[j].x; o[3 * j + 1] = P[j].y; o[3 * j + 2] = P[j].z;
-        nan_out |= !(isfinite(P[j].x) & isfinite(P[j].y) & isfinite(P[j].z));
-    }
-    if (a.iters)
-        a.iters[i] = step;
-    if (nan_out && isfinite(T.x) && isfinite(T.y) && isfinite(T.z))
-        atomicMin(&a.stats->first_zero_division, i);
-    atomicAdd(&a.stats->sum_iterations, (unsigned long long)step);
-    atomicAdd(&a.stats->n_solved, 1ULL);
-}
-
 // ---- generic ikine: robots whose seed chain leaves the vertical plane (general DH tables) ----------------------
 // One target per thread, IEEE fp64 in 3-D with the reference's operation order: seed chain = the theta_1 = 0
 // chain rotated about z by atan2(y, x) (inverse.py:123-130), Fabrik.calculate (fabrik.py:44-67), __get_angles
@@ -1073,19 +996,5 @@ cudaError_t ikb_launch_fabrik_generic_ikine(const void *xyz, int xyz_f64, long l
     a.xyz = xyz; a.xyz_f64 = xyz_f64; a.n = n; a.index_base = index_base; a.angles = angles;
     a.angles_f64 = angles_f64; a.iters = iters; a.stats = stats; a.rc = rc;
     fabrik_generic_ikine_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(a);
-    return cudaGetLastError();
-}
-
-cudaError_t ikb_launch_fabrik_generic(const double *init, long long n_init, const double *goals,
-                                      long long n, double *chain_out, int *iters,
-                                      IkbDeviceStats *stats, const IkbRobot &rc, cudaStream_t stream)
-{
-    if (n <= 0)
-        return cudaSuccess;
-    FabrikGenericArgs a;
-    a.init = init; a.n_init = n_init; a.goals = goals; a.n = n; a.chain_out = chain_out;
-    a.iters = iters; a.stats = stats; a.rc = rc;
-    const unsigned grid = (unsigned)((n + 127) / 128);
-    fabrik_generic_kernel<<<grid, 128, 0, stream>>>(a);
     return cudaGetLastError();
 }

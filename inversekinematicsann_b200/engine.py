@@ -195,8 +195,38 @@ class IkEngine:
             res += (fk_err,)
         return res
 
+    @staticmethod
+    def _chain_links(links):
+        links = np.ascontiguousarray(links, dtype=np.float64)
+        if links.ndim != 1 or not 1 <= links.shape[0] <= _native.IKB_CHAIN_MAX_POINTS:
+            raise ValueError(f"a chain needs 1..{_native.IKB_CHAIN_MAX_POINTS} link lengths, got shape {links.shape}")
+        return links
+
+    def fabrik_chain(self, links, tol, max_iter, init, goals):
+        """reference fabrik.py:44-67 on J-point chains: J = len(links) link lengths, init (J,3) or (n,J,3), goals (n,3).
+        Returns (chains[n,J,3], iters[n], stats); stats.first_zero_division >= 0 marks a zero-length segment."""
+        links = self._chain_links(links)
+        J = links.shape[0]
+        init = np.ascontiguousarray(init, dtype=np.float64)
+        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(-1, 3)
+        n = goals.shape[0]
+        if init.shape == (J, 3):
+            n_init = 1
+        elif init.shape == (n, J, 3):
+            n_init = n
+        else:
+            raise ValueError(f"initial chains must have shape ({J}, 3) or ({n}, {J}, 3), got {init.shape}")
+        chain = np.empty((n, J, 3), dtype=np.float64)
+        iters = np.empty(n, dtype=np.int32)
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_fabrik_chain_host(self._handle, J, links.ctypes.data, float(tol), int(max_iter),
+                                                    init.ctypes.data, n_init, goals.ctypes.data, n, chain.ctypes.data,
+                                                    iters.ctypes.data, ctypes.byref(s)), "ikb_fabrik_chain_host")
+        return chain, iters, IkStats.from_c(s)
+
     def fabrik_calculate(self, init, goals):
-        """reference fabrik.py:44-67 for explicit initial chains.  init: (4,3) or (n,4,3); goals (n,3)."""
+        """reference fabrik.py:44-67 for explicit 4-point chains with the engine's links, tolerance and iteration cap.
+        init: (4,3) or (n,4,3); goals (n,3)."""
         init = np.ascontiguousarray(init, dtype=np.float64)
         goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(-1, 3)
         n = goals.shape[0]
@@ -352,6 +382,31 @@ class IkEngine:
             _torch_dtype_code(out), iters.data_ptr() if iters is not None else None,
             fk_err.data_ptr() if fk_err is not None else None, int(bool(fk_stats)), prec,
             _torch_stream_ptr(self.device)), "ikb_fabrik_solve_device")
+
+    def fabrik_chain_device(self, links, tol, max_iter, init, goals, out, iters=None):
+        """fabrik_chain on float64 CUDA tensors of this engine's device, enqueued on torch's current stream (no
+        synchronisation): init (J,3) or (n,J,3), goals (n,3), out (n,J,3), iters int32 (n,) or None.  Statistics
+        accumulate in the engine's block (stats_fetch_torch)."""
+        links = self._chain_links(links)
+        J = links.shape[0]
+        goals = self._dev_rows(goals, 3, "goals")
+        n = goals.shape[0]
+        for t, what in ((init, "init"), (goals, "goals"), (out, "out")):
+            self._dev_vec(t, t.numel() if _is_torch_tensor(t) else -1, "torch.float64", what)
+        if tuple(init.shape) == (J, 3):
+            n_init = 1
+        elif tuple(init.shape) == (n, J, 3):
+            n_init = n
+        else:
+            raise ValueError(f"init must have shape ({J}, 3) or ({n}, {J}, 3), got {tuple(init.shape)}")
+        if tuple(out.shape) != (n, J, 3):
+            raise ValueError(f"out must have shape ({n}, {J}, 3), got {tuple(out.shape)}")
+        if iters is not None:
+            self._dev_vec(iters, n, "torch.int32", "iters")
+        self._check(self._lib.ikb_fabrik_chain_device(
+            self._handle, J, links.ctypes.data, float(tol), int(max_iter), init.data_ptr(), n_init, goals.data_ptr(), n,
+            out.data_ptr(), iters.data_ptr() if iters is not None else None, _torch_stream_ptr(self.device)),
+            "ikb_fabrik_chain_device")
 
     def ann_solve_device(self, xyz, out, mode="fp32", fk_err=None, fk_stats=False):
         mode_code = _choice(_MLP_MODES, mode, "mode")
