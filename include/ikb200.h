@@ -159,8 +159,28 @@ int ikb_fk_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n
 int ikb_fk_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n,
                 void *pos_out, const void *targets, int xyz_dtype, void *err_out, ikb_stats *stats);
 /* all four cumulative 4x4 matrices of ONE angle set (the (T, [T1..T4]) return of fkine):
- * chain_out = 4 x 16 doubles, row-major.  Host pointers. */
+ * chain_out = 4 x 16 doubles, row-major.  Host pointers.  *status = 1 when an angle (or alpha) is outside
+ * [-2pi, 2pi] (forward.py:23-25; the matrices are still written), else 0.  This is ikb_fk_transforms_host at n = 1. */
 int ikb_fk_chain_host(ikb_engine *e, const double angles[4], double chain_out[64], int *status);
+/* The cumulative DH matrices T_1..T_4 of n angle sets (fkine's (T, [T1..T4]) for a batch).  angles: n x 4 of
+ * angles_dtype; the arithmetic is fp64 (float32 angles are widened exactly) and is the same as ikb_fk_chain_host's, so
+ * a row's bits do not depend on the batch it is in.  `out` has the angles' dtype (a float32 output is the fp64 result
+ * rounded once) and, by `what`:
+ *   IKB_FK_MATRICES  n x 4 x 4 x 4, row-major T_1..T_4 (the layout of chain_out above): 512 B per row in fp64
+ *   IKB_FK_JOINTS    n x 4 x 3, column 3 of T_1..T_4 -- the joint origins (inverse.py:128-130), which is the `init`
+ *                    layout of ikb_fabrik_chain_* for fp64
+ * Rows with an angle (or alpha) outside [-2pi, 2pi] are still written; the lowest such row goes to
+ * stats.first_fk_angle_range (NaN passes; float32 angles are tested after widening, so float32(2pi), which is
+ * above 2pi, is outside).  `angles` and `out` must be aligned to their element size; an `out` that
+ * is not 16-byte aligned is written with element stores instead of bulk copies.
+ * _device: DEVICE pointers, enqueued on `stream`, the guard accumulates in the statistics block; _host: HOST pointers,
+ * staged through the engine's pipeline, `stats` filled (nullable). */
+#define IKB_FK_MATRICES 0
+#define IKB_FK_JOINTS 1
+int ikb_fk_transforms_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n,
+                             int what, void *out, void *stream);
+int ikb_fk_transforms_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n,
+                           int what, void *out, ikb_stats *stats);
 
 /* ---- ANN (ann.py:70-85, inverse.py:142-155) -------------------------------------------------- */
 /* replaces ANN.load_model (ann.py:78-85): upload the Keras Sequential's Dense kernels/biases and the

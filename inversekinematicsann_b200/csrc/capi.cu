@@ -27,8 +27,9 @@ cudaError_t ikb_launch_fabrik_generic_ikine(const void *xyz, int xyz_f64, long l
 cudaError_t ikb_launch_fk(const void *angles, int angles_f64, long long n, long long index_base,
                           void *pos_out, const void *targets, int xyz_f64, void *err_out,
                           IkbDeviceStats *stats, const IkbRobot &rc, int num_sms, cudaStream_t stream);
-cudaError_t ikb_launch_fk_chain(const double *angles, long long n, double *chain_out, int *status,
-                                const IkbRobot &rc, cudaStream_t stream);
+cudaError_t ikb_launch_fk_transforms(const void *angles, int angles_f64, long long n, long long index_base, int what,
+                                     void *out, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                     cudaStream_t stream);
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,
                                     IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                     cudaStream_t stream);
@@ -284,18 +285,20 @@ int ikb_engine_create(const ikb_config *cfg, ikb_engine **out)
     {
         double seed[4] = {0.0, cfg->dh[1], cfg->dh[2], cfg->dh[3]};
         double chain[64];
-        int status = 0;
         double *d_ang = nullptr, *d_chain = nullptr;
-        int *d_st = nullptr;
         IKB_CREATE_CUDA(cudaMalloc(&d_ang, sizeof seed));
         IKB_CREATE_CUDA(cudaMalloc(&d_chain, sizeof chain));
-        IKB_CREATE_CUDA(cudaMalloc(&d_st, sizeof(int)));
         IKB_CREATE_CUDA(cudaMemcpy(d_ang, seed, sizeof seed, cudaMemcpyHostToDevice));
-        IKB_CREATE_CUDA(ikb_launch_fk_chain(d_ang, 1, d_chain, d_st, rc, nullptr));
+        IKB_CREATE_CUDA(ikb_launch_fk_transforms(d_ang, 1, 1, 0, IKB_FK_MATRICES, d_chain, e->d_stats, rc, e->num_sms,
+                                                 nullptr));
         e->launches++;
         IKB_CREATE_CUDA(cudaMemcpy(chain, d_chain, sizeof chain, cudaMemcpyDeviceToHost));
-        IKB_CREATE_CUDA(cudaMemcpy(&status, d_st, sizeof(int), cudaMemcpyDeviceToHost));
-        cudaFree(d_ang); cudaFree(d_chain); cudaFree(d_st);
+        IKB_CREATE_CUDA(cudaMemcpy(e->h_stats, e->d_stats, sizeof(IkbDeviceStats), cudaMemcpyDeviceToHost));
+        const bool status = e->h_stats->first_fk_angle_range != IKB_I64_MAX;
+        // the guard of the seed chain is the engine's business, not its callers': start them with a clean block
+        *e->h_stats = fresh_stats();
+        IKB_CREATE_CUDA(cudaMemcpy(e->d_stats, e->h_stats, sizeof(IkbDeviceStats), cudaMemcpyHostToDevice));
+        cudaFree(d_ang); cudaFree(d_chain);
         rc.planar = 1;
         for (int j = 0; j < 4; ++j) {
             const double x = chain[16 * j + 3], y = chain[16 * j + 7], z = chain[16 * j + 11];
@@ -304,7 +307,7 @@ int ikb_engine_create(const ikb_config *cfg, ikb_engine **out)
             if (std::fabs(y) > 1e-9 || !(std::fabs(x) < 1e300))
                 rc.planar = 0;
         }
-        if (status != 0)
+        if (status)
             rc.planar = 0;
         rc.seed_ab = std::sqrt(rc.seed_r[0] * rc.seed_r[0] + rc.seed_z[0] * rc.seed_z[0]);
         rc.seed_ab2 = rc.seed_ab * rc.seed_ab;
@@ -611,21 +614,67 @@ int ikb_fk_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, 
     return host_end(e, stats);
 }
 
+static bool fk_transforms_bad_args(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what,
+                                   const void *out)
+{
+    const uintptr_t align = esize(angles_dtype) - 1;
+    return !e || n < 0 || (n > 0 && (!angles || !out)) || bad_dtype(angles_dtype) ||
+           (what != IKB_FK_MATRICES && what != IKB_FK_JOINTS) || ((uintptr_t)angles & align) || ((uintptr_t)out & align);
+}
+
+static size_t fk_transforms_row_bytes(int angles_dtype, int what)
+{
+    return (what == IKB_FK_JOINTS ? 12 : 64) * esize(angles_dtype);
+}
+
+int ikb_fk_transforms_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what, void *out,
+                             void *stream)
+{
+    if (fk_transforms_bad_args(e, angles, angles_dtype, n, what, out))
+        return fail(e, IKB_ERR_INVALID, "ikb_fk_transforms_device: bad argument");
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    IKB_CUDA(e, ikb_launch_fk_transforms(angles, angles_dtype == IKB_F64, n, 0, what, out, e->d_stats, e->rc,
+                                         e->num_sms, (cudaStream_t)stream));
+    e->launches += (n > 0);
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline: angles in d_in (32 B per slot row holds a row of either dtype), results in d_out, as
+// many rows as its 32 B per slot row hold at the output row size.
+int ikb_fk_transforms_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what, void *out,
+                           ikb_stats *stats)
+{
+    if (fk_transforms_bad_args(e, angles, angles_dtype, n, what, out))
+        return fail(e, IKB_ERR_INVALID, "ikb_fk_transforms_host: bad argument");
+    int rc = host_begin(e, n);
+    if (rc)
+        return rc;
+    const size_t in_row = 4 * esize(angles_dtype), out_row = fk_transforms_row_bytes(angles_dtype, what);
+    const long long m_max = e->slot_rows * 32 / (long long)out_row;
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)angles + lo * in_row, m * in_row, cudaMemcpyHostToDevice,
+                                    s.stream));
+        IKB_CUDA(e, ikb_launch_fk_transforms(s.d_in, angles_dtype == IKB_F64, m, lo, what, s.d_out, e->d_stats, e->rc,
+                                             e->num_sms, s.stream));
+        e->launches++;
+        IKB_CUDA(e, cudaMemcpyAsync((char *)out + lo * out_row, s.d_out, m * out_row, cudaMemcpyDeviceToHost, s.stream));
+    }
+    return host_end(e, stats);
+}
+
 int ikb_fk_chain_host(ikb_engine *e, const double angles[4], double chain_out[64], int *status)
 {
     if (!e || !angles || !chain_out || !status)
         return fail(e, IKB_ERR_INVALID, "ikb_fk_chain_host: NULL argument");
-    int rc = host_begin(e, 64);
+    ikb_stats st;
+    int rc = ikb_fk_transforms_host(e, angles, IKB_F64, 1, IKB_FK_MATRICES, chain_out, &st);
     if (rc)
         return rc;
-    Slot &s = e->slots[0];
-    double *d_ang = (double *)s.d_in, *d_chain = (double *)s.d_out;
-    IKB_CUDA(e, cudaMemcpyAsync(d_ang, angles, 4 * sizeof(double), cudaMemcpyHostToDevice, s.stream));
-    IKB_CUDA(e, ikb_launch_fk_chain(d_ang, 1, d_chain, s.d_aux, e->rc, s.stream));
-    e->launches++;
-    IKB_CUDA(e, cudaMemcpyAsync(chain_out, d_chain, 64 * sizeof(double), cudaMemcpyDeviceToHost, s.stream));
-    IKB_CUDA(e, cudaMemcpyAsync(status, s.d_aux, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-    return host_end(e, nullptr);
+    *status = st.first_fk_angle_range >= 0 ? 1 : 0;
+    return IKB_OK;
 }
 
 // ---- ANN ------------------------------------------------------------------------------------------

@@ -4,8 +4,8 @@
 // K3 replaces reference ForwardKinematics.fkine (forward.py:73-94) for batches:
 //   T = prod_i Rz(theta_i) Tz(eps_i) Tx(a_i) Rx(alpha_i)                      (forward.py:62-70)
 // Only what callers read is produced in the batched form -- the end-effector position T[0:3, 3]
-// (cli.py:60, inverse.py:130, tests/forward_unit.py:30) and ||pos - target||.  The chain kernel
-// returns all four cumulative 4x4 matrices for the (T, [T1..T4]) return value of fkine.
+// (cli.py:60, inverse.py:130, tests/forward_unit.py:30) and ||pos - target||.  fk_transforms_kernel
+// returns all four cumulative 4x4 matrices (or the joint origins) for the (T, [T1..T4]) return value of fkine.
 // HBM-bound: 16 B angles + 12 B target in, 4 B error out per row (fp32 buffers).
 #include <cstdlib>
 
@@ -319,42 +319,132 @@ __global__ void __launch_bounds__(FK_STREAM_WARPS * 32, 4) fk_error_stream_kerne
     }
 }
 
-// all four cumulative homogeneous matrices (forward.py:79-94), fp64, one thread per angle set
-__global__ void fk_chain_kernel(const double *angles, long long n, double *chain_out, int *status,
-                                const IkbRobot rc)
+// ---- all four cumulative DH matrices of a batch (forward.py:79-94) -----------------------------------------------------
+// Row r of T_j = T_{j-1} D_j depends only on row r of T_{j-1} and on D_j, so one angle set is served by four lanes (a
+// quad): lane r computes sincos of joint r, the quad exchanges the four (sin, cos) pairs with shuffles, and lane r
+// carries row r of T_1..T_4.  Every matrix element is the expression the single-pose path has always used (fp64,
+// default contraction: `acc += T * D` in m order), so a row's bits do not depend on the batch it is in.
+//
+// The workload is store-bound (fp64: 32 B of angles in, 512 B of matrices out per angle set).  A CTA computes a tile of
+// FKT_ROWS consecutive angle sets into shared memory -- one contiguous span of the output -- and one thread sends it
+// to global memory with a 1-D bulk copy (cp.async.bulk, the TMA engine) while the CTA computes the next tile into the
+// other buffer.  An output base that is not 16-byte aligned takes coalesced element stores from the same tile instead.
+
+// row r of T_j from row r of T_{j-1} (`t`) and D_j = Rz(theta) Tz(eps) Tx(a) Rx(alpha) of joint j
+__device__ __forceinline__ void fk_dh_step_row(const double (&t)[4], double s, double c, double ca, double sa, double aj,
+                                               double ej, double (&out)[4])
 {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n)
-        return;
+    const double D[16] = {c, -s * ca, s * sa, aj * c,
+                          s, c * ca, -c * sa, aj * s,
+                          0, sa, ca, ej,
+                          0, 0, 0, 1};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        double acc = 0;
+#pragma unroll
+        for (int m = 0; m < 4; ++m)
+            acc += t[m] * D[4 * m + q];
+        out[q] = acc;
+    }
+}
+
+__device__ __forceinline__ unsigned fkt_smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
+
+// shared -> global 1-D bulk copy (SASS: UBLKCP); dst 16-byte aligned, bytes a multiple of 16
+__device__ __forceinline__ void fkt_bulk_store(void *dst, const void *src, unsigned bytes)
+{
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(fkt_smem_u32(src)),
+                 "r"(bytes)
+                 : "memory");
+    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+}
+
+constexpr int FKT_ROWS = 64;              // angle sets per tile
+constexpr int FKT_THREADS = 4 * FKT_ROWS;  // one quad per angle set
+
+// Real: dtype of angles and output.  JOINTS: n x 4 x 3 (column 3 of T_1..T_4) instead of n x 4 x 4 x 4.
+// Dynamic shared memory: two tiles of FKT_ROWS * ROW_ELEMS elements.
+template <typename Real, bool JOINTS>
+__global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *__restrict__ angles, long long n,
+                                                                    long long index_base, Real *out,
+                                                                    IkbDeviceStats *stats, const IkbRobot rc)
+{
+    constexpr int ROW_ELEMS = JOINTS ? 12 : 64;
+    constexpr int TILE_ELEMS = FKT_ROWS * ROW_ELEMS;
+    extern __shared__ __align__(128) unsigned char fkt_smem[];
+    Real *const tiles = reinterpret_cast<Real *>(fkt_smem);
     const double TWO_PI = 6.283185307179586;
-    double T[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    int st = 0;
-    for (int j = 0; j < 4; ++j) {
-        const double t = angles[4 * i + j], al = rc.alpha[j];
-        if (t < -TWO_PI || t > TWO_PI || al < -TWO_PI || al > TWO_PI)
-            st = 1;
+    const int tid = threadIdx.x, r = tid & 3, lrow = tid >> 2;
+    const int odd = lrow & 1;
+    const bool bulk = ((uintptr_t)out & 15) == 0;  // every row size here is a multiple of 16 bytes
+    const bool alpha_bad = rc.alpha[r] < -TWO_PI || rc.alpha[r] > TWO_PI;
+    const long long n_tiles = (n + FKT_ROWS - 1) / FKT_ROWS;
+    int buf = 0;
+    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, buf ^= 1) {
+        const long long row0 = tile * FKT_ROWS;
+        const int rows = (int)(n - row0 < FKT_ROWS ? n - row0 : FKT_ROWS);
+        const bool live = lrow < rows;
+        const double th = live ? (double)__ldg(angles + 4 * (row0 + lrow) + r) : 0.0;  // a warp reads 256 or 128 B
+        // angle guard of forward.py:23-25 (NaN passes): the lowest offending row of the warp, one atomic per warp
+        const unsigned bad = __ballot_sync(IKB_FULL_MASK, live && (th < -TWO_PI || th > TWO_PI || alpha_bad));
+        if (bad && (tid & 31) == __ffs(bad) - 1)
+            atomicMin(&stats->first_fk_angle_range, index_base + row0 + lrow);
         double s, c;
-        sincos(t, &s, &c);
-        const double ca = rc.cos_alpha[j], sa = rc.sin_alpha[j], aj = rc.a[j], ej = rc.eps[j];
-        // D = Rz(t) Tz(e) Tx(a) Rx(alpha)
-        const double D[16] = {c, -s * ca, s * sa, aj * c,
-                              s, c * ca, -c * sa, aj * s,
-                              0, sa, ca, ej,
-                              0, 0, 0, 1};
-        double N[16];
-        for (int r = 0; r < 4; ++r)
-            for (int q = 0; q < 4; ++q) {
-                double acc = 0;
-                for (int m = 0; m < 4; ++m)
-                    acc += T[4 * r + m] * D[4 * m + q];
-                N[4 * r + q] = acc;
+        sincos(th, &s, &c);
+        // the bulk copy that last read this buffer (two tiles ago) must be done reading it
+        if (bulk && tid == 0)
+            asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        __syncthreads();
+        Real *const dst = tiles + buf * TILE_ELEMS + lrow * ROW_ELEMS;
+        double t[4] = {r == 0 ? 1.0 : 0.0, r == 1 ? 1.0 : 0.0, r == 2 ? 1.0 : 0.0, r == 3 ? 1.0 : 0.0};
+        double prev[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double sj = __shfl_sync(IKB_FULL_MASK, s, j, 4), cj = __shfl_sync(IKB_FULL_MASK, c, j, 4);
+            double nr[4];
+            fk_dh_step_row(t, sj, cj, rc.cos_alpha[j], rc.sin_alpha[j], rc.a[j], rc.eps[j], nr);
+            if (live) {
+                // Stores are arranged so that the 8 lanes of a 16-byte shared-memory phase (two angle sets) hit 8
+                // different bank groups: an unrotated 512-B (or 256-B) row stride would put them all in one.
+                if (JOINTS) {
+                    if (r < 3)
+                        dst[3 * j + r] = (Real)nr[3];
+                } else if (sizeof(Real) == 8) {
+                    // row r of T_j is two 16-byte halves; odd angle sets store the second half first
+                    double2 *p = reinterpret_cast<double2 *>(dst + 16 * j + 4 * r);
+                    const double2 lo = make_double2(nr[0], nr[1]), hi = make_double2(nr[2], nr[3]);
+                    p[odd] = odd ? hi : lo;
+                    p[odd ^ 1] = odd ? lo : hi;
+                } else if (j & 1) {
+                    // row r of T_j is one float4; T_{j-1} and T_j go out together, odd angle sets T_j first
+                    float4 *p = reinterpret_cast<float4 *>(dst + 4 * r);
+                    const float4 a = make_float4((float)prev[0], (float)prev[1], (float)prev[2], (float)prev[3]);
+                    const float4 b = make_float4((float)nr[0], (float)nr[1], (float)nr[2], (float)nr[3]);
+                    p[4 * (j - 1 + odd)] = odd ? b : a;
+                    p[4 * (j - odd)] = odd ? a : b;
+                }
             }
-        for (int m = 0; m < 16; ++m) {
-            T[m] = N[m];
-            chain_out[64 * i + 16 * j + m] = N[m];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                prev[q] = nr[q];
+                t[q] = nr[q];
+            }
+        }
+        const Real *src = tiles + buf * TILE_ELEMS;
+        Real *gdst = out + row0 * ROW_ELEMS;
+        if (bulk) {
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // make the stores visible to the copy engine
+            __syncthreads();
+            if (tid == 0)
+                fkt_bulk_store(gdst, src, (unsigned)(rows * ROW_ELEMS * sizeof(Real)));
+        } else {
+            __syncthreads();
+            for (int w = tid; w < rows * ROW_ELEMS; w += FKT_THREADS)
+                gdst[w] = src[w];
         }
     }
-    status[i] = st;
+    if (bulk && tid == 0)
+        asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
 }
 
 struct LimitsArgs {
@@ -483,13 +573,48 @@ cudaError_t ikb_launch_fk(const void *angles, int angles_f64, long long n, long 
     return cudaGetLastError();
 }
 
-cudaError_t ikb_launch_fk_chain(const double *angles, long long n, double *chain_out, int *status,
-                                const IkbRobot &rc, cudaStream_t stream)
+// Persistent grid: as many CTAs as fit the SMs at once (shared memory bounds it for fp64 matrices: 64 KB per CTA).
+template <typename Real, bool JOINTS>
+static cudaError_t launch_fk_transforms(const void *angles, long long n, long long index_base, void *out,
+                                        IkbDeviceStats *stats, const IkbRobot &rc, int num_sms, cudaStream_t stream)
+{
+    constexpr int smem = 2 * FKT_ROWS * (JOINTS ? 12 : 64) * (int)sizeof(Real);
+    constexpr int kMaxDevices = 64;
+    static int ctas_per_sm[kMaxDevices] = {};  // 0: the attribute is not set on that device yet (it is per device)
+    int dev = 0;
+    cudaError_t err = cudaGetDevice(&dev);
+    if (err != cudaSuccess)
+        return err;
+    int ctas = dev < kMaxDevices ? ctas_per_sm[dev] : 0;
+    if (ctas == 0) {
+        err = cudaFuncSetAttribute(fk_transforms_kernel<Real, JOINTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (err == cudaSuccess)
+            err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fk_transforms_kernel<Real, JOINTS>, FKT_THREADS,
+                                                                smem);
+        if (err != cudaSuccess)
+            return err;
+        ctas = ctas > 0 ? ctas : 1;
+        if (dev < kMaxDevices)
+            ctas_per_sm[dev] = ctas;
+    }
+    const long long tiles = (n + FKT_ROWS - 1) / FKT_ROWS, cap = (long long)num_sms * ctas;
+    fk_transforms_kernel<Real, JOINTS><<<(unsigned)(tiles < cap ? tiles : cap), FKT_THREADS, smem, stream>>>(
+        reinterpret_cast<const Real *>(angles), n, index_base, reinterpret_cast<Real *>(out), stats, rc);
+    return cudaGetLastError();
+}
+
+cudaError_t ikb_launch_fk_transforms(const void *angles, int angles_f64, long long n, long long index_base, int what,
+                                     void *out, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                     cudaStream_t stream)
 {
     if (n <= 0)
         return cudaSuccess;
-    fk_chain_kernel<<<(unsigned)((n + 63) / 64), 64, 0, stream>>>(angles, n, chain_out, status, rc);
-    return cudaGetLastError();
+    const bool joints = what == IKB_FK_JOINTS;
+    if (angles_f64)
+        return joints ? launch_fk_transforms<double, true>(angles, n, index_base, out, stats, rc, num_sms, stream)
+                      : launch_fk_transforms<double, false>(angles, n, index_base, out, stats, rc, num_sms, stream);
+    return joints ? launch_fk_transforms<float, true>(angles, n, index_base, out, stats, rc, num_sms, stream)
+                  : launch_fk_transforms<float, false>(angles, n, index_base, out, stats, rc, num_sms, stream);
 }
 
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,

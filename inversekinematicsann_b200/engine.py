@@ -151,7 +151,7 @@ class IkEngine:
         write past or into the wrong places (wrong shape, strided view, read-only, unexpected dtype)."""
         if not isinstance(out, np.ndarray):
             raise TypeError(f"{what} must be a numpy.ndarray, not {type(out).__name__}")
-        want = (n, cols) if cols else (n,)
+        want = (n,) + (cols if isinstance(cols, tuple) else (cols,) if cols else ())
         if out.shape != want:
             raise ValueError(f"{what} must have shape {want}, got {out.shape}")
         if out.dtype not in dtypes:
@@ -269,6 +269,22 @@ class IkEngine:
         self._check(self._lib.ikb_fk_chain_host(self._handle, ang.ctypes.data, chain.ctypes.data,
                                                 ctypes.byref(status)), "ikb_fk_chain_host")
         return chain, int(status.value)
+
+    def fk_transforms(self, angles, what="matrices", out=None):
+        """The cumulative DH matrices T_1..T_4 of (n, 4) angles: (out, stats) with out (n, 4, 4, 4) for
+        what="matrices" or the joint origins (n, 4, 3) for what="joints", in the angles' dtype.
+        stats.first_fk_angle_range >= 0 marks the lowest row with an angle outside [-2pi, 2pi]."""
+        code = _choice(_FK_LAYOUTS, what, "what")
+        angles = self._rows(angles, 4, "angles")
+        n = angles.shape[0]
+        tail = _FK_TAIL[code]
+        if out is None:
+            out = np.empty((n,) + tail, dtype=angles.dtype)
+        self._check_out(out, n, tail, (angles.dtype,), "out")
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_fk_transforms_host(self._handle, angles.ctypes.data, _np_dtype_code(angles), n, code,
+                                                     out.ctypes.data, ctypes.byref(s)), "ikb_fk_transforms_host")
+        return out, IkStats.from_c(s)
 
     def mlp_load(self, weights, biases, mean_x, scale_x, mean_y, scale_y):
         """reference ann.py:78-85: upload Keras Dense kernels (in, out) + biases and both scalers."""
@@ -442,6 +458,21 @@ class IkEngine:
             _torch_dtype_code(targets) if targets is not None else _native.IKB_F64,
             err.data_ptr() if err is not None else None, _torch_stream_ptr(self.device)), "ikb_fk_device")
 
+    def fk_transforms_device(self, angles, out, what="matrices"):
+        """fk_transforms on CUDA tensors of this engine's device, enqueued on torch's current stream (no
+        synchronisation): angles (n, 4) float32 or float64, out (n, 4, 4, 4) or (n, 4, 3) in the angles' dtype.  The
+        angle guard accumulates in the engine's statistics (stats_fetch_torch)."""
+        code = _choice(_FK_LAYOUTS, what, "what")
+        angles = self._dev_rows(angles, 4, "angles")
+        n = angles.shape[0]
+        self._dev_vec(out, out.numel() if _is_torch_tensor(out) else -1, str(angles.dtype), "out")
+        want = (n,) + _FK_TAIL[code]
+        if tuple(out.shape) != want:
+            raise ValueError(f"out must have shape {want}, got {tuple(out.shape)}")
+        self._check(self._lib.ikb_fk_transforms_device(self._handle, angles.data_ptr(), _torch_dtype_code(angles), n,
+                                                       code, out.data_ptr(), _torch_stream_ptr(self.device)),
+                    "ikb_fk_transforms_device")
+
     def check_limits_device(self, xyz):
         xyz = self._dev_rows(xyz, 3, "points")
         self._check(self._lib.ikb_check_limits_device(self._handle, xyz.data_ptr(), _torch_dtype_code(xyz),
@@ -494,6 +525,8 @@ class PinnedBuffer:
 _MLP_MODES = {"fp32": _native.IKB_MLP_FP32_SIMT, "fp16x3": _native.IKB_MLP_FP16X3_TC,
               "fp16x3_ts": _native.IKB_MLP_FP16X3_TS}
 _FABRIK_PRECISIONS = {"f64": _native.IKB_FABRIK_F64, "f32": _native.IKB_FABRIK_F32}
+_FK_LAYOUTS = {"matrices": _native.IKB_FK_MATRICES, "joints": _native.IKB_FK_JOINTS}
+_FK_TAIL = {_native.IKB_FK_MATRICES: (4, 4, 4), _native.IKB_FK_JOINTS: (4, 3)}  # per-row shape of each layout
 
 
 def _choice(table, key, what):

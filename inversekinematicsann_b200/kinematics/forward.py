@@ -3,7 +3,8 @@
 ``ForwardKinematics(dh_matrix).fkine(angles)`` returns ``(T_final, [T_1 .. T_4])`` as 4x4 NumPy
 arrays exactly like the reference (forward.py:73-94); callers read the position as T[0:3, 3]
 (cli.py:60, inverse.py:130).  ``fkine_positions`` is the batched form used for the
-position-error check of both solvers.
+position-error check of both solvers.  ``fkine_batch`` is ``fkine`` for n angle sets, ``joint_positions`` gives
+the joint origins of every set, and ``fkine_device`` keeps inputs and outputs in GPU memory.
 """
 import numpy as np
 
@@ -39,6 +40,32 @@ class ForwardKinematics:
             raise OutOfRobotReachException(_ANGLE_MSG)
         mats = [np.array(chain[i]) for i in range(4)]
         return mats[-1], mats
+
+    def fkine_batch(self, angles):
+        """fkine for (n, 4) angles -> (T[n,4,4], chain[n,4,4,4]) in the angles' dtype; T is a view of chain[:, 3]."""
+        chain, stats = self._engine().fk_transforms(angles, "matrices")
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+        return chain[:, 3], chain
+
+    def joint_positions(self, angles):
+        """The four joint origins (column 3 of T_1..T_4) for (n, 4) angles -> (n, 4, 3) in the angles' dtype."""
+        joints, stats = self._engine().fk_transforms(angles, "joints")
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+        return joints
+
+    def fkine_device(self, angles, out=None, what="matrices"):
+        """fkine_batch (what="matrices": out (n,4,4,4)) or joint_positions (what="joints": out (n,4,3)) on a CUDA
+        tensor, enqueued on torch's current stream without a synchronisation; out is allocated when None.  An angle
+        outside [-2pi, 2pi] sets first_fk_angle_range of the engine's statistics (``stats_fetch_torch``)."""
+        import torch
+        eng = self._engine()
+        if out is None:
+            tail = (4, 4, 4) if what == "matrices" else (4, 3)
+            out = torch.empty((angles.shape[0],) + tail, dtype=angles.dtype, device=angles.device)
+        eng.fk_transforms_device(angles, out, what)
+        return out
 
     def fkine_positions(self, angles, targets=None):
         """Batched end-effector positions for (n, 4) angles; with `targets` also ||pos - target||."""

@@ -11,11 +11,13 @@ mkdir -p "$out/obj_$name"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 ARCH="-gencode arch=compute_100a,code=sm_100a"
 extra=""
-[ "$src" = "fabrik.cu" ] && extra="--fmad=false"
+case "$src" in fabrik.cu|fabrik_chain.cu) extra="--fmad=false" ;; esac  # as csrc/Makefile compiles them
 $NVCC $ARCH -O3 -std=c++17 -lineinfo -Xcompiler -fPIC --expt-relaxed-constexpr $extra "$@" -c -o "$out/obj_$name/${src%.cu}.o" "$csrc/$src"
+# every object the library links, from the Makefile's SRCS, so that the list cannot drift from it
+srcs=$(make -s -C "$csrc" --no-print-directory --eval 'print-srcs: ; @echo $(SRCS)' print-srcs)
 objs=""
-for f in capi fabrik fk mlp mlp_tc mlp_tc2 generators; do
-  if [ "$f.cu" = "$src" ]; then objs="$objs $out/obj_$name/$f.o"; else objs="$objs $csrc/$f.o"; fi
+for f in $srcs; do
+  if [ "$f" = "$src" ]; then objs="$objs $out/obj_$name/${f%.cu}.o"; else objs="$objs $csrc/${f%.cu}.o"; fi
 done
 $NVCC $ARCH -shared -o "$out/$name.so" $objs
 echo "$out/$name.so"
