@@ -427,6 +427,8 @@ int ikb_fabrik_solve_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64
     if (!e || n < 0 || (n > 0 && (!xyz || !angles_out)) || bad_dtype(xyz_dtype) || bad_dtype(angles_dtype) ||
         (precision != IKB_FABRIK_F64 && precision != IKB_FABRIK_F32) || n > 0x7fffffffLL)
         return fail(e, IKB_ERR_INVALID, "ikb_fabrik_solve_device: bad argument (n must be < 2^31 per call)");
+    if (((uintptr_t)angles_out & 15))  // rows are stored as float4 / double2 pairs
+        return fail(e, IKB_ERR_INVALID, "ikb_fabrik_solve_device: angles must be 16-byte aligned");
     IKB_CUDA(e, cudaSetDevice(e->device));
     const bool want_fk = n > 0 && (fk_err_out || fk_stats);
     const bool fuse = want_fk && e->rc.planar && fk_fusable(e->rc, n);
@@ -575,6 +577,8 @@ int ikb_fk_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n
     if (!e || n < 0 || (n > 0 && !angles) || bad_dtype(angles_dtype) || bad_dtype(xyz_dtype) ||
         (err_out && !targets))
         return fail(e, IKB_ERR_INVALID, "ikb_fk_device: bad argument");
+    if (((uintptr_t)angles & 15))  // rows are loaded as float4 / double2 pairs
+        return fail(e, IKB_ERR_INVALID, "ikb_fk_device: angles must be 16-byte aligned");
     IKB_CUDA(e, cudaSetDevice(e->device));
     IKB_CUDA(e, ikb_launch_fk(angles, angles_dtype == IKB_F64, n, 0, pos_out, targets, xyz_dtype == IKB_F64,
                               err_out, e->d_stats, e->rc, e->num_sms, (cudaStream_t)stream));
@@ -697,6 +701,8 @@ int ikb_ann_solve_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t 
 {
     if (!e || n < 0 || (n > 0 && (!xyz || !angles_out)) || bad_dtype(xyz_dtype))
         return fail(e, IKB_ERR_INVALID, "ikb_ann_solve_device: bad argument");
+    if (((uintptr_t)angles_out & 15))  // rows are stored as float4
+        return fail(e, IKB_ERR_INVALID, "ikb_ann_solve_device: angles must be 16-byte aligned");
     if (!e->mlp.loaded)
         return fail(e, IKB_ERR_NO_MODEL, "ikb_ann_solve: no model loaded (call ikb_mlp_load first)");
     IKB_CUDA(e, cudaSetDevice(e->device));

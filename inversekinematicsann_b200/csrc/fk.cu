@@ -137,7 +137,7 @@ __global__ void __launch_bounds__(256, FK_PAIR_MINB) fk_error_pairs_kernel(const
     const long long n_pairs = a.n >> 1;  // the odd last row (if any) is handled by one thread after the loop
     const long long stride = (long long)gridDim.x * blockDim.x;
     const float *k = a.rc.fkc_f;
-    const float TWO_PI = 6.283185307179586f;
+    const float TWO_PI = IKB_TWO_PI_F32;
     double err_sum = 0.0;
     unsigned err_cnt = 0;
     const float4 *ang = reinterpret_cast<const float4 *>(a.angles);
@@ -248,7 +248,7 @@ __global__ void __launch_bounds__(FK_STREAM_WARPS * 32, 4) fk_error_stream_kerne
     FkStage *ring = s_ring[warp];
     const long long w = (long long)blockIdx.x * FK_STREAM_WARPS + warp, W = (long long)gridDim.x * FK_STREAM_WARPS;
     const float *k = a.rc.fkc_f;
-    const float TWO_PI = 6.283185307179586f;
+    const float TWO_PI = IKB_TWO_PI_F32;
     const char *ang = reinterpret_cast<const char *>(a.angles);
     const char *tgt = reinterpret_cast<const char *>(a.targets);
     float2 *out = reinterpret_cast<float2 *>(a.err_out);

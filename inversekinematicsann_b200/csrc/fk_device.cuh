@@ -4,6 +4,18 @@
 #pragma once
 #include "ikb_common.cuh"
 
+// The angle guard of forward.py:23-25 rejects |theta| > 2 pi, compared in fp64.  (float)(2 pi) = 6.2831855f lies ABOVE
+// 2 pi, so comparing a float angle with it would accept float32(2 pi), which the reference (and fk_transforms_kernel,
+// which widens to double) rejects.  The float guard compares with the largest float below 2 pi instead: for a float
+// theta, |theta| > 6.2831850f  <=>  |(double)theta| > 2 pi.
+#define IKB_TWO_PI_F32 6.28318500518798828125f
+template <typename Real>
+__device__ __forceinline__ Real ikb_two_pi();
+template <>
+__device__ __forceinline__ float ikb_two_pi<float>() { return IKB_TWO_PI_F32; }
+template <>
+__device__ __forceinline__ double ikb_two_pi<double>() { return 6.283185307179586; }
+
 // sin/cos for |x| <= 2 pi (larger angles are rejected by the guard of forward.py:23-25 anyway):
 // two-term Cody-Waite reduction by pi/2 (|k| <= 4, exact products) + the cephes single-precision
 // kernels on [-pi/4, pi/4]; max error ~1.2e-7.  libdevice's sincosf carries a Payne-Hanek slow path whose
@@ -130,7 +142,7 @@ template <typename Real>
 __device__ __forceinline__ Real ikb_fk_error_planar_tail(const Real th[4], Real tx, Real ty, Real tz, Real a0, Real a1,
                                                          Real a2, Real a3, Real eps0, Real w, Real ca, Real sa)
 {
-    const Real TWO_PI = (Real)6.283185307179586;
+    const Real TWO_PI = ikb_two_pi<Real>();
     bool ok = true;
     Real s[4], c[4];
 #pragma unroll
@@ -163,7 +175,7 @@ template <typename Real>
 __device__ __forceinline__ bool fk_position(const IkbRobot &rc, const Real th[4], Real &px, Real &py,
                                             Real &pz)
 {
-    const Real TWO_PI = (Real)6.283185307179586;
+    const Real TWO_PI = ikb_two_pi<Real>();
     bool ok = true;
     Real s[4], c[4];
 #pragma unroll
