@@ -181,6 +181,37 @@ int ikb_fk_transforms_device(ikb_engine *e, const void *angles, int angles_dtype
                              int what, void *out, void *stream);
 int ikb_fk_transforms_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n,
                            int what, void *out, ikb_stats *stats);
+/* The arm Jacobian of n angle sets: how the effector moves when the four joints turn.  With T_0 = I and the cumulative
+ * DH matrices T_1..T_4 of ikb_fk_transforms_*, joint i turns about z_{i-1} through p_{i-1} (columns 2 and 3 of
+ * T_{i-1}) and p_4 is the effector.  angles: n x 4 of angles_dtype; the arithmetic is fp64 (float32 angles are widened
+ * exactly), outputs have the angles' dtype (a float32 output is the fp64 result rounded once).
+ *   jac_out, by `what`:
+ *     IKB_JAC_GEOMETRIC  n x 6 x 4, row-major: rows 0-2 the linear part z_{i-1} x (p_4 - p_{i-1}), rows 3-5 the
+ *                        angular part z_{i-1}; column i-1 belongs to joint i.  192 B per row in fp64.
+ *     IKB_JAC_POSITION   n x 3 x 4, rows 0-2 only.
+ *   manip_out: n values, the Yoshikawa manipulability w = sqrt(det(Jv Jv^T)) of the 3 x 4 position Jacobian Jv,
+ *     evaluated as sqrt(sum over the four 3-column subsets of det^2) (Cauchy-Binet): non-negative, 0 at singular poses.
+ *   Either output may be NULL, not both; `what` must be valid even without jac_out.
+ * Bits: z_{i-1} and p_{i-1} are the bits of ikb_fk_transforms_*'s matrices (z_0 = (0, 0, 1), p_0 = 0), and every
+ * later operation is IEEE fp64 with round-to-nearest and no contraction, in this order:
+ *   d = p_4 - p_{i-1};  linear = (z.y*d.z - z.z*d.y, z.z*d.x - z.x*d.z, z.x*d.y - z.y*d.x)
+ *   for the column subsets c_0 = (0,1,2), c_1 = (0,1,3), c_2 = (0,2,3), c_3 = (1,2,3) of Jv, with columns (a, b, c):
+ *     m = b x c in the order of the linear rows;  det_k = (a.x*m.x + a.y*m.y) + a.z*m.z;  s_k = det_k * det_k
+ *   w = sqrt((s_0 + s_1) + (s_2 + s_3)), correctly rounded.
+ * Rows with an angle (or alpha) outside [-2pi, 2pi] are still written; the lowest such row goes to
+ * stats.first_fk_angle_range (NaN passes, as for ikb_fk_transforms_*).  `angles` and both outputs must be aligned to
+ * their element size; a jac_out that is not 16-byte aligned is written with element stores instead of bulk copies.
+ * _device: DEVICE pointers, enqueued on `stream`, the guard accumulates in the statistics block; _host: HOST pointers,
+ * staged through the engine's pipeline, `stats` filled (nullable).  A host chunk holds min(S, 32 S / B) rows, S the
+ * rows of a staging slot and B the bytes of a jac_out row (S rows without jac_out); w is staged beside the Jacobians.
+ * A NULL engine with otherwise valid arguments is refused too; the text of any refusal with e == NULL is read with
+ * ikb_last_error(NULL). */
+#define IKB_JAC_GEOMETRIC 0
+#define IKB_JAC_POSITION 1
+int ikb_jacobian_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what,
+                        void *jac_out, void *manip_out, void *stream);
+int ikb_jacobian_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what,
+                      void *jac_out, void *manip_out, ikb_stats *stats);
 
 /* ---- ANN (ann.py:70-85, inverse.py:142-155) -------------------------------------------------- */
 /* replaces ANN.load_model (ann.py:78-85): upload the Keras Sequential's Dense kernels/biases and the

@@ -30,6 +30,9 @@ cudaError_t ikb_launch_fk(const void *angles, int angles_f64, long long n, long 
 cudaError_t ikb_launch_fk_transforms(const void *angles, int angles_f64, long long n, long long index_base, int what,
                                      void *out, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                      cudaStream_t stream);
+cudaError_t ikb_launch_jacobian(const void *angles, int angles_f64, long long n, long long index_base, int what,
+                                void *jac, void *manip, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                cudaStream_t stream);
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,
                                     IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                     cudaStream_t stream);
@@ -665,6 +668,79 @@ int ikb_fk_transforms_host(ikb_engine *e, const void *angles, int angles_dtype, 
                                              e->num_sms, s.stream));
         e->launches++;
         IKB_CUDA(e, cudaMemcpyAsync((char *)out + lo * out_row, s.d_out, m * out_row, cudaMemcpyDeviceToHost, s.stream));
+    }
+    return host_end(e, stats);
+}
+
+// ---- arm Jacobian and manipulability --------------------------------------------------------------
+// what is wrong with the arguments, or nullptr; the engine is checked last, so that each refusal can be told apart
+// without one
+static const char *jacobian_bad_args(const ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what,
+                                     const void *jac_out, const void *manip_out)
+{
+    if (n < 0)
+        return "negative n";
+    if (bad_dtype(angles_dtype))
+        return "unknown dtype";
+    if (what != IKB_JAC_GEOMETRIC && what != IKB_JAC_POSITION)
+        return "unknown `what`";
+    if (!jac_out && !manip_out)
+        return "both outputs are NULL";
+    if (n > 0 && !angles)
+        return "NULL angles";
+    const uintptr_t align = esize(angles_dtype) - 1;
+    if (((uintptr_t)angles | (uintptr_t)jac_out | (uintptr_t)manip_out) & align)
+        return "angles and outputs must be aligned to their element size";
+    if (!e)
+        return "NULL engine";
+    return nullptr;
+}
+
+static size_t jacobian_row_bytes(int angles_dtype, int what)
+{
+    return (what == IKB_JAC_GEOMETRIC ? 24 : 12) * esize(angles_dtype);
+}
+
+int ikb_jacobian_device(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what, void *jac_out,
+                        void *manip_out, void *stream)
+{
+    if (const char *why = jacobian_bad_args(e, angles, angles_dtype, n, what, jac_out, manip_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_jacobian_device: ") + why);
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    IKB_CUDA(e, ikb_launch_jacobian(angles, angles_dtype == IKB_F64, n, 0, what, jac_out, manip_out, e->d_stats, e->rc,
+                                    e->num_sms, (cudaStream_t)stream));
+    e->launches += (n > 0);
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline: angles in d_in (32 B per slot row), Jacobians in d_out (as many rows as its 32 B per
+// slot row hold at the Jacobian's row size, at most one per slot row), manipulabilities in d_in2 (24 B per slot row).
+int ikb_jacobian_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what, void *jac_out,
+                      void *manip_out, ikb_stats *stats)
+{
+    if (const char *why = jacobian_bad_args(e, angles, angles_dtype, n, what, jac_out, manip_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_jacobian_host: ") + why);
+    int rc = host_begin(e, n);
+    if (rc)
+        return rc;
+    const size_t in_row = 4 * esize(angles_dtype), jac_row = jacobian_row_bytes(angles_dtype, what);
+    const size_t w_row = esize(angles_dtype);
+    const long long m_max = jac_out ? std::min(e->slot_rows, e->slot_rows * 32 / (long long)jac_row) : e->slot_rows;
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)angles + lo * in_row, m * in_row, cudaMemcpyHostToDevice,
+                                    s.stream));
+        IKB_CUDA(e, ikb_launch_jacobian(s.d_in, angles_dtype == IKB_F64, m, lo, what, jac_out ? s.d_out : nullptr,
+                                        manip_out ? s.d_in2 : nullptr, e->d_stats, e->rc, e->num_sms, s.stream));
+        e->launches++;
+        if (jac_out)
+            IKB_CUDA(e, cudaMemcpyAsync((char *)jac_out + lo * jac_row, s.d_out, m * jac_row, cudaMemcpyDeviceToHost,
+                                        s.stream));
+        if (manip_out)
+            IKB_CUDA(e, cudaMemcpyAsync((char *)manip_out + lo * w_row, s.d_in2, m * w_row, cudaMemcpyDeviceToHost,
+                                        s.stream));
     }
     return host_end(e, stats);
 }

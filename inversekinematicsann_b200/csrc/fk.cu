@@ -5,7 +5,8 @@
 //   T = prod_i Rz(theta_i) Tz(eps_i) Tx(a_i) Rx(alpha_i)                      (forward.py:62-70)
 // Only what callers read is produced in the batched form -- the end-effector position T[0:3, 3]
 // (cli.py:60, inverse.py:130, tests/forward_unit.py:30) and ||pos - target||.  fk_transforms_kernel
-// returns all four cumulative 4x4 matrices (or the joint origins) for the (T, [T1..T4]) return value of fkine.
+// returns all four cumulative 4x4 matrices (or the joint origins) for the (T, [T1..T4]) return value of fkine, and
+// from the same chain the arm Jacobian and its manipulability.
 // HBM-bound: 16 B angles + 12 B target in, 4 B error out per row (fp32 buffers).
 #include <cstdlib>
 
@@ -362,21 +363,39 @@ __device__ __forceinline__ void fkt_bulk_store(void *dst, const void *src, unsig
 constexpr int FKT_ROWS = 64;              // angle sets per tile
 constexpr int FKT_THREADS = 4 * FKT_ROWS;  // one quad per angle set
 
-// Real: dtype of angles and output.  JOINTS: n x 4 x 3 (column 3 of T_1..T_4) instead of n x 4 x 4 x 4.
-// Dynamic shared memory: two tiles of FKT_ROWS * ROW_ELEMS elements.
-template <typename Real, bool JOINTS>
+// What fk_transforms_kernel writes per angle set (the tile row, in elements):
+//   FKT_MATRICES      T_1..T_4, 4 x 4 x 4 (64)
+//   FKT_JOINTS        column 3 of T_1..T_4, 4 x 3 (12)
+//   FKT_JAC_GEOMETRIC the 6 x 4 geometric Jacobian (24)
+//   FKT_JAC_POSITION  its rows 0-2, the 3 x 4 position Jacobian (12)
+//   FKT_MANIP_ONLY    no tile; only the manipulability below
+// The Jacobian kinds may also write the manipulability w (template MANIP), one element per angle set straight from the
+// quad to `manip`.
+enum FktKind { FKT_MATRICES, FKT_JOINTS, FKT_JAC_GEOMETRIC, FKT_JAC_POSITION, FKT_MANIP_ONLY };
+
+constexpr int fkt_row_elems(int kind)
+{
+    return kind == FKT_MATRICES ? 64 : kind == FKT_JAC_GEOMETRIC ? 24 : kind == FKT_MANIP_ONLY ? 0 : 12;
+}
+
+// Real: dtype of angles and outputs.  Dynamic shared memory: two tiles of FKT_ROWS * fkt_row_elems(KIND) elements.
+template <typename Real, int KIND, bool MANIP>
 __global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *__restrict__ angles, long long n,
                                                                     long long index_base, Real *out,
-                                                                    IkbDeviceStats *stats, const IkbRobot rc)
+                                                                    IkbDeviceStats *stats, const IkbRobot rc,
+                                                                    Real *manip)
 {
-    constexpr int ROW_ELEMS = JOINTS ? 12 : 64;
+    constexpr bool JOINTS = KIND == FKT_JOINTS;
+    constexpr bool JAC = KIND >= FKT_JAC_GEOMETRIC;
+    constexpr int ROW_ELEMS = fkt_row_elems(KIND);
+    constexpr bool TILED = ROW_ELEMS > 0;
     constexpr int TILE_ELEMS = FKT_ROWS * ROW_ELEMS;
     extern __shared__ __align__(128) unsigned char fkt_smem[];
     Real *const tiles = reinterpret_cast<Real *>(fkt_smem);
     const double TWO_PI = 6.283185307179586;
     const int tid = threadIdx.x, r = tid & 3, lrow = tid >> 2;
     const int odd = lrow & 1;
-    const bool bulk = ((uintptr_t)out & 15) == 0;  // every row size here is a multiple of 16 bytes
+    const bool bulk = TILED && ((uintptr_t)out & 15) == 0;  // every row size here is a multiple of 16 bytes
     const bool alpha_bad = rc.alpha[r] < -TWO_PI || rc.alpha[r] > TWO_PI;
     const long long n_tiles = (n + FKT_ROWS - 1) / FKT_ROWS;
     int buf = 0;
@@ -394,16 +413,20 @@ __global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *
         // the bulk copy that last read this buffer (two tiles ago) must be done reading it
         if (bulk && tid == 0)
             asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-        __syncthreads();
+        if (TILED)
+            __syncthreads();
         Real *const dst = tiles + buf * TILE_ELEMS + lrow * ROW_ELEMS;
         double t[4] = {r == 0 ? 1.0 : 0.0, r == 1 ? 1.0 : 0.0, r == 2 ? 1.0 : 0.0, r == 3 ? 1.0 : 0.0};
         double prev[4];
+        double zs[4], ps[5];  // Jacobian kinds: element r of z_j and p_j, columns 2 and 3 of T_j (T_0 = I)
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const double sj = __shfl_sync(IKB_FULL_MASK, s, j, 4), cj = __shfl_sync(IKB_FULL_MASK, c, j, 4);
             double nr[4];
+            zs[j] = t[2];
+            ps[j] = t[3];
             fk_dh_step_row(t, sj, cj, rc.cos_alpha[j], rc.sin_alpha[j], rc.a[j], rc.eps[j], nr);
-            if (live) {
+            if (!JAC && live) {
                 // Stores are arranged so that the 8 lanes of a 16-byte shared-memory phase (two angle sets) hit 8
                 // different bank groups: an unrotated 512-B (or 256-B) row stride would put them all in one.
                 if (JOINTS) {
@@ -430,17 +453,95 @@ __global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *
                 t[q] = nr[q];
             }
         }
-        const Real *src = tiles + buf * TILE_ELEMS;
-        Real *gdst = out + row0 * ROW_ELEMS;
-        if (bulk) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // make the stores visible to the copy engine
-            __syncthreads();
-            if (tid == 0)
-                fkt_bulk_store(gdst, src, (unsigned)(rows * ROW_ELEMS * sizeof(Real)));
-        } else {
-            __syncthreads();
-            for (int w = tid; w < rows * ROW_ELEMS; w += FKT_THREADS)
-                gdst[w] = src[w];
+        ps[4] = t[3];
+        if (JAC) {
+            // Column i-1 (joint i) of the position Jacobian is z_{i-1} x (p_4 - p_{i-1}).  Lane r < 3 computes element r:
+            // z[r+1] * d[r+2] - z[r+2] * d[r+1] (indices mod 3: y*z' - z*y' for x, ...), with the operands of the other
+            // two elements fetched from their lanes.  Every operation is explicitly rounded (no contraction), so a
+            // NumPy restatement on fkine_batch's matrices reproduces the bits.  Lane 3 computes an unused value.
+            const int r1 = r < 2 ? r + 1 : r - 2, r2 = r == 0 ? 2 : r - 1;
+            const double p4a = __shfl_sync(IKB_FULL_MASK, ps[4], r1, 4), p4b = __shfl_sync(IKB_FULL_MASK, ps[4], r2, 4);
+            double lin[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                // z_0 = (0, 0, 1) and p_0 = 0 are constants
+                const double za = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r1, 4) : (r1 == 2 ? 1.0 : 0.0);
+                const double zb = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r2, 4) : (r2 == 2 ? 1.0 : 0.0);
+                const double pa = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r1, 4) : 0.0;
+                const double pb = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r2, 4) : 0.0;
+                lin[k] = __dsub_rn(__dmul_rn(za, __dsub_rn(p4b, pb)), __dmul_rn(zb, __dsub_rn(p4a, pa)));
+            }
+            if (MANIP) {
+                // w^2 = sum over the four 3-column subsets of det^2 (Cauchy-Binet).  Lane r takes the subset without
+                // column 3 - r: (0,1,2), (0,1,3), (0,2,3), (1,2,3) for r = 0..3, det = a . (b x c), b x c in the
+                // order of the linear rows, the dot product summed (x + y) + z; then w = sqrt((s0 + s1) + (s2 + s3)).
+                double J[3][4];
+#pragma unroll
+                for (int q = 0; q < 3; ++q)
+#pragma unroll
+                    for (int k = 0; k < 4; ++k)
+                        J[q][k] = __shfl_sync(IKB_FULL_MASK, lin[k], q, 4);
+                double a[3], b[3], cc[3];
+#pragma unroll
+                for (int q = 0; q < 3; ++q) {
+                    a[q] = r == 3 ? J[q][1] : J[q][0];
+                    b[q] = r >= 2 ? J[q][2] : J[q][1];
+                    cc[q] = r >= 1 ? J[q][3] : J[q][2];
+                }
+                const double m0 = __dsub_rn(__dmul_rn(b[1], cc[2]), __dmul_rn(b[2], cc[1]));
+                const double m1 = __dsub_rn(__dmul_rn(b[2], cc[0]), __dmul_rn(b[0], cc[2]));
+                const double m2 = __dsub_rn(__dmul_rn(b[0], cc[1]), __dmul_rn(b[1], cc[0]));
+                const double det = __dadd_rn(__dadd_rn(__dmul_rn(a[0], m0), __dmul_rn(a[1], m1)), __dmul_rn(a[2], m2));
+                double w2 = __dmul_rn(det, det);
+                w2 = __dadd_rn(w2, __shfl_xor_sync(IKB_FULL_MASK, w2, 1, 4));  // lanes 0, 1: s0 + s1 (addition commutes)
+                w2 = __dadd_rn(w2, __shfl_xor_sync(IKB_FULL_MASK, w2, 2, 4));
+                if (live && r == 0)
+                    manip[row0 + lrow] = (Real)__dsqrt_rn(w2);
+            }
+            if (TILED && live && r < 3) {
+                // row r (linear) and row 3 + r (angular: z_{i-1}, i.e. element r of zs) of the 6 x 4 Jacobian.
+                // As for the matrices, the stores are arranged so that the two angle sets of a 16-byte shared-memory
+                // phase hit distinct bank groups.
+                if (sizeof(Real) == 8) {
+                    // each row is two 16-byte halves; odd angle sets store the second half first
+                    double2 *pl = reinterpret_cast<double2 *>(dst + 4 * r);
+                    const double2 l0 = make_double2(lin[0], lin[1]), l1 = make_double2(lin[2], lin[3]);
+                    pl[odd] = odd ? l1 : l0;
+                    pl[odd ^ 1] = odd ? l0 : l1;
+                    if (KIND == FKT_JAC_GEOMETRIC) {
+                        double2 *pa = reinterpret_cast<double2 *>(dst + 12 + 4 * r);
+                        const double2 a0 = make_double2(zs[0], zs[1]), a1 = make_double2(zs[2], zs[3]);
+                        pa[odd] = odd ? a1 : a0;
+                        pa[odd ^ 1] = odd ? a0 : a1;
+                    }
+                } else {
+                    float4 *q = reinterpret_cast<float4 *>(dst);
+                    const float4 L = make_float4((float)lin[0], (float)lin[1], (float)lin[2], (float)lin[3]);
+                    if (KIND == FKT_JAC_POSITION) {
+                        q[r] = L;  // 48-B rows: the two angle sets of a phase already cover six distinct bank groups
+                    } else {
+                        // 96-B rows, six 16-B slots: lane 2 of an odd angle set stores its angular row first
+                        const float4 A = make_float4((float)zs[0], (float)zs[1], (float)zs[2], (float)zs[3]);
+                        const bool swap = odd && r == 2;
+                        q[swap ? 3 + r : r] = swap ? A : L;
+                        q[swap ? r : 3 + r] = swap ? L : A;
+                    }
+                }
+            }
+        }
+        if (TILED) {
+            const Real *src = tiles + buf * TILE_ELEMS;
+            Real *gdst = out + row0 * ROW_ELEMS;
+            if (bulk) {
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // make the stores visible to the copy engine
+                __syncthreads();
+                if (tid == 0)
+                    fkt_bulk_store(gdst, src, (unsigned)(rows * ROW_ELEMS * sizeof(Real)));
+            } else {
+                __syncthreads();
+                for (int w = tid; w < rows * ROW_ELEMS; w += FKT_THREADS)
+                    gdst[w] = src[w];
+            }
         }
     }
     if (bulk && tid == 0)
@@ -574,11 +675,12 @@ cudaError_t ikb_launch_fk(const void *angles, int angles_f64, long long n, long 
 }
 
 // Persistent grid: as many CTAs as fit the SMs at once (shared memory bounds it for fp64 matrices: 64 KB per CTA).
-template <typename Real, bool JOINTS>
+template <typename Real, int KIND, bool MANIP = false>
 static cudaError_t launch_fk_transforms(const void *angles, long long n, long long index_base, void *out,
-                                        IkbDeviceStats *stats, const IkbRobot &rc, int num_sms, cudaStream_t stream)
+                                        IkbDeviceStats *stats, const IkbRobot &rc, int num_sms, cudaStream_t stream,
+                                        void *manip = nullptr)
 {
-    constexpr int smem = 2 * FKT_ROWS * (JOINTS ? 12 : 64) * (int)sizeof(Real);
+    constexpr int smem = 2 * FKT_ROWS * fkt_row_elems(KIND) * (int)sizeof(Real);
     constexpr int kMaxDevices = 64;
     static int ctas_per_sm[kMaxDevices] = {};  // 0: the attribute is not set on that device yet (it is per device)
     int dev = 0;
@@ -587,10 +689,11 @@ static cudaError_t launch_fk_transforms(const void *angles, long long n, long lo
         return err;
     int ctas = dev < kMaxDevices ? ctas_per_sm[dev] : 0;
     if (ctas == 0) {
-        err = cudaFuncSetAttribute(fk_transforms_kernel<Real, JOINTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        err = cudaFuncSetAttribute(fk_transforms_kernel<Real, KIND, MANIP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   smem);
         if (err == cudaSuccess)
-            err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fk_transforms_kernel<Real, JOINTS>, FKT_THREADS,
-                                                                smem);
+            err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, fk_transforms_kernel<Real, KIND, MANIP>,
+                                                                FKT_THREADS, smem);
         if (err != cudaSuccess)
             return err;
         ctas = ctas > 0 ? ctas : 1;
@@ -598,8 +701,9 @@ static cudaError_t launch_fk_transforms(const void *angles, long long n, long lo
             ctas_per_sm[dev] = ctas;
     }
     const long long tiles = (n + FKT_ROWS - 1) / FKT_ROWS, cap = (long long)num_sms * ctas;
-    fk_transforms_kernel<Real, JOINTS><<<(unsigned)(tiles < cap ? tiles : cap), FKT_THREADS, smem, stream>>>(
-        reinterpret_cast<const Real *>(angles), n, index_base, reinterpret_cast<Real *>(out), stats, rc);
+    fk_transforms_kernel<Real, KIND, MANIP><<<(unsigned)(tiles < cap ? tiles : cap), FKT_THREADS, smem, stream>>>(
+        reinterpret_cast<const Real *>(angles), n, index_base, reinterpret_cast<Real *>(out), stats, rc,
+        reinterpret_cast<Real *>(manip));
     return cudaGetLastError();
 }
 
@@ -611,10 +715,41 @@ cudaError_t ikb_launch_fk_transforms(const void *angles, int angles_f64, long lo
         return cudaSuccess;
     const bool joints = what == IKB_FK_JOINTS;
     if (angles_f64)
-        return joints ? launch_fk_transforms<double, true>(angles, n, index_base, out, stats, rc, num_sms, stream)
-                      : launch_fk_transforms<double, false>(angles, n, index_base, out, stats, rc, num_sms, stream);
-    return joints ? launch_fk_transforms<float, true>(angles, n, index_base, out, stats, rc, num_sms, stream)
-                  : launch_fk_transforms<float, false>(angles, n, index_base, out, stats, rc, num_sms, stream);
+        return joints ? launch_fk_transforms<double, FKT_JOINTS>(angles, n, index_base, out, stats, rc, num_sms, stream)
+                      : launch_fk_transforms<double, FKT_MATRICES>(angles, n, index_base, out, stats, rc, num_sms, stream);
+    return joints ? launch_fk_transforms<float, FKT_JOINTS>(angles, n, index_base, out, stats, rc, num_sms, stream)
+                  : launch_fk_transforms<float, FKT_MATRICES>(angles, n, index_base, out, stats, rc, num_sms, stream);
+}
+
+template <typename Real>
+static cudaError_t launch_jacobian(const void *angles, long long n, long long index_base, bool geometric, void *jac,
+                                   void *manip, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                   cudaStream_t stream)
+{
+    if (!jac)
+        return launch_fk_transforms<Real, FKT_MANIP_ONLY, true>(angles, n, index_base, nullptr, stats, rc, num_sms,
+                                                                stream, manip);
+    if (geometric)
+        return manip ? launch_fk_transforms<Real, FKT_JAC_GEOMETRIC, true>(angles, n, index_base, jac, stats, rc, num_sms,
+                                                                           stream, manip)
+                     : launch_fk_transforms<Real, FKT_JAC_GEOMETRIC, false>(angles, n, index_base, jac, stats, rc,
+                                                                            num_sms, stream);
+    return manip ? launch_fk_transforms<Real, FKT_JAC_POSITION, true>(angles, n, index_base, jac, stats, rc, num_sms,
+                                                                      stream, manip)
+                 : launch_fk_transforms<Real, FKT_JAC_POSITION, false>(angles, n, index_base, jac, stats, rc, num_sms,
+                                                                       stream);
+}
+
+// the arm Jacobian (what: IKB_JAC_GEOMETRIC / IKB_JAC_POSITION) into jac and/or the manipulability into manip
+cudaError_t ikb_launch_jacobian(const void *angles, int angles_f64, long long n, long long index_base, int what,
+                                void *jac, void *manip, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                cudaStream_t stream)
+{
+    if (n <= 0)
+        return cudaSuccess;
+    const bool geometric = what == IKB_JAC_GEOMETRIC;
+    return angles_f64 ? launch_jacobian<double>(angles, n, index_base, geometric, jac, manip, stats, rc, num_sms, stream)
+                      : launch_jacobian<float>(angles, n, index_base, geometric, jac, manip, stats, rc, num_sms, stream);
 }
 
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,

@@ -286,6 +286,39 @@ class IkEngine:
                                                      out.ctypes.data, ctypes.byref(s)), "ikb_fk_transforms_host")
         return out, IkStats.from_c(s)
 
+    def jacobian(self, angles, what="geometric", manipulability=False, out=None):
+        """The arm Jacobian of (n, 4) angles: (jac, manip, stats) in the angles' dtype.  jac is (n, 6, 4) for
+        what="geometric" (rows 0-2 linear, rows 3-5 angular, column i-1 for joint i), (n, 3, 4) for what="position",
+        and None for what=None; manip is the manipulability sqrt(det(Jv Jv^T)) (n,) when `manipulability`, else None.
+        stats.first_fk_angle_range >= 0 marks the lowest row with an angle outside [-2pi, 2pi]."""
+        angles, code, out = self._jacobian_args(angles, what, manipulability, out)
+        manip = np.empty(angles.shape[0], dtype=angles.dtype) if manipulability else None
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_jacobian_host(self._handle, angles.ctypes.data, _np_dtype_code(angles),
+                                                angles.shape[0], code, out.ctypes.data if out is not None else None,
+                                                manip.ctypes.data if manip is not None else None, ctypes.byref(s)),
+                    "ikb_jacobian_host")
+        return out, manip, IkStats.from_c(s)
+
+    @staticmethod
+    def _jacobian_args(angles, what, manipulability, out):
+        """The checks of `jacobian` that need no device -> (angles, layout code, out or None)."""
+        if what is None:
+            if not manipulability:
+                raise ValueError("what=None asks for no Jacobian: ask for the manipulability then")
+            if out is not None:
+                raise ValueError("out holds Jacobians, but what=None")
+            code = _native.IKB_JAC_GEOMETRIC  # ignored without a Jacobian output
+        else:
+            code = _choice(_JAC_LAYOUTS, what, "what")
+        angles = IkEngine._rows(angles, 4, "angles")
+        if what is not None:
+            tail = _JAC_TAIL[code]
+            if out is None:
+                out = np.empty((angles.shape[0],) + tail, dtype=angles.dtype)
+            IkEngine._check_out(out, angles.shape[0], tail, (angles.dtype,), "out")
+        return angles, code, out
+
     def mlp_load(self, weights, biases, mean_x, scale_x, mean_y, scale_y):
         """reference ann.py:78-85: upload Keras Dense kernels (in, out) + biases and both scalers."""
         ws = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
@@ -473,6 +506,32 @@ class IkEngine:
                                                        code, out.data_ptr(), _torch_stream_ptr(self.device)),
                     "ikb_fk_transforms_device")
 
+    def jacobian_device(self, angles, out, what="geometric", manip=None):
+        """jacobian on CUDA tensors of this engine's device, enqueued on torch's current stream (no synchronisation):
+        angles (n, 4) float32 or float64; out (n, 6, 4) or (n, 3, 4) by `what`, or None for no Jacobian; manip (n,) or
+        None; not both None, all in the angles' dtype.  The angle guard accumulates in the engine's statistics
+        (stats_fetch_torch)."""
+        code = _choice(_JAC_LAYOUTS, what, "what")
+        angles = self._dev_rows(angles, 4, "angles")
+        n = angles.shape[0]
+        if out is None and manip is None:
+            raise ValueError("jacobian_device needs out, manip or both")
+        if out is not None:
+            self._dev_vec(out, out.numel() if _is_torch_tensor(out) else -1, str(angles.dtype), "out")
+            want = (n,) + _JAC_TAIL[code]
+            if tuple(out.shape) != want:
+                raise ValueError(f"out must have shape {want}, got {tuple(out.shape)}")
+        if manip is not None:
+            self._dev_vec(manip, n, str(angles.dtype), "manip")
+            if tuple(manip.shape) != (n,):
+                raise ValueError(f"manip must have shape ({n},), got {tuple(manip.shape)}")
+        if n == 0:  # nothing to do, and an empty tensor's data_ptr() may be NULL
+            return
+        self._check(self._lib.ikb_jacobian_device(self._handle, angles.data_ptr(), _torch_dtype_code(angles), n, code,
+                                                  out.data_ptr() if out is not None else None,
+                                                  manip.data_ptr() if manip is not None else None,
+                                                  _torch_stream_ptr(self.device)), "ikb_jacobian_device")
+
     def check_limits_device(self, xyz):
         xyz = self._dev_rows(xyz, 3, "points")
         self._check(self._lib.ikb_check_limits_device(self._handle, xyz.data_ptr(), _torch_dtype_code(xyz),
@@ -527,6 +586,8 @@ _MLP_MODES = {"fp32": _native.IKB_MLP_FP32_SIMT, "fp16x3": _native.IKB_MLP_FP16X
 _FABRIK_PRECISIONS = {"f64": _native.IKB_FABRIK_F64, "f32": _native.IKB_FABRIK_F32}
 _FK_LAYOUTS = {"matrices": _native.IKB_FK_MATRICES, "joints": _native.IKB_FK_JOINTS}
 _FK_TAIL = {_native.IKB_FK_MATRICES: (4, 4, 4), _native.IKB_FK_JOINTS: (4, 3)}  # per-row shape of each layout
+_JAC_LAYOUTS = {"geometric": _native.IKB_JAC_GEOMETRIC, "position": _native.IKB_JAC_POSITION}
+_JAC_TAIL = {_native.IKB_JAC_GEOMETRIC: (6, 4), _native.IKB_JAC_POSITION: (3, 4)}
 
 
 def _choice(table, key, what):

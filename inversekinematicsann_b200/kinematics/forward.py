@@ -4,7 +4,8 @@
 arrays exactly like the reference (forward.py:73-94); callers read the position as T[0:3, 3]
 (cli.py:60, inverse.py:130).  ``fkine_positions`` is the batched form used for the
 position-error check of both solvers.  ``fkine_batch`` is ``fkine`` for n angle sets, ``joint_positions`` gives
-the joint origins of every set, and ``fkine_device`` keeps inputs and outputs in GPU memory.
+the joint origins of every set, and ``fkine_device`` keeps inputs and outputs in GPU memory.  ``jacobian``,
+``jacobian_batch``, ``manipulability`` and ``jacobian_device`` give how the effector moves when the joints turn.
 """
 import numpy as np
 
@@ -73,3 +74,37 @@ class ForwardKinematics:
         if stats.first_fk_angle_range >= 0:
             raise OutOfRobotReachException(_ANGLE_MSG)
         return (pos, err) if targets is not None else pos
+
+    def jacobian(self, angles):
+        """The (6, 4) fp64 geometric Jacobian of one set of joint angles: rows 0-2 the linear part
+        z_{i-1} x (p_4 - p_{i-1}), rows 3-5 the joint axis z_{i-1}, column i-1 for joint i.  The batch kernel at n = 1."""
+        return self.jacobian_batch(np.asarray(angles, dtype=np.float64).reshape(1, 4))[0]
+
+    def jacobian_batch(self, angles, what="geometric"):
+        """jacobian for (n, 4) angles -> (n, 6, 4) (what="geometric") or the position rows only, (n, 3, 4)
+        (what="position"), in the angles' dtype."""
+        jac, _, stats = self._engine().jacobian(angles, what)
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+        return jac
+
+    def manipulability(self, angles):
+        """Yoshikawa manipulability sqrt(det(Jv Jv^T)) of the 3 x 4 position Jacobian for (n, 4) angles -> (n,) in the
+        angles' dtype: 0 at a singular pose, such as the stretched arm."""
+        _, w, stats = self._engine().jacobian(angles, None, manipulability=True)
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+        return w
+
+    def jacobian_device(self, angles, out=None, what="geometric", manip_out=None):
+        """jacobian_batch on a CUDA tensor, enqueued on torch's current stream without a synchronisation: out (n,6,4)
+        or (n,3,4) by `what`, allocated when None (what=None: no Jacobian, out stays None); manip_out (n,), when given,
+        receives the manipulability.  Returns out.  An angle outside [-2pi, 2pi] sets first_fk_angle_range of the
+        engine's statistics (``stats_fetch_torch``)."""
+        import torch
+        eng = self._engine()
+        if out is None and what is not None:
+            tail = (6, 4) if what == "geometric" else (3, 4)
+            out = torch.empty((angles.shape[0],) + tail, dtype=angles.dtype, device=angles.device)
+        eng.jacobian_device(angles, out, what if what is not None else "geometric", manip_out)
+        return out
