@@ -213,6 +213,53 @@ int ikb_jacobian_device(ikb_engine *e, const void *angles, int angles_dtype, int
 int ikb_jacobian_host(ikb_engine *e, const void *angles, int angles_dtype, int64_t n, int what,
                       void *jac_out, void *manip_out, ikb_stats *stats);
 
+/* Damped-least-squares (DLS) refinement of joint angles onto position targets: from a seed, every row repeats
+ * Delta theta = Jv^T (Jv Jv^T + lambda^2 I)^-1 e, e = target - p_4, until it meets its own tolerance.  It puts the
+ * effector on the target where FABRIK stops at its err_margin and the network's prediction a few millimetres away.
+ *   xyz: n x 3 targets of xyz_dtype.  seed: n_seed x 4 angles of angles_dtype, n_seed == 1 (one seed for every row,
+ *   e.g. the DH table's seed row) or n.  angles_out: n x 4 of angles_dtype; angles_out == seed with n_seed == n refines
+ *   in place, any other overlap of the two is refused.  iters_out (nullable): the steps taken per row.  err_out
+ *   (nullable, angles_dtype): ||target - p_4(theta_out)|| per row.  damping = lambda (metres), tol in metres,
+ *   max_iter >= 0; max_iter = 0 returns the seeds with their errors.
+ * The arithmetic is fp64 (float32 seeds and targets are widened exactly; a float32 output is the fp64 result rounded
+ * once).  p_4 and Jv of an iterate are the bits of ikb_fk_transforms_* (IKB_FK_JOINTS, column 3 of T_4) and of
+ * ikb_jacobian_* (IKB_JAC_POSITION) for it.  Every later operation is IEEE fp64 with round-to-nearest and no
+ * contraction.  Per row, with k = 0:
+ *   1. e = target - p_4;  err = sqrt((e.x*e.x + e.y*e.y) + e.z*e.z)
+ *   2. err <= tol: stop (converged).   3. k == max_iter: stop (not converged; NaN rows end here).
+ *   4. A = Jv Jv^T + lambda^2 I: A_ij = (J_i0*J_j0 + J_i1*J_j1) + (J_i2*J_j2 + J_i3*J_j3), then A_ii += L, where
+ *      L = lambda*lambda rounded once.  A y = e by LDL^T:
+ *        l10 = A01/A00;  l20 = A02/A00;  d1 = A11 - l10*A01;  t = A12 - l20*A01;  l21 = t/d1;
+ *        d2 = (A22 - l20*A02) - l21*t;
+ *        z1 = e.y - l10*e.x;  z2 = (e.z - l20*e.x) - l21*z1;
+ *        y2 = z2/d2;  y1 = z1/d1 - l21*y2;  y0 = (e.x/A00 - l10*y1) - l20*y2
+ *      theta_k = theta_k + ((J_0k*y0 + J_1k*y1) + J_2k*y2), then theta_k = remainder(theta_k, 2pi) when
+ *      |theta_k| > pi (IEEE remainder, exact: every iterate stays inside the FK guard);  k += 1;  back to 1.
+ *   (pi and 2pi are the doubles nearest them.)  iters_out = k and err_out = err at the stop.
+ * Guards (rows are still computed and written): a target outside the workspace box sets stats.first_out_of_limits
+ * (the inclusive test of ikb_check_limits_*, NaN passes); a seed angle, or an alpha, outside [-2pi, 2pi] sets
+ * stats.first_fk_angle_range (the test of ikb_fk_transforms_*).  Statistics: n_solved rows, sum_iterations steps,
+ * n_iter_capped rows that ended above tol (NaN rows included), sum_fk_error / n_fk_error the final errors of the
+ * finite rows.
+ * Refused with IKB_ERR_INVALID before the engine is looked at, each with its own message (read with
+ * ikb_last_error(NULL) when e == NULL): NULL targets, seeds or angles_out (n > 0), negative n, n_seed not 1 or n, an
+ * unknown dtype, damping <= 0 or not finite, tol < 0 or NaN, max_iter < 0, a buffer not aligned to its element size
+ * (iters_out: 4 bytes), a partial overlap of seed and angles_out, and a NULL engine.  Nothing is launched for a
+ * refused call or for n = 0.
+ * _device: DEVICE pointers, enqueued on `stream`, one launch; statistics accumulate in the engine's block.  _host:
+ * HOST pointers, staged through the engine's pipeline with no per-call allocation, `stats` filled (nullable): targets
+ * in the slot's target buffer, seeds in its input buffer (a single seed copied once per slot), angles in its output
+ * buffer, iterations in its auxiliary buffer, and err_out behind the targets.  A host chunk, one launch, holds
+ * 3 S / 4 rows with err_out and S rows without, S the rows of a staging slot. */
+int ikb_dls_refine_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n, const void *seed, int64_t n_seed,
+                          void *angles_out, int angles_dtype, double damping, double tol, int32_t max_iter,
+                          int32_t *iters_out /* nullable */, void *err_out /* nullable, angles_dtype */,
+                          void *stream);
+int ikb_dls_refine_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n, const void *seed, int64_t n_seed,
+                        void *angles_out, int angles_dtype, double damping, double tol, int32_t max_iter,
+                        int32_t *iters_out /* nullable */, void *err_out /* nullable, angles_dtype */,
+                        ikb_stats *stats);
+
 /* ---- ANN (ann.py:70-85, inverse.py:142-155) -------------------------------------------------- */
 /* replaces ANN.load_model (ann.py:78-85): upload the Keras Sequential's Dense kernels/biases and the
  * two StandardScalers.  dims[n_layers+1] = {3, 500, ..., 500, 4}; weights[l] is row-major

@@ -26,7 +26,7 @@ EXPORTED_SYMBOLS = [
     "ikb_fabrik_solve_device", "ikb_fabrik_solve_host", "ikb_fabrik_calculate_host",
     "ikb_fabrik_chain_device", "ikb_fabrik_chain_host",
     "ikb_fk_device", "ikb_fk_host", "ikb_fk_chain_host", "ikb_fk_transforms_device", "ikb_fk_transforms_host",
-    "ikb_jacobian_device", "ikb_jacobian_host",
+    "ikb_jacobian_device", "ikb_jacobian_host", "ikb_dls_refine_device", "ikb_dls_refine_host",
     "ikb_mlp_load", "ikb_ann_solve_device", "ikb_ann_solve_host",
     "ikb_generate_device", "ikb_microbench_fma", "ikb_launch_count",
     "ikb_host_alloc", "ikb_host_free", "ikb_host_register", "ikb_host_unregister",
@@ -95,6 +95,9 @@ def load():
         "ikb_fk_transforms_host": (i32, [engine, vp, i32, i64, i32, vp, stats_p]),
         "ikb_jacobian_device": (i32, [engine, vp, i32, i64, i32, vp, vp, vp]),
         "ikb_jacobian_host": (i32, [engine, vp, i32, i64, i32, vp, vp, stats_p]),
+        "ikb_dls_refine_device": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl, dbl, ctypes.c_int32, vp, vp, vp]),
+        "ikb_dls_refine_host": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl, dbl, ctypes.c_int32, vp, vp,
+                                      stats_p]),
         "ikb_mlp_load": (i32, [engine, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
                                ctypes.POINTER(vp), ctypes.POINTER(vp), vp, vp, vp, vp]),
         "ikb_ann_solve_device": (i32, [engine, vp, i32, i64, vp, vp, i32, i32, vp]),

@@ -33,6 +33,11 @@ cudaError_t ikb_launch_fk_transforms(const void *angles, int angles_f64, long lo
 cudaError_t ikb_launch_jacobian(const void *angles, int angles_f64, long long n, long long index_base, int what,
                                 void *jac, void *manip, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                 cudaStream_t stream);
+cudaError_t ikb_launch_dls_refine(const void *xyz, int xyz_f64, const void *seed, long long n_seed, void *angles_out,
+                                  int angles_f64, int *iters, void *err_out, long long n, long long index_base,
+                                  double damping, double tol, int max_iter, IkbDeviceStats *stats,
+                                  unsigned long long *work_counter, const IkbRobot &rc, int num_sms,
+                                  cudaStream_t stream);
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,
                                     IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                     cudaStream_t stream);
@@ -741,6 +746,104 @@ int ikb_jacobian_host(ikb_engine *e, const void *angles, int angles_dtype, int64
         if (manip_out)
             IKB_CUDA(e, cudaMemcpyAsync((char *)manip_out + lo * w_row, s.d_in2, m * w_row, cudaMemcpyDeviceToHost,
                                         s.stream));
+    }
+    return host_end(e, stats);
+}
+
+// ---- damped-least-squares refinement --------------------------------------------------------------
+// what is wrong with the arguments, or nullptr; the engine is checked last, as for the Jacobian
+static const char *dls_bad_args(const ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n, const void *seed,
+                                int64_t n_seed, const void *angles_out, int angles_dtype, double damping, double tol,
+                                int32_t max_iter, const int32_t *iters_out, const void *err_out)
+{
+    if (n > 0 && !xyz)
+        return "NULL targets";
+    if (n > 0 && !seed)
+        return "NULL seeds";
+    if (n > 0 && !angles_out)
+        return "NULL angles_out";
+    if (n < 0)
+        return "negative n";
+    if (n_seed != 1 && n_seed != n)
+        return "n_seed must be 1 or n";
+    if (bad_dtype(xyz_dtype) || bad_dtype(angles_dtype))
+        return "unknown dtype";
+    if (!(damping > 0.0) || !std::isfinite(damping))
+        return "damping must be positive and finite";
+    if (!(tol >= 0.0))
+        return "tol must be >= 0 and not NaN";
+    if (max_iter < 0)
+        return "max_iter must be >= 0";
+    const uintptr_t a_align = esize(angles_dtype) - 1;
+    if (((uintptr_t)xyz & (esize(xyz_dtype) - 1)) || (((uintptr_t)seed | (uintptr_t)angles_out | (uintptr_t)err_out) & a_align) ||
+        ((uintptr_t)iters_out & 3))
+        return "buffers must be aligned to their element size";
+    if (n > 0) {
+        const uintptr_t row = 4 * esize(angles_dtype), s0 = (uintptr_t)seed, o0 = (uintptr_t)angles_out;
+        const bool overlap = s0 < o0 + (uintptr_t)n * row && o0 < s0 + (uintptr_t)n_seed * row;
+        if (overlap && !(s0 == o0 && n_seed == n))
+            return "seed and angles_out overlap other than in place (angles_out == seed, n_seed == n)";
+    }
+    if (!e)
+        return "NULL engine";
+    return nullptr;
+}
+
+int ikb_dls_refine_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n, const void *seed, int64_t n_seed,
+                          void *angles_out, int angles_dtype, double damping, double tol, int32_t max_iter,
+                          int32_t *iters_out, void *err_out, void *stream)
+{
+    if (const char *why = dls_bad_args(e, xyz, xyz_dtype, n, seed, n_seed, angles_out, angles_dtype, damping, tol,
+                                       max_iter, iters_out, err_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_dls_refine_device: ") + why);
+    if (n == 0)
+        return IKB_OK;
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    IKB_CUDA(e, ikb_launch_dls_refine(xyz, xyz_dtype == IKB_F64, seed, n_seed, angles_out, angles_dtype == IKB_F64,
+                                      iters_out, err_out, n, 0, damping, tol, max_iter, e->d_stats, next_counter(e),
+                                      e->rc, e->num_sms, (cudaStream_t)stream));
+    e->launches++;
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline: targets in d_in2 (24 B per slot row), seeds in d_in, angles in d_out, iterations in
+// d_aux.  The fp64 errors (8 B per row) go behind the targets in d_in2, so a chunk then holds 3 S / 4 rows (S the rows
+// of a slot), else S.  A single seed (n_seed == 1) is copied to d_in of every slot once.
+int ikb_dls_refine_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n, const void *seed, int64_t n_seed,
+                        void *angles_out, int angles_dtype, double damping, double tol, int32_t max_iter,
+                        int32_t *iters_out, void *err_out, ikb_stats *stats)
+{
+    if (const char *why = dls_bad_args(e, xyz, xyz_dtype, n, seed, n_seed, angles_out, angles_dtype, damping, tol,
+                                       max_iter, iters_out, err_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_dls_refine_host: ") + why);
+    int rc = host_begin(e, n);
+    if (rc)
+        return rc;
+    const size_t t_row = 3 * esize(xyz_dtype), a_row = 4 * esize(angles_dtype), e_row = esize(angles_dtype);
+    const long long m_max = err_out ? 3 * e->slot_rows / 4 : e->slot_rows;
+    const bool per_row_seed = n_seed != 1;
+    if (n > 0 && !per_row_seed)
+        for (int i = 0; i < kSlots; ++i)
+            IKB_CUDA(e, cudaMemcpyAsync(e->slots[i].d_in, seed, a_row, cudaMemcpyHostToDevice, e->slots[i].stream));
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        void *d_err = err_out ? (void *)((char *)s.d_in2 + 24 * m_max) : nullptr;
+        IKB_CUDA(e, cudaMemcpyAsync(s.d_in2, (const char *)xyz + lo * t_row, m * t_row, cudaMemcpyHostToDevice, s.stream));
+        if (per_row_seed)
+            IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)seed + lo * a_row, m * a_row, cudaMemcpyHostToDevice,
+                                        s.stream));
+        IKB_CUDA(e, ikb_launch_dls_refine(s.d_in2, xyz_dtype == IKB_F64, s.d_in, per_row_seed ? m : 1, s.d_out,
+                                          angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr, d_err, m, lo,
+                                          damping, tol, max_iter, e->d_stats, next_counter(e), e->rc, e->num_sms,
+                                          s.stream));
+        e->launches++;
+        IKB_CUDA(e, cudaMemcpyAsync((char *)angles_out + lo * a_row, s.d_out, m * a_row, cudaMemcpyDeviceToHost, s.stream));
+        if (iters_out)
+            IKB_CUDA(e, cudaMemcpyAsync(iters_out + lo, s.d_aux, m * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+        if (err_out)
+            IKB_CUDA(e, cudaMemcpyAsync((char *)err_out + lo * e_row, d_err, m * e_row, cudaMemcpyDeviceToHost, s.stream));
     }
     return host_end(e, stats);
 }

@@ -349,6 +349,28 @@ __device__ __forceinline__ void fk_dh_step_row(const double (&t)[4], double s, d
     }
 }
 
+// Row r of the 3 x 4 position Jacobian, for the quad lane r that carries row r of T_1..T_4 (zs[j], ps[j]: element r
+// of z_j and p_j, columns 2 and 3 of T_j, with T_0 = I; ps[4] = element r of p_4).  Column i-1 (joint i) is
+// z_{i-1} x (p_4 - p_{i-1}).  Lane r < 3 computes element r: z[r+1] * d[r+2] - z[r+2] * d[r+1] (indices mod 3: y*z' -
+// z*y' for x, ...), with the operands of the other two elements fetched from their lanes.  Every operation is
+// explicitly rounded (no contraction), so a NumPy restatement on fkine_batch's matrices reproduces the bits.  Lane 3
+// computes an unused value.  All four lanes of the quad must call it (quad shuffles).
+__device__ __forceinline__ void fk_quad_position_jacobian_row(int r, const double (&zs)[4], const double (&ps)[5],
+                                                              double (&lin)[4])
+{
+    const int r1 = r < 2 ? r + 1 : r - 2, r2 = r == 0 ? 2 : r - 1;
+    const double p4a = __shfl_sync(IKB_FULL_MASK, ps[4], r1, 4), p4b = __shfl_sync(IKB_FULL_MASK, ps[4], r2, 4);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        // z_0 = (0, 0, 1) and p_0 = 0 are constants
+        const double za = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r1, 4) : (r1 == 2 ? 1.0 : 0.0);
+        const double zb = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r2, 4) : (r2 == 2 ? 1.0 : 0.0);
+        const double pa = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r1, 4) : 0.0;
+        const double pb = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r2, 4) : 0.0;
+        lin[k] = __dsub_rn(__dmul_rn(za, __dsub_rn(p4b, pb)), __dmul_rn(zb, __dsub_rn(p4a, pa)));
+    }
+}
+
 __device__ __forceinline__ unsigned fkt_smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 
 // shared -> global 1-D bulk copy (SASS: UBLKCP); dst 16-byte aligned, bytes a multiple of 16
@@ -455,22 +477,8 @@ __global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *
         }
         ps[4] = t[3];
         if (JAC) {
-            // Column i-1 (joint i) of the position Jacobian is z_{i-1} x (p_4 - p_{i-1}).  Lane r < 3 computes element r:
-            // z[r+1] * d[r+2] - z[r+2] * d[r+1] (indices mod 3: y*z' - z*y' for x, ...), with the operands of the other
-            // two elements fetched from their lanes.  Every operation is explicitly rounded (no contraction), so a
-            // NumPy restatement on fkine_batch's matrices reproduces the bits.  Lane 3 computes an unused value.
-            const int r1 = r < 2 ? r + 1 : r - 2, r2 = r == 0 ? 2 : r - 1;
-            const double p4a = __shfl_sync(IKB_FULL_MASK, ps[4], r1, 4), p4b = __shfl_sync(IKB_FULL_MASK, ps[4], r2, 4);
             double lin[4];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                // z_0 = (0, 0, 1) and p_0 = 0 are constants
-                const double za = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r1, 4) : (r1 == 2 ? 1.0 : 0.0);
-                const double zb = k ? __shfl_sync(IKB_FULL_MASK, zs[k], r2, 4) : (r2 == 2 ? 1.0 : 0.0);
-                const double pa = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r1, 4) : 0.0;
-                const double pb = k ? __shfl_sync(IKB_FULL_MASK, ps[k], r2, 4) : 0.0;
-                lin[k] = __dsub_rn(__dmul_rn(za, __dsub_rn(p4b, pb)), __dmul_rn(zb, __dsub_rn(p4a, pa)));
-            }
+            fk_quad_position_jacobian_row(r, zs, ps, lin);
             if (MANIP) {
                 // w^2 = sum over the four 3-column subsets of det^2 (Cauchy-Binet).  Lane r takes the subset without
                 // column 3 - r: (0,1,2), (0,1,3), (0,2,3), (1,2,3) for r = 0..3, det = a . (b x c), b x c in the
@@ -546,6 +554,184 @@ __global__ void __launch_bounds__(FKT_THREADS) fk_transforms_kernel(const Real *
     }
     if (bulk && tid == 0)
         asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+}
+
+// ---- damped-least-squares refinement of joint angles onto position targets ---------------------------------------
+// One quad per row, as in fk_transforms_kernel: lane r holds joint r's angle, runs the chain with fk_dh_step_row and
+// forms the position Jacobian with fk_quad_position_jacobian_row, so p_4 and Jv are the bits of joint_positions and
+// jacobian_batch(..., "position").  After the chain every lane of the quad holds all of Jv, p_4 and e, and solves the
+// 3 x 3 damped system redundantly (explicitly rounded fp64 in the order of include/ikb200.h); lane k applies
+// Delta theta_k.  Iteration counts are bimodal (a few steps from a good seed, max_iter for a target out of reach), so
+// the warps are persistent: a quad whose row finishes stores it and takes the next row, one atomicAdd per warp and
+// trip on the work counter.  Rows finish out of order, so each quad stores its own row (one 32-B or 16-B angle row).
+struct DlsArgs {
+    const void *xyz;     // n x 3, xyz dtype
+    int xyz_f64;
+    const void *seed;    // n_seed x 4 (n_seed 1 or n), angles dtype; may equal angles_out when n_seed == n
+    long long n_seed;
+    void *angles_out;    // n x 4, angles dtype
+    int *iters;          // nullable, n
+    void *err_out;       // nullable, n (angles dtype)
+    long long n;
+    long long index_base;  // global row of row 0 (host pipeline chunks): the row numbers in the statistics
+    double lam2;         // damping^2, rounded once
+    double tol;
+    int max_iter;
+    IkbDeviceStats *stats;
+    unsigned long long *work_counter;  // zero at launch
+    IkbRobot rc;
+};
+
+constexpr int DLS_THREADS = 256;
+
+template <typename Real>
+__global__ void __launch_bounds__(DLS_THREADS) dls_refine_kernel(const DlsArgs a)
+{
+    const double TWO_PI = 6.283185307179586, PI = 3.141592653589793;
+    const int lane = threadIdx.x & 31, r = lane & 3;
+    const unsigned quads_below = (1u << (lane & ~3)) - 1u;  // lanes of the lower quads of this warp
+    const bool alpha_bad = a.rc.alpha[r] < -TWO_PI || a.rc.alpha[r] > TWO_PI;
+    double th = 0.0, tx = 0.0, ty = 0.0, tz = 0.0;
+    long long row = 0;
+    int k = 0;
+    bool live = false, exhausted = false;
+    unsigned long long n_solved = 0, sum_k = 0, capped = 0, n_err = 0;
+    double err_sum = 0.0;
+    long long first_limits = IKB_I64_MAX, first_range = IKB_I64_MAX;
+    for (;;) {
+        if (!exhausted) {  // refill: every quad without a row takes the next one
+            const unsigned want = __ballot_sync(IKB_FULL_MASK, !live) & 0x11111111u;  // lane 0 of each idle quad
+            if (want) {
+                unsigned long long base = 0;
+                if (lane == 0)
+                    base = atomicAdd(a.work_counter, (unsigned long long)__popc(want));
+                base = __shfl_sync(IKB_FULL_MASK, base, 0);
+                if (!live) {
+                    const long long rw = (long long)base + __popc(want & quads_below);
+                    if (rw < a.n) {
+                        row = rw;
+                        k = 0;
+                        live = true;
+                        // plain loads: seed may be angles_out (in place), whose rows other quads are writing
+                        th = (double)reinterpret_cast<const Real *>(a.seed)[4 * (a.n_seed == 1 ? 0 : rw) + r];
+                        ikb_load_xyz(a.xyz, a.xyz_f64, rw, tx, ty, tz);
+                        // the guards of fk_transforms_kernel (angles) and K0 (targets); NaN passes both
+                        if (th < -TWO_PI || th > TWO_PI || alpha_bad)
+                            first_range = min(first_range, a.index_base + rw);
+                        if (ikb_out_of_limits(a.rc, tx, ty, tz))
+                            first_limits = min(first_limits, a.index_base + rw);
+                    }
+                }
+                exhausted = (long long)(base + __popc(want)) >= a.n;
+            }
+        }
+        if (__ballot_sync(IKB_FULL_MASK, live) == 0)
+            break;
+        // the chain, at full warp width (quads without a row compute on stale registers and write nothing)
+        double s, c;
+        sincos(th, &s, &c);
+        double t[4] = {r == 0 ? 1.0 : 0.0, r == 1 ? 1.0 : 0.0, r == 2 ? 1.0 : 0.0, r == 3 ? 1.0 : 0.0};
+        double zs[4], ps[5];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double sj = __shfl_sync(IKB_FULL_MASK, s, j, 4), cj = __shfl_sync(IKB_FULL_MASK, c, j, 4);
+            double nr[4];
+            zs[j] = t[2];
+            ps[j] = t[3];
+            fk_dh_step_row(t, sj, cj, a.rc.cos_alpha[j], a.rc.sin_alpha[j], a.rc.a[j], a.rc.eps[j], nr);
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+                t[q] = nr[q];
+        }
+        ps[4] = t[3];
+        double lin[4];
+        fk_quad_position_jacobian_row(r, zs, ps, lin);
+        double J[3][4];
+#pragma unroll
+        for (int q = 0; q < 3; ++q)
+#pragma unroll
+            for (int m = 0; m < 4; ++m)
+                J[q][m] = __shfl_sync(IKB_FULL_MASK, lin[m], q, 4);
+        const double ex = __dsub_rn(tx, __shfl_sync(IKB_FULL_MASK, ps[4], 0, 4));
+        const double ey = __dsub_rn(ty, __shfl_sync(IKB_FULL_MASK, ps[4], 1, 4));
+        const double ez = __dsub_rn(tz, __shfl_sync(IKB_FULL_MASK, ps[4], 2, 4));
+        const double err = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)), __dmul_rn(ez, ez)));
+        if (live && (err <= a.tol || k >= a.max_iter)) {  // quad-uniform: every lane holds the same err and k
+            const long long o = 4 * row + r;
+            reinterpret_cast<Real *>(a.angles_out)[o] = (Real)th;
+            if (r == 0) {
+                if (a.iters)
+                    a.iters[row] = k;
+                if (a.err_out)
+                    reinterpret_cast<Real *>(a.err_out)[row] = (Real)err;
+                ++n_solved;
+                sum_k += (unsigned)k;
+                capped += err <= a.tol ? 0u : 1u;  // NaN rows included
+                if (isfinite(err)) {
+                    err_sum += err;
+                    ++n_err;
+                }
+            }
+            live = false;
+        }
+        if (live) {
+            // A = Jv Jv^T + lambda^2 I, element (i, j) summed as (j0 + j1) + (j2 + j3)
+            double A[3][3];
+#pragma unroll
+            for (int i = 0; i < 3; ++i)
+#pragma unroll
+                for (int j = i; j < 3; ++j)
+                    A[i][j] = __dadd_rn(__dadd_rn(__dmul_rn(J[i][0], J[j][0]), __dmul_rn(J[i][1], J[j][1])),
+                                        __dadd_rn(__dmul_rn(J[i][2], J[j][2]), __dmul_rn(J[i][3], J[j][3])));
+#pragma unroll
+            for (int i = 0; i < 3; ++i)
+                A[i][i] = __dadd_rn(A[i][i], a.lam2);
+            // A y = e by LDL^T (no square root)
+            const double l10 = __ddiv_rn(A[0][1], A[0][0]), l20 = __ddiv_rn(A[0][2], A[0][0]);
+            const double d1 = __dsub_rn(A[1][1], __dmul_rn(l10, A[0][1]));
+            const double t12 = __dsub_rn(A[1][2], __dmul_rn(l20, A[0][1]));
+            const double l21 = __ddiv_rn(t12, d1);
+            const double d2 = __dsub_rn(__dsub_rn(A[2][2], __dmul_rn(l20, A[0][2])), __dmul_rn(l21, t12));
+            const double z1 = __dsub_rn(ey, __dmul_rn(l10, ex));
+            const double z2 = __dsub_rn(__dsub_rn(ez, __dmul_rn(l20, ex)), __dmul_rn(l21, z1));
+            const double y2 = __ddiv_rn(z2, d2);
+            const double y1 = __dsub_rn(__ddiv_rn(z1, d1), __dmul_rn(l21, y2));
+            const double y0 = __dsub_rn(__dsub_rn(__ddiv_rn(ex, A[0][0]), __dmul_rn(l10, y1)), __dmul_rn(l20, y2));
+            // lane k: column k of Jv
+            const double c0 = r == 0 ? J[0][0] : r == 1 ? J[0][1] : r == 2 ? J[0][2] : J[0][3];
+            const double c1 = r == 0 ? J[1][0] : r == 1 ? J[1][1] : r == 2 ? J[1][2] : J[1][3];
+            const double c2 = r == 0 ? J[2][0] : r == 1 ? J[2][1] : r == 2 ? J[2][2] : J[2][3];
+            th = __dadd_rn(th, __dadd_rn(__dadd_rn(__dmul_rn(c0, y0), __dmul_rn(c1, y1)), __dmul_rn(c2, y2)));
+            if (fabs(th) > PI)
+                th = remainder(th, TWO_PI);  // exact: the angle stays inside the FK guard
+            ++k;
+        }
+    }
+    // statistics: one atomic per warp and counter (lane 0 of each quad counted its rows)
+    n_solved = ikb_warp_sum(n_solved);
+    sum_k = ikb_warp_sum(sum_k);
+    capped = ikb_warp_sum(capped);
+    n_err = ikb_warp_sum(n_err);
+    err_sum = ikb_warp_sum(err_sum);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        first_limits = min(first_limits, __shfl_xor_sync(IKB_FULL_MASK, first_limits, o));
+        first_range = min(first_range, __shfl_xor_sync(IKB_FULL_MASK, first_range, o));
+    }
+    if (lane == 0 && n_solved != 0) {
+        atomicAdd(&a.stats->n_solved, n_solved);
+        atomicAdd(&a.stats->sum_iterations, sum_k);
+        if (capped)
+            atomicAdd(&a.stats->n_iter_capped, capped);
+        if (n_err) {
+            atomicAdd(&a.stats->sum_fk_error, err_sum);
+            atomicAdd(&a.stats->n_fk_error, n_err);
+        }
+        if (first_limits != IKB_I64_MAX)
+            atomicMin(&a.stats->first_out_of_limits, first_limits);
+        if (first_range != IKB_I64_MAX)
+            atomicMin(&a.stats->first_fk_angle_range, first_range);
+    }
 }
 
 struct LimitsArgs {
@@ -750,6 +936,38 @@ cudaError_t ikb_launch_jacobian(const void *angles, int angles_f64, long long n,
     const bool geometric = what == IKB_JAC_GEOMETRIC;
     return angles_f64 ? launch_jacobian<double>(angles, n, index_base, geometric, jac, manip, stats, rc, num_sms, stream)
                       : launch_jacobian<float>(angles, n, index_base, geometric, jac, manip, stats, rc, num_sms, stream);
+}
+
+// damped-least-squares refinement (ikb_dls_refine_*); work_counter: a counter of the engine's ring (reset here)
+cudaError_t ikb_launch_dls_refine(const void *xyz, int xyz_f64, const void *seed, long long n_seed, void *angles_out,
+                                  int angles_f64, int *iters, void *err_out, long long n, long long index_base,
+                                  double damping, double tol, int max_iter, IkbDeviceStats *stats,
+                                  unsigned long long *work_counter, const IkbRobot &rc, int num_sms,
+                                  cudaStream_t stream)
+{
+    if (n <= 0)
+        return cudaSuccess;
+    DlsArgs a;
+    a.xyz = xyz; a.xyz_f64 = xyz_f64; a.seed = seed; a.n_seed = n_seed; a.angles_out = angles_out;
+    a.iters = iters; a.err_out = err_out; a.n = n; a.index_base = index_base;
+    a.lam2 = damping * damping; a.tol = tol; a.max_iter = max_iter;
+    a.stats = stats; a.work_counter = work_counter; a.rc = rc;
+    void (*kern)(DlsArgs) = angles_f64 ? dls_refine_kernel<double> : dls_refine_kernel<float>;
+    static int blocks_per_sm[2] = {};
+    int &bps = blocks_per_sm[angles_f64 ? 1 : 0];
+    if (bps == 0) {
+        cudaError_t err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, DLS_THREADS, 0);
+        if (err != cudaSuccess)
+            return err;
+        bps = bps > 0 ? bps : 1;
+    }
+    cudaError_t err = cudaMemsetAsync(work_counter, 0, sizeof(unsigned long long), stream);
+    if (err != cudaSuccess)
+        return err;
+    // persistent grid: resident CTAs per SM x SM count, trimmed for small batches (one quad per row)
+    const long long want = (n + DLS_THREADS / 4 - 1) / (DLS_THREADS / 4), cap = (long long)num_sms * bps;
+    kern<<<(unsigned)(want < cap ? want : cap), DLS_THREADS, 0, stream>>>(a);
+    return cudaGetLastError();
 }
 
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,

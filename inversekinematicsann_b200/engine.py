@@ -319,6 +319,49 @@ class IkEngine:
             IkEngine._check_out(out, angles.shape[0], tail, (angles.dtype,), "out")
         return angles, code, out
 
+    def dls_refine(self, xyz, seed, damping=None, tol=None, max_iter=None, out=None, return_iters=False,
+                   return_error=False):
+        """Damped-least-squares refinement of joint angles onto (n, 3) targets (include/ikb200.h ikb_dls_refine_*):
+        seed (n, 4), or one row (4,) / (1, 4) for every target, float32 or float64; the result has the seeds' dtype and
+        may be written in place (out=seed).  Defaults: DLS_DAMPING, DLS_TOL, DLS_MAX_ITER.  Returns
+        (angles[n,4], stats[, iters int32 [n]][, error [n]]); stats.first_out_of_limits / first_fk_angle_range >= 0
+        mark the lowest out-of-box target and the lowest seed with an angle outside [-2pi, 2pi]."""
+        xyz, seed, n_seed, out = self._dls_args(xyz, seed, out)
+        n = xyz.shape[0]
+        damping, tol, max_iter = _dls_params(damping, tol, max_iter)
+        iters = np.empty(n, dtype=np.int32) if return_iters else None
+        err = np.empty(n, dtype=out.dtype) if return_error else None
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_dls_refine_host(
+            self._handle, xyz.ctypes.data, _np_dtype_code(xyz), n, seed.ctypes.data, n_seed, out.ctypes.data,
+            _np_dtype_code(out), damping, tol, max_iter, iters.ctypes.data if return_iters else None,
+            err.ctypes.data if return_error else None, ctypes.byref(s)), "ikb_dls_refine_host")
+        res = (out, IkStats.from_c(s))
+        if return_iters:
+            res += (iters,)
+        if return_error:
+            res += (err,)
+        return res
+
+    @staticmethod
+    def _dls_args(xyz, seed, out):
+        """The checks of `dls_refine` that need no device -> (xyz, seed (n_seed, 4), n_seed, out)."""
+        xyz = IkEngine._rows(xyz, 3, "points")
+        n = xyz.shape[0]
+        if out is not None and out is seed:  # in place: the seeds must already be the buffer the library writes
+            IkEngine._check_out(out, n, 4, (np.float32, np.float64), "out")
+            return xyz, seed, n, out
+        seed = np.asarray(seed)
+        if seed.ndim == 1:
+            seed = seed.reshape(1, -1)
+        seed = IkEngine._rows(seed, 4, "seed")
+        if seed.shape[0] not in (1, n):
+            raise ValueError(f"seed must have 1 or {n} rows, got {seed.shape[0]}")
+        if out is None:
+            out = np.empty((n, 4), dtype=seed.dtype)
+        IkEngine._check_out(out, n, 4, (seed.dtype,), "out")
+        return xyz, seed, seed.shape[0], out
+
     def mlp_load(self, weights, biases, mean_x, scale_x, mean_y, scale_y):
         """reference ann.py:78-85: upload Keras Dense kernels (in, out) + biases and both scalers."""
         ws = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
@@ -532,6 +575,35 @@ class IkEngine:
                                                   manip.data_ptr() if manip is not None else None,
                                                   _torch_stream_ptr(self.device)), "ikb_jacobian_device")
 
+    def dls_refine_device(self, xyz, seed, out, iters=None, err=None, damping=None, tol=None, max_iter=None):
+        """dls_refine on CUDA tensors of this engine's device, enqueued on torch's current stream (no
+        synchronisation): xyz (n, 3); seed (n, 4), or (1, 4) / (4,) for every row, float32 or float64; out (n, 4) in
+        the seeds' dtype (out may be seed: in place); iters int32 (n,) and err (n,) in the seeds' dtype, or None.  The
+        guards and statistics accumulate in the engine's block (stats_fetch_torch)."""
+        xyz = self._dev_rows(xyz, 3, "points")
+        n = xyz.shape[0]
+        if _is_torch_tensor(seed) and seed.dim() == 1:
+            seed = seed.view(1, -1)
+        seed = self._dev_rows(seed, 4, "seed")
+        if seed.shape[0] not in (1, n):
+            raise ValueError(f"seed must have 1 or {n} rows, got {seed.shape[0]}")
+        _torch_dtype_code(seed)
+        out = self._dev_rows(out, 4, "angles")
+        self._same_rows(xyz, out, "angles")
+        if out.dtype != seed.dtype:
+            raise TypeError(f"angles must have the seeds' dtype {seed.dtype}, got {out.dtype}")
+        if iters is not None:
+            self._dev_vec(iters, n, "torch.int32", "iters")
+        if err is not None:
+            self._dev_vec(err, n, str(seed.dtype), "err")
+        damping, tol, max_iter = _dls_params(damping, tol, max_iter)
+        if n == 0:  # nothing to do, and an empty tensor's data_ptr() may be NULL
+            return
+        self._check(self._lib.ikb_dls_refine_device(
+            self._handle, xyz.data_ptr(), _torch_dtype_code(xyz), n, seed.data_ptr(), seed.shape[0], out.data_ptr(),
+            _torch_dtype_code(out), damping, tol, max_iter, iters.data_ptr() if iters is not None else None,
+            err.data_ptr() if err is not None else None, _torch_stream_ptr(self.device)), "ikb_dls_refine_device")
+
     def check_limits_device(self, xyz):
         xyz = self._dev_rows(xyz, 3, "points")
         self._check(self._lib.ikb_check_limits_device(self._handle, xyz.data_ptr(), _torch_dtype_code(xyz),
@@ -588,6 +660,21 @@ _FK_LAYOUTS = {"matrices": _native.IKB_FK_MATRICES, "joints": _native.IKB_FK_JOI
 _FK_TAIL = {_native.IKB_FK_MATRICES: (4, 4, 4), _native.IKB_FK_JOINTS: (4, 3)}  # per-row shape of each layout
 _JAC_LAYOUTS = {"geometric": _native.IKB_JAC_GEOMETRIC, "position": _native.IKB_JAC_POSITION}
 _JAC_TAIL = {_native.IKB_JAC_GEOMETRIC: (6, 4), _native.IKB_JAC_POSITION: (3, 4)}
+
+
+# defaults of the damped-least-squares refinement, chosen from the damping sweep of profiles/r06_dls_bench.json
+# (DESIGN.md §5): from 0.5 m down to 0.005 m every seed kind needs fewer steps, and at 0.005 m every FABRIK- and
+# ANN-seeded reachable row converged to 1e-9 m within 23 / 41 steps; 64 steps also cover the stretched-arm seed past
+# its 99.9th percentile (56).  Out-of-reach rows always take max_iter steps, so it is not larger.
+DLS_DAMPING = 0.005  # lambda, metres (the links are 2 m)
+DLS_TOL = 1e-9       # metres
+DLS_MAX_ITER = 64
+
+
+def _dls_params(damping, tol, max_iter):
+    """None -> the defaults; the library checks the values (each refusal has its own message)."""
+    return (float(DLS_DAMPING if damping is None else damping), float(DLS_TOL if tol is None else tol),
+            int(DLS_MAX_ITER if max_iter is None else max_iter))
 
 
 def _choice(table, key, what):

@@ -16,10 +16,11 @@ from abc import ABC, abstractmethod
 
 import numpy as np
 
+from ..engine import DLS_DAMPING, DLS_MAX_ITER, DLS_TOL
 from ..robot.robot import OutOfRobotReachException
 from ._shared import get_engine, points_to_array
 from .ann import ANN
-from .forward import ForwardKinematics
+from .forward import _ANGLE_MSG, ForwardKinematics
 
 
 class InverseKinematics(ABC):
@@ -67,6 +68,54 @@ class InverseKinematics(ABC):
     @abstractmethod
     def ikine(self, dest_points):
         """Calculate inverse kinematics"""
+
+    def refine(self, dest_points, angles, damping=DLS_DAMPING, tol=DLS_TOL, max_iter=DLS_MAX_ITER, as_array=False,
+               return_iterations=False, return_fk_error=False):
+        """Refine joint angles onto the destination points by damped least squares on the GPU: from `angles` (one row
+        per point, or one row for all of them; e.g. what `ikine` returned), each row repeats
+        Delta theta = Jv^T (Jv Jv^T + damping^2 I)^-1 (point - FK(theta)) until ||FK(theta) - point|| <= tol or
+        `max_iter` steps (include/ikb200.h ikb_dls_refine_* states the arithmetic).  The angles come back wrapped to
+        [-pi, pi] where a step left that range.
+
+        The result has the seeds' dtype: a list gives float64, a float32 array float32.  The network's float32
+        predictions should be widened (``angles.astype(np.float64)``) to refine below about 1e-6 m, since float32
+        angles cannot resolve the effector more finely than that.  Return shapes follow `ikine`: a list of rows, or an
+        (n, 4) array with `as_array`, then the step counts (`return_iterations`) and ||FK(theta) - point||
+        (`return_fk_error`).  A point outside the workspace box raises OutOfRobotReachException with `ikine`'s message
+        (checked first), a seed angle outside [-2pi, 2pi] with the forward-kinematics one."""
+        arr = points_to_array(dest_points)
+        seed = angles if isinstance(angles, np.ndarray) and angles.dtype in (np.float32, np.float64) else \
+            np.asarray(angles, dtype=np.float64)
+        if arr.shape[0] == 0:
+            empty = np.zeros((0, 4), dtype=seed.dtype)
+            empty = empty if as_array else []
+            extras = ((np.zeros(0, np.int32),) if return_iterations else ()) + \
+                     ((np.zeros(0, seed.dtype),) if return_fk_error else ())
+            return (empty,) + extras if extras else empty
+        res = self._engine().dls_refine(arr, seed, damping, tol, max_iter, return_iters=return_iterations,
+                                        return_error=return_fk_error)
+        out, stats = res[0], res[1]
+        self.last_stats = stats
+        if stats.first_out_of_limits >= 0:
+            raise self._limits_error(dest_points, stats.first_out_of_limits)
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+        out = out if as_array else out.tolist()
+        return (out,) + tuple(res[2:]) if len(res) > 2 else out
+
+    def refine_device(self, points, angles, out=None, iters=None, fk_err=None, damping=DLS_DAMPING, tol=DLS_TOL,
+                      max_iter=DLS_MAX_ITER):
+        """`refine` on CUDA tensors, enqueued on torch's current stream without a synchronisation: points (n, 3),
+        angles (n, 4) or one row for all points, float32 or float64; out (n, 4) in the angles' dtype is allocated when
+        None and may be `angles` itself (in place), so ``ann_solve_device`` -> ``refine_device(..., out=angles)``
+        needs no host round trip.  iters (int32) and fk_err (angles' dtype), when given, receive the step counts and
+        the final errors.  Returns out.  The guards set first_out_of_limits / first_fk_angle_range of the engine's
+        statistics (``stats_fetch_torch``) instead of raising."""
+        import torch
+        if out is None:
+            out = torch.empty((points.shape[0], 4), dtype=angles.dtype, device=angles.device)
+        self._engine().dls_refine_device(points, angles, out, iters, fk_err, damping, tol, max_iter)
+        return out
 
 
 class FabrikInverseKinematics(InverseKinematics):
