@@ -16,7 +16,9 @@
  *   - *_device entry points take DEVICE pointers, enqueue on `stream` (a cudaStream_t passed as
  *     void*, NULL = the legacy default stream) and return without synchronising; per-call
  *     diagnostics accumulate in the engine's device-side statistics block, read with
- *     ikb_stats_fetch().
+ *     ikb_stats_fetch().  Calls on different streams may overlap (the engine orders only launches
+ *     that would share one of its work counters); the statistics block is engine-wide and sums
+ *     over them.
  *   - *_host entry points take HOST pointers (pinned or pageable), run a chunked
  *     H2D -> kernel -> D2H pipeline on the engine's own streams, synchronise, and fill `stats`.
  *   - The reference's whole-batch exception semantics (inverse.py:117: check_limits raises before

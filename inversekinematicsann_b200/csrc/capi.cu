@@ -85,7 +85,8 @@ struct ikb_engine {
     int num_sms = 0;
     IkbDeviceStats *d_stats = nullptr;
     IkbDeviceStats *h_stats = nullptr;  // pinned
-    unsigned long long *d_counters = nullptr;
+    unsigned long long *d_counters = nullptr;     // kCounterRing work counters of the persistent kernels
+    cudaEvent_t counter_free[kCounterRing] = {};  // recorded after the last launch that used each counter
     int counter_seq = 0;
     Slot slots[kSlots];
     long long slot_rows = 0;  // current capacity of every slot buffer, grows on demand
@@ -136,11 +137,21 @@ void to_public(const IkbDeviceStats &d, ikb_stats *o)
     o->n_fk_error = (int64_t)d.n_fk_error;
 }
 
-unsigned long long *next_counter(ikb_engine *e)
+// The work counter of the next persistent launch, taken round-robin from the engine's ring.  Launches on different
+// streams may overlap, so a counter is only handed out once the last launch that used it has finished: `stream` first
+// waits for that launch's event (a no-op for an event that was never recorded).  After the launch, call
+// counter_release(e, slot, stream) with the slot returned here.
+cudaError_t counter_claim(ikb_engine *e, cudaStream_t stream, unsigned long long **counter, int *slot)
 {
-    unsigned long long *p = e->d_counters + 2 * (e->counter_seq % kCounterRing);  // pairs: lane-refill + far kernel
+    *slot = e->counter_seq % kCounterRing;
     e->counter_seq++;
-    return p;
+    *counter = e->d_counters + *slot;
+    return cudaStreamWaitEvent(stream, e->counter_free[*slot], 0);
+}
+
+cudaError_t counter_release(ikb_engine *e, int slot, cudaStream_t stream)
+{
+    return cudaEventRecord(e->counter_free[slot], stream);
 }
 
 // staging buffers of the host pipelines: sized for min(rows, kHostChunkRows), grown on demand
@@ -251,7 +262,9 @@ int ikb_engine_create(const ikb_config *cfg, ikb_engine **out)
     e->num_sms = prop.multiProcessorCount;
     IKB_CREATE_CUDA(cudaMalloc(&e->d_stats, sizeof(IkbDeviceStats)));
     IKB_CREATE_CUDA(cudaMallocHost(&e->h_stats, sizeof(IkbDeviceStats)));
-    IKB_CREATE_CUDA(cudaMalloc(&e->d_counters, 2 * kCounterRing * sizeof(unsigned long long)));
+    IKB_CREATE_CUDA(cudaMalloc(&e->d_counters, kCounterRing * sizeof(unsigned long long)));
+    for (int i = 0; i < kCounterRing; ++i)
+        IKB_CREATE_CUDA(cudaEventCreateWithFlags(&e->counter_free[i], cudaEventDisableTiming));
     *e->h_stats = fresh_stats();
     IKB_CREATE_CUDA(cudaMemcpy(e->d_stats, e->h_stats, sizeof(IkbDeviceStats), cudaMemcpyHostToDevice));
 
@@ -348,6 +361,8 @@ void ikb_engine_destroy(ikb_engine *e)
     if (e->d_stats) cudaFree(e->d_stats);
     if (e->h_stats) cudaFreeHost(e->h_stats);
     if (e->d_counters) cudaFree(e->d_counters);
+    for (int i = 0; i < kCounterRing; ++i)
+        if (e->counter_free[i]) cudaEventDestroy(e->counter_free[i]);
     delete e;
 }
 
@@ -440,14 +455,19 @@ int ikb_fabrik_solve_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64
     IKB_CUDA(e, cudaSetDevice(e->device));
     const bool want_fk = n > 0 && (fk_err_out || fk_stats);
     const bool fuse = want_fk && e->rc.planar && fk_fusable(e->rc, n);
-    if (!e->rc.planar)  // general DH table: the seed chain leaves the vertical plane -> 3-D kernel
+    if (!e->rc.planar) {  // general DH table: the seed chain leaves the vertical plane -> 3-D kernel
         IKB_CUDA(e, ikb_launch_fabrik_generic_ikine(xyz, xyz_dtype == IKB_F64, n, 0, angles_out,
                                                     angles_dtype == IKB_F64, iters_out, e->d_stats, e->rc,
                                                     (cudaStream_t)stream));
-    else
+    } else {
+        unsigned long long *counter;
+        int slot;
+        IKB_CUDA(e, counter_claim(e, (cudaStream_t)stream, &counter, &slot));
         IKB_CUDA(e, ikb_launch_fabrik_planar(xyz, xyz_dtype == IKB_F64, n, 0, angles_out, angles_dtype == IKB_F64,
                                              iters_out, fuse ? fk_err_out : nullptr, fuse ? fk_stats : 0, precision,
-                                             e->d_stats, next_counter(e), e->rc, e->num_sms, (cudaStream_t)stream));
+                                             e->d_stats, counter, e->rc, e->num_sms, (cudaStream_t)stream));
+        IKB_CUDA(e, counter_release(e, slot, (cudaStream_t)stream));
+    }
     if (want_fk && !fuse) {  // no closed-form FK for this DH table: K3 as a second launch
         IKB_CUDA(e, ikb_launch_fk(angles_out, angles_dtype == IKB_F64, n, 0, nullptr, xyz, xyz_dtype == IKB_F64,
                                   fk_err_out, e->d_stats, e->rc, e->num_sms, (cudaStream_t)stream));
@@ -476,15 +496,20 @@ int ikb_fabrik_solve_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t
         m = host_chunk_rows(lo, n);
         void *d_err = fk_err_out ? s.d_in2 : nullptr;  // d_in2 is free here (FK targets only)
         IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)xyz + lo * in_row, m * in_row, cudaMemcpyHostToDevice, s.stream));
-        if (!e->rc.planar)
+        if (!e->rc.planar) {
             IKB_CUDA(e, ikb_launch_fabrik_generic_ikine(s.d_in, xyz_dtype == IKB_F64, m, lo, s.d_out,
                                                         angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr,
                                                         e->d_stats, e->rc, s.stream));
-        else
+        } else {
+            unsigned long long *counter;
+            int slot;
+            IKB_CUDA(e, counter_claim(e, s.stream, &counter, &slot));
             IKB_CUDA(e, ikb_launch_fabrik_planar(s.d_in, xyz_dtype == IKB_F64, m, lo, s.d_out,
                                                  angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr,
                                                  fuse ? d_err : nullptr, fuse ? fk_stats : 0, precision, e->d_stats,
-                                                 next_counter(e), e->rc, e->num_sms, s.stream));
+                                                 counter, e->rc, e->num_sms, s.stream));
+            IKB_CUDA(e, counter_release(e, slot, s.stream));
+        }
         if (want_fk && !fuse) {
             IKB_CUDA(e, ikb_launch_fk(s.d_out, angles_dtype == IKB_F64, m, lo, nullptr, s.d_in, xyz_dtype == IKB_F64,
                                       d_err, e->d_stats, e->rc, e->num_sms, s.stream));
@@ -522,8 +547,12 @@ int ikb_fabrik_chain_device(ikb_engine *e, int32_t n_points, const double *links
     if (rc)
         return rc;
     IKB_CUDA(e, cudaSetDevice(e->device));
+    unsigned long long *counter;
+    int slot;
+    IKB_CUDA(e, counter_claim(e, (cudaStream_t)stream, &counter, &slot));
     IKB_CUDA(e, ikb_launch_fabrik_chain(n_points, links, tol, max_iter, init, n_init, goals, n, 0, chain_out, iters_out,
-                                        e->d_stats, next_counter(e), e->num_sms, (cudaStream_t)stream));
+                                        e->d_stats, counter, e->num_sms, (cudaStream_t)stream));
+    IKB_CUDA(e, counter_release(e, slot, (cudaStream_t)stream));
     e->launches += (n > 0);
     return IKB_OK;
 }
@@ -557,9 +586,13 @@ int ikb_fabrik_chain_host(ikb_engine *e, int32_t n_points, const double *links, 
             IKB_CUDA(e, cudaMemcpyAsync(d_init, init + lo * row_doubles, m * row_doubles * sizeof(double),
                                         cudaMemcpyHostToDevice, s.stream));
         IKB_CUDA(e, cudaMemcpyAsync(d_goals, goals + 3 * lo, m * 3 * sizeof(double), cudaMemcpyHostToDevice, s.stream));
+        unsigned long long *counter;
+        int slot;
+        IKB_CUDA(e, counter_claim(e, s.stream, &counter, &slot));
         IKB_CUDA(e, ikb_launch_fabrik_chain(n_points, links, tol, max_iter, d_init, per_row_init ? m : 1, d_goals, m, lo,
-                                            d_chain, iters_out ? s.d_aux : nullptr, e->d_stats, next_counter(e),
-                                            e->num_sms, s.stream));
+                                            d_chain, iters_out ? s.d_aux : nullptr, e->d_stats, counter, e->num_sms,
+                                            s.stream));
+        IKB_CUDA(e, counter_release(e, slot, s.stream));
         e->launches++;
         IKB_CUDA(e, cudaMemcpyAsync(chain_out + lo * row_doubles, d_chain, m * row_doubles * sizeof(double),
                                     cudaMemcpyDeviceToHost, s.stream));
@@ -799,9 +832,13 @@ int ikb_dls_refine_device(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t
     if (n == 0)
         return IKB_OK;
     IKB_CUDA(e, cudaSetDevice(e->device));
+    unsigned long long *counter;
+    int slot;
+    IKB_CUDA(e, counter_claim(e, (cudaStream_t)stream, &counter, &slot));
     IKB_CUDA(e, ikb_launch_dls_refine(xyz, xyz_dtype == IKB_F64, seed, n_seed, angles_out, angles_dtype == IKB_F64,
-                                      iters_out, err_out, n, 0, damping, tol, max_iter, e->d_stats, next_counter(e),
-                                      e->rc, e->num_sms, (cudaStream_t)stream));
+                                      iters_out, err_out, n, 0, damping, tol, max_iter, e->d_stats, counter, e->rc,
+                                      e->num_sms, (cudaStream_t)stream));
+    IKB_CUDA(e, counter_release(e, slot, (cudaStream_t)stream));
     e->launches++;
     return IKB_OK;
 }
@@ -834,10 +871,13 @@ int ikb_dls_refine_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n
         if (per_row_seed)
             IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)seed + lo * a_row, m * a_row, cudaMemcpyHostToDevice,
                                         s.stream));
+        unsigned long long *counter;
+        int slot;
+        IKB_CUDA(e, counter_claim(e, s.stream, &counter, &slot));
         IKB_CUDA(e, ikb_launch_dls_refine(s.d_in2, xyz_dtype == IKB_F64, s.d_in, per_row_seed ? m : 1, s.d_out,
                                           angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr, d_err, m, lo,
-                                          damping, tol, max_iter, e->d_stats, next_counter(e), e->rc, e->num_sms,
-                                          s.stream));
+                                          damping, tol, max_iter, e->d_stats, counter, e->rc, e->num_sms, s.stream));
+        IKB_CUDA(e, counter_release(e, slot, s.stream));
         e->launches++;
         IKB_CUDA(e, cudaMemcpyAsync((char *)angles_out + lo * a_row, s.d_out, m * a_row, cudaMemcpyDeviceToHost, s.stream));
         if (iters_out)

@@ -439,6 +439,9 @@ class IkEngine:
             "ikb_copy_pipeline_host")
 
     # ---- device-buffer entry points (torch CUDA tensors; async on torch's current stream) ---------
+    # Each call is enqueued on torch's current stream and ordered after the work already there.  Calls on different
+    # streams may overlap: the library orders only the launches that would share one of its work counters.  The
+    # statistics block is engine-wide, so it sums over the calls of every stream since the last stats_reset.
     def _dev_rows(self, t, cols, what):
         if not _is_torch_tensor(t) or not t.is_cuda:
             raise TypeError(f"{what} must be a CUDA torch tensor")
