@@ -262,7 +262,63 @@ int ikb_dls_refine_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n
                         int32_t *iters_out /* nullable */, void *err_out /* nullable, angles_dtype */,
                         ikb_stats *stats);
 
-/* ---- ANN (ann.py:70-85, inverse.py:142-155) -------------------------------------------------- */
+/* Damped-least-squares refinement of joint angles onto full effector poses (position and orientation), weighted per
+ * task axis: from a seed, every row repeats Delta theta = (J^T W J + lambda^2 I)^-1 J^T W e, J the 6 x 4 geometric
+ * Jacobian, W = diag(weights), until it meets its own tolerance.  The arm has 4 joints and a pose 6 components, so a
+ * pose that is not the FK of some angles is generally not reachable; the weights decide what is matched then.
+ *   poses: n x 4 x 4 of pose_dtype, row-major, the layout of one matrix of ikb_fk_transforms_* (IKB_FK_MATRICES): rows
+ *   0-2 hold [R_d | p_d], row 3 is not read.  weights: 6 HOST doubles, the position axes x, y, z then the three
+ *   orientation axes, each >= 0 and finite, not all zero.  damping = lambda (joint space: A's unit is that of J^T W J),
+ *   tol >= 0 on err below.  Everything else -- seeds, n_seed, in place, iters_out, err_out (angles_dtype), max_iter = 0
+ *   returning the seeds with their errors -- is as for ikb_dls_refine_*.
+ * The arithmetic is fp64 (float32 seeds and poses are widened exactly; a float32 output is the fp64 result rounded
+ * once).  R, p = T_4 of an iterate are the bits of ikb_fk_transforms_* (IKB_FK_MATRICES) and J those of
+ * ikb_jacobian_* (IKB_JAC_GEOMETRIC) for it.  Every later operation is IEEE fp64 with round-to-nearest and no
+ * contraction (sqrt correctly rounded).  Per row, with k = 0:
+ *   1. e_p = p_d - p.  M = R_d R^T: M_ij = (Rd_i0*R_j0 + Rd_i1*R_j1) + Rd_i2*R_j2.  tr = (M00 + M11) + M22;
+ *      dx = M21 - M12, dy = M02 - M20, dz = M10 - M01.  e_o = 2 x the vector part of M's unit quaternion with a
+ *      non-negative scalar part (Shepperd), zero only for no rotation, so a row 180 degrees off is not converged:
+ *        tr >= M00, tr >= M11 and tr >= M22:  h = sqrt(1 + tr);  e_o = (dx/h, dy/h, dz/h)
+ *        else M00 >= M11 and M00 >= M22:     h = sqrt(((1 + M00) - M11) - M22);
+ *                                            e_o = (h, (M01 + M10)/h, (M02 + M20)/h), negated when dx < 0
+ *        else M11 >= M22:                    h = sqrt(((1 + M11) - M00) - M22);
+ *                                            e_o = ((M01 + M10)/h, h, (M12 + M21)/h), negated when dy < 0
+ *        else:                               h = sqrt(((1 + M22) - M00) - M11);
+ *                                            e_o = ((M02 + M20)/h, (M12 + M21)/h, h), negated when dz < 0
+ *      e = (e_p, e_o), s_i = w_i*(e_i*e_i);  err = sqrt(((s0 + s1) + s2) + ((s3 + s4) + s5))
+ *   2. err <= tol: stop (converged).   3. k == max_iter: stop (not converged; NaN rows end here).
+ *   4. For task rows q = 0..5 (J_q: row q of J): g_q = w_q*J_q elementwise.  For i = 0, 1, 2, pairing linear row i
+ *      with angular row 3 + i:  P_i[k][m] = g_ik*J_im + g_(3+i)k*J_(3+i)m  (k <= m),  c_i[k] = g_ik*e_i + g_(3+i)k*e_(3+i);
+ *      A_km = (P_0 + P_1) + (P_2 + 0) and b_k = (c_0 + c_1) + (c_2 + 0) elementwise (the "+ 0" turns -0 into +0);
+ *      then A_kk += L, L = lambda*lambda rounded once.  A y = b by LDL^T:
+ *        l10 = A01/A00;  l20 = A02/A00;  l30 = A03/A00;
+ *        d1 = A11 - l10*A01;  t21 = A12 - l20*A01;  t31 = A13 - l30*A01;  l21 = t21/d1;  l31 = t31/d1;
+ *        d2 = (A22 - l20*A02) - l21*t21;  t32 = (A23 - l30*A02) - l31*t21;  l32 = t32/d2;
+ *        d3 = ((A33 - l30*A03) - l31*t31) - l32*t32;
+ *        z1 = b1 - l10*b0;  z2 = (b2 - l20*b0) - l21*z1;  z3 = ((b3 - l30*b0) - l31*z1) - l32*z2;
+ *        y3 = z3/d3;  y2 = z2/d2 - l32*y3;  y1 = (z1/d1 - l21*y2) - l31*y3;  y0 = ((b0/A00 - l10*y1) - l20*y2) - l30*y3
+ *      theta_k = theta_k + y_k, then theta_k = remainder(theta_k, 2pi) when |theta_k| > pi;  k += 1;  back to 1.
+ *   iters_out = k and err_out = err at the stop.  With weights (1, 1, 1, 0, 0, 0) the step equals ikb_dls_refine_*'s
+ *   mathematically (J^T (J J^T + L I)^-1 = (J^T J + L I)^-1 J^T), not in bits.
+ * Guards and statistics are those of ikb_dls_refine_*, the box test on the position column p_d; sum_fk_error /
+ * n_fk_error sum the final weighted errors of the finite rows.
+ * Refused with IKB_ERR_INVALID before the engine is looked at, each with its own message: NULL weights, a weight
+ * that is negative or not finite, all six weights zero, then every refusal of ikb_dls_refine_* (NULL poses are "NULL
+ * targets"; the pose buffer must be aligned to its element size).  Nothing is launched for a refused call or n = 0.
+ * _device: DEVICE pointers, enqueued on `stream`, one launch.  _host: HOST pointers, staged through the engine's
+ * pipeline with no per-call allocation, `stats` filled (nullable): poses in the slot's input buffer, seeds in its
+ * target buffer with err_out behind them, angles in its output buffer, iterations in its auxiliary buffer.  A host
+ * chunk, one launch, holds S / 4 rows, S the rows of a staging slot. */
+int ikb_dls_pose_refine_device(ikb_engine *e, const void *poses, int pose_dtype, int64_t n, const void *seed,
+                               int64_t n_seed, void *angles_out, int angles_dtype, const double weights[6],
+                               double damping, double tol, int32_t max_iter, int32_t *iters_out /* nullable */,
+                               void *err_out /* nullable, angles_dtype */, void *stream);
+int ikb_dls_pose_refine_host(ikb_engine *e, const void *poses, int pose_dtype, int64_t n, const void *seed,
+                             int64_t n_seed, void *angles_out, int angles_dtype, const double weights[6],
+                             double damping, double tol, int32_t max_iter, int32_t *iters_out /* nullable */,
+                             void *err_out /* nullable, angles_dtype */, ikb_stats *stats);
+
+/* ---- ANN (ann.py:70-85, inverse.py:142-155)-------------------------------------------------- */
 /* replaces ANN.load_model (ann.py:78-85): upload the Keras Sequential's Dense kernels/biases and the
  * two StandardScalers.  dims[n_layers+1] = {3, 500, ..., 500, 4}; weights[l] is row-major
  * (dims[l] x dims[l+1]) float32 = Keras `kernel`, biases[l] has dims[l+1] floats.  Hidden layers

@@ -27,6 +27,7 @@ EXPORTED_SYMBOLS = [
     "ikb_fabrik_chain_device", "ikb_fabrik_chain_host",
     "ikb_fk_device", "ikb_fk_host", "ikb_fk_chain_host", "ikb_fk_transforms_device", "ikb_fk_transforms_host",
     "ikb_jacobian_device", "ikb_jacobian_host", "ikb_dls_refine_device", "ikb_dls_refine_host",
+    "ikb_dls_pose_refine_device", "ikb_dls_pose_refine_host",
     "ikb_mlp_load", "ikb_ann_solve_device", "ikb_ann_solve_host",
     "ikb_generate_device", "ikb_microbench_fma", "ikb_launch_count",
     "ikb_host_alloc", "ikb_host_free", "ikb_host_register", "ikb_host_unregister",
@@ -71,6 +72,7 @@ def load():
     vp, i32, i64, dbl = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
     engine = ctypes.c_void_p
     stats_p = ctypes.POINTER(IkbStats)
+    dbl_p = ctypes.POINTER(dbl)
     protos = {
         "ikb_engine_create": (i32, [ctypes.POINTER(IkbConfig), ctypes.POINTER(engine)]),
         "ikb_engine_destroy": (None, [engine]),
@@ -98,6 +100,10 @@ def load():
         "ikb_dls_refine_device": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl, dbl, ctypes.c_int32, vp, vp, vp]),
         "ikb_dls_refine_host": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl, dbl, ctypes.c_int32, vp, vp,
                                       stats_p]),
+        "ikb_dls_pose_refine_device": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl_p, dbl, dbl, ctypes.c_int32,
+                                             vp, vp, vp]),
+        "ikb_dls_pose_refine_host": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl_p, dbl, dbl, ctypes.c_int32, vp,
+                                           vp, stats_p]),
         "ikb_mlp_load": (i32, [engine, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
                                ctypes.POINTER(vp), ctypes.POINTER(vp), vp, vp, vp, vp]),
         "ikb_ann_solve_device": (i32, [engine, vp, i32, i64, vp, vp, i32, i32, vp]),

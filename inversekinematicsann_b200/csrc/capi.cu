@@ -38,6 +38,11 @@ cudaError_t ikb_launch_dls_refine(const void *xyz, int xyz_f64, const void *seed
                                   double damping, double tol, int max_iter, IkbDeviceStats *stats,
                                   unsigned long long *work_counter, const IkbRobot &rc, int num_sms,
                                   cudaStream_t stream);
+cudaError_t ikb_launch_dls_pose_refine(const void *poses, int pose_f64, const void *seed, long long n_seed,
+                                       void *angles_out, int angles_f64, int *iters, void *err_out, long long n,
+                                       long long index_base, const double weights[6], double damping, double tol,
+                                       int max_iter, IkbDeviceStats *stats, unsigned long long *work_counter,
+                                       const IkbRobot &rc, int num_sms, cudaStream_t stream);
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,
                                     IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                     cudaStream_t stream);
@@ -877,6 +882,97 @@ int ikb_dls_refine_host(ikb_engine *e, const void *xyz, int xyz_dtype, int64_t n
         IKB_CUDA(e, ikb_launch_dls_refine(s.d_in2, xyz_dtype == IKB_F64, s.d_in, per_row_seed ? m : 1, s.d_out,
                                           angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr, d_err, m, lo,
                                           damping, tol, max_iter, e->d_stats, counter, e->rc, e->num_sms, s.stream));
+        IKB_CUDA(e, counter_release(e, slot, s.stream));
+        e->launches++;
+        IKB_CUDA(e, cudaMemcpyAsync((char *)angles_out + lo * a_row, s.d_out, m * a_row, cudaMemcpyDeviceToHost, s.stream));
+        if (iters_out)
+            IKB_CUDA(e, cudaMemcpyAsync(iters_out + lo, s.d_aux, m * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
+        if (err_out)
+            IKB_CUDA(e, cudaMemcpyAsync((char *)err_out + lo * e_row, d_err, m * e_row, cudaMemcpyDeviceToHost, s.stream));
+    }
+    return host_end(e, stats);
+}
+
+// ---- damped-least-squares refinement onto poses ---------------------------------------------------------------------
+// the weights first, then everything dls_bad_args checks (the engine last)
+static const char *pose_bad_args(const ikb_engine *e, const void *poses, int pose_dtype, int64_t n, const void *seed,
+                                 int64_t n_seed, const void *angles_out, int angles_dtype, const double *weights,
+                                 double damping, double tol, int32_t max_iter, const int32_t *iters_out,
+                                 const void *err_out)
+{
+    if (!weights)
+        return "NULL weights";
+    bool any = false;
+    for (int i = 0; i < 6; ++i) {
+        if (!(weights[i] >= 0.0) || !std::isfinite(weights[i]))
+            return "weights must be >= 0 and finite";
+        any = any || weights[i] > 0.0;
+    }
+    if (!any)
+        return "all six weights are zero";
+    return dls_bad_args(e, poses, pose_dtype, n, seed, n_seed, angles_out, angles_dtype, damping, tol, max_iter,
+                        iters_out, err_out);
+}
+
+int ikb_dls_pose_refine_device(ikb_engine *e, const void *poses, int pose_dtype, int64_t n, const void *seed,
+                               int64_t n_seed, void *angles_out, int angles_dtype, const double weights[6],
+                               double damping, double tol, int32_t max_iter, int32_t *iters_out, void *err_out,
+                               void *stream)
+{
+    if (const char *why = pose_bad_args(e, poses, pose_dtype, n, seed, n_seed, angles_out, angles_dtype, weights,
+                                        damping, tol, max_iter, iters_out, err_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_dls_pose_refine_device: ") + why);
+    if (n == 0)
+        return IKB_OK;
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    unsigned long long *counter;
+    int slot;
+    IKB_CUDA(e, counter_claim(e, (cudaStream_t)stream, &counter, &slot));
+    IKB_CUDA(e, ikb_launch_dls_pose_refine(poses, pose_dtype == IKB_F64, seed, n_seed, angles_out,
+                                           angles_dtype == IKB_F64, iters_out, err_out, n, 0, weights, damping, tol,
+                                           max_iter, e->d_stats, counter, e->rc, e->num_sms, (cudaStream_t)stream));
+    IKB_CUDA(e, counter_release(e, slot, (cudaStream_t)stream));
+    e->launches++;
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline, S / 4 rows each (S the rows of a slot): poses in d_in (32 B per slot row, so 128 B per
+// chunk row), seeds in d_in2 (24 B per slot row) with the fp64 errors behind them, angles in d_out, iterations in
+// d_aux.  A single seed (n_seed == 1) is copied to d_in2 of every slot once.
+int ikb_dls_pose_refine_host(ikb_engine *e, const void *poses, int pose_dtype, int64_t n, const void *seed,
+                             int64_t n_seed, void *angles_out, int angles_dtype, const double weights[6],
+                             double damping, double tol, int32_t max_iter, int32_t *iters_out, void *err_out,
+                             ikb_stats *stats)
+{
+    if (const char *why = pose_bad_args(e, poses, pose_dtype, n, seed, n_seed, angles_out, angles_dtype, weights,
+                                        damping, tol, max_iter, iters_out, err_out))
+        return fail(e, IKB_ERR_INVALID, std::string("ikb_dls_pose_refine_host: ") + why);
+    int rc = host_begin(e, n);
+    if (rc)
+        return rc;
+    const size_t p_row = 16 * esize(pose_dtype), a_row = 4 * esize(angles_dtype), e_row = esize(angles_dtype);
+    const long long m_max = e->slot_rows / 4;
+    const bool per_row_seed = n_seed != 1;
+    if (n > 0 && !per_row_seed)
+        for (int i = 0; i < kSlots; ++i)
+            IKB_CUDA(e, cudaMemcpyAsync(e->slots[i].d_in2, seed, a_row, cudaMemcpyHostToDevice, e->slots[i].stream));
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        void *d_err = err_out ? (void *)((char *)s.d_in2 + 32 * m_max) : nullptr;
+        IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)poses + lo * p_row, m * p_row, cudaMemcpyHostToDevice,
+                                    s.stream));
+        if (per_row_seed)
+            IKB_CUDA(e, cudaMemcpyAsync(s.d_in2, (const char *)seed + lo * a_row, m * a_row, cudaMemcpyHostToDevice,
+                                        s.stream));
+        unsigned long long *counter;
+        int slot;
+        IKB_CUDA(e, counter_claim(e, s.stream, &counter, &slot));
+        IKB_CUDA(e, ikb_launch_dls_pose_refine(s.d_in, pose_dtype == IKB_F64, s.d_in2, per_row_seed ? m : 1, s.d_out,
+                                               angles_dtype == IKB_F64, iters_out ? s.d_aux : nullptr, d_err, m, lo,
+                                               weights, damping, tol, max_iter, e->d_stats, counter, e->rc,
+                                               e->num_sms, s.stream));
         IKB_CUDA(e, counter_release(e, slot, s.stream));
         e->launches++;
         IKB_CUDA(e, cudaMemcpyAsync((char *)angles_out + lo * a_row, s.d_out, m * a_row, cudaMemcpyDeviceToHost, s.stream));

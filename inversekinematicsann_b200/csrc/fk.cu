@@ -734,6 +734,250 @@ __global__ void __launch_bounds__(DLS_THREADS) dls_refine_kernel(const DlsArgs a
     }
 }
 
+// ---- damped-least-squares refinement of joint angles onto full effector poses --------------------------------------
+// The sibling of dls_refine_kernel for a 6-D task: position and orientation of T_4, weighted per axis.  Same quad per
+// row, chain, guards, refill loop, statistics and stores.  Lane r < 3 holds row r of the target ([R_d | p_d] row r),
+// row r of T_4, element r of every z_j and row r of the position Jacobian, so it owns task rows r (linear) and 3 + r
+// (angular).  Row r of R_e = R_d R^T needs the rows of R from the other lanes (quad shuffles); the quaternion error is
+// then formed redundantly in every lane.  A = J^T W J + lambda^2 I and b = J^T W e are summed over the task rows as
+// per-lane partials reduced across the quad (lane 3 contributes zero), and every lane solves the 4 x 4 system by
+// LDL^T; lane k applies Delta theta_k.  Operation order: include/ikb200.h (ikb_dls_pose_refine_*).
+struct DlsPoseArgs {
+    const void *poses;   // n x 4 x 4 row-major, pose dtype; row 3 is not read
+    int pose_f64;
+    const void *seed;    // n_seed x 4 (n_seed 1 or n), angles dtype; may equal angles_out when n_seed == n
+    long long n_seed;
+    void *angles_out;    // n x 4, angles dtype
+    int *iters;          // nullable, n
+    void *err_out;       // nullable, n (angles dtype)
+    long long n;
+    long long index_base;  // global row of row 0 (host pipeline chunks): the row numbers in the statistics
+    double w[6];         // task weights: x, y, z, then the three orientation axes
+    double lam2;         // damping^2, rounded once
+    double tol;
+    int max_iter;
+    IkbDeviceStats *stats;
+    unsigned long long *work_counter;  // zero at launch
+    IkbRobot rc;
+};
+
+__device__ __forceinline__ double ikb_load_elem(const void *p, int f64, long long i)
+{
+    return f64 ? __ldg(reinterpret_cast<const double *>(p) + i) : (double)__ldg(reinterpret_cast<const float *>(p) + i);
+}
+
+// a + b over the four lanes of a quad, as (lane 0 + lane 1) + (lane 2 + lane 3) in every lane (addition commutes)
+__device__ __forceinline__ double ikb_quad_sum(double v)
+{
+    v = __dadd_rn(v, __shfl_xor_sync(IKB_FULL_MASK, v, 1, 4));
+    return __dadd_rn(v, __shfl_xor_sync(IKB_FULL_MASK, v, 2, 4));
+}
+
+template <typename Real>
+__global__ void __launch_bounds__(DLS_THREADS) dls_pose_refine_kernel(const DlsPoseArgs a)
+{
+    const double TWO_PI = 6.283185307179586, PI = 3.141592653589793;
+    const int lane = threadIdx.x & 31, r = lane & 3;
+    const unsigned quads_below = (1u << (lane & ~3)) - 1u;
+    const bool alpha_bad = a.rc.alpha[r] < -TWO_PI || a.rc.alpha[r] > TWO_PI;
+    const bool task = r < 3;  // lane r owns task rows r and 3 + r
+    const double w_lin = r == 0 ? a.w[0] : r == 1 ? a.w[1] : a.w[2];
+    const double w_ang = r == 0 ? a.w[3] : r == 1 ? a.w[4] : a.w[5];
+    double th = 0.0, rd0 = 0.0, rd1 = 0.0, rd2 = 0.0, pd = 0.0;  // row r of the target: R_d row r and p_d[r]
+    long long row = 0;
+    int k = 0;
+    bool live = false, exhausted = false;
+    unsigned long long n_solved = 0, sum_k = 0, capped = 0, n_err = 0;
+    double err_sum = 0.0;
+    long long first_limits = IKB_I64_MAX, first_range = IKB_I64_MAX;
+    for (;;) {
+        if (!exhausted) {  // refill: every quad without a row takes the next one
+            const unsigned want = __ballot_sync(IKB_FULL_MASK, !live) & 0x11111111u;
+            if (want) {
+                unsigned long long base = 0;
+                if (lane == 0)
+                    base = atomicAdd(a.work_counter, (unsigned long long)__popc(want));
+                base = __shfl_sync(IKB_FULL_MASK, base, 0);
+                if (!live) {
+                    const long long rw = (long long)base + __popc(want & quads_below);
+                    if (rw < a.n) {
+                        row = rw;
+                        k = 0;
+                        live = true;
+                        th = (double)reinterpret_cast<const Real *>(a.seed)[4 * (a.n_seed == 1 ? 0 : rw) + r];
+                        if (task) {
+                            const long long o = 16 * rw + 4 * r;
+                            rd0 = ikb_load_elem(a.poses, a.pose_f64, o);
+                            rd1 = ikb_load_elem(a.poses, a.pose_f64, o + 1);
+                            rd2 = ikb_load_elem(a.poses, a.pose_f64, o + 2);
+                            pd = ikb_load_elem(a.poses, a.pose_f64, o + 3);
+                        }
+                        if (th < -TWO_PI || th > TWO_PI || alpha_bad)
+                            first_range = min(first_range, a.index_base + rw);
+                        if (r == 0 && ikb_out_of_limits(a.rc, pd, ikb_load_elem(a.poses, a.pose_f64, 16 * rw + 7),
+                                                        ikb_load_elem(a.poses, a.pose_f64, 16 * rw + 11)))
+                            first_limits = min(first_limits, a.index_base + rw);
+                    }
+                }
+                exhausted = (long long)(base + __popc(want)) >= a.n;
+            }
+        }
+        if (__ballot_sync(IKB_FULL_MASK, live) == 0)
+            break;
+        // the chain, at full warp width (quads without a row compute on stale registers and write nothing)
+        double s, c;
+        sincos(th, &s, &c);
+        double t[4] = {r == 0 ? 1.0 : 0.0, r == 1 ? 1.0 : 0.0, r == 2 ? 1.0 : 0.0, r == 3 ? 1.0 : 0.0};
+        double zs[4], ps[5];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double sj = __shfl_sync(IKB_FULL_MASK, s, j, 4), cj = __shfl_sync(IKB_FULL_MASK, c, j, 4);
+            double nr[4];
+            zs[j] = t[2];
+            ps[j] = t[3];
+            fk_dh_step_row(t, sj, cj, a.rc.cos_alpha[j], a.rc.sin_alpha[j], a.rc.a[j], a.rc.eps[j], nr);
+#pragma unroll
+            for (int q = 0; q < 4; ++q)
+                t[q] = nr[q];
+        }
+        ps[4] = t[3];
+        double lin[4];
+        fk_quad_position_jacobian_row(r, zs, ps, lin);
+        // row r of R_e = R_d R^T: (R_e)_rj = (Rd_r0 R_j0 + Rd_r1 R_j1) + Rd_r2 R_j2, row j of R from lane j
+        double me[3];
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            const double r0 = __shfl_sync(IKB_FULL_MASK, t[0], j, 4), r1 = __shfl_sync(IKB_FULL_MASK, t[1], j, 4);
+            const double r2 = __shfl_sync(IKB_FULL_MASK, t[2], j, 4);
+            me[j] = __dadd_rn(__dadd_rn(__dmul_rn(rd0, r0), __dmul_rn(rd1, r1)), __dmul_rn(rd2, r2));
+        }
+        double M[3][3];
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j)
+                M[i][j] = __shfl_sync(IKB_FULL_MASK, me[j], i, 4);
+        // e_o = 2 x the vector part of R_e's unit quaternion, scalar part >= 0 (Shepperd: branch on the largest of
+        // the trace and the diagonal, first on ties; h = 2 |q_w| or 2 |q_x|, 2 |q_y|, 2 |q_z|)
+        const double tr = __dadd_rn(__dadd_rn(M[0][0], M[1][1]), M[2][2]);
+        const double dx = __dsub_rn(M[2][1], M[1][2]), dy = __dsub_rn(M[0][2], M[2][0]), dz = __dsub_rn(M[1][0], M[0][1]);
+        double eo0, eo1, eo2;
+        if (tr >= M[0][0] && tr >= M[1][1] && tr >= M[2][2]) {  // a NaN diagonal falls through to the last case
+            const double h = __dsqrt_rn(__dadd_rn(1.0, tr));
+            eo0 = __ddiv_rn(dx, h); eo1 = __ddiv_rn(dy, h); eo2 = __ddiv_rn(dz, h);
+        } else if (M[0][0] >= M[1][1] && M[0][0] >= M[2][2]) {
+            const double h = __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, M[0][0]), M[1][1]), M[2][2]));
+            eo0 = h; eo1 = __ddiv_rn(__dadd_rn(M[0][1], M[1][0]), h); eo2 = __ddiv_rn(__dadd_rn(M[0][2], M[2][0]), h);
+            if (dx < 0.0) { eo0 = -eo0; eo1 = -eo1; eo2 = -eo2; }
+        } else if (M[1][1] >= M[2][2]) {
+            const double h = __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, M[1][1]), M[0][0]), M[2][2]));
+            eo0 = __ddiv_rn(__dadd_rn(M[0][1], M[1][0]), h); eo1 = h; eo2 = __ddiv_rn(__dadd_rn(M[1][2], M[2][1]), h);
+            if (dy < 0.0) { eo0 = -eo0; eo1 = -eo1; eo2 = -eo2; }
+        } else {
+            const double h = __dsqrt_rn(__dsub_rn(__dsub_rn(__dadd_rn(1.0, M[2][2]), M[0][0]), M[1][1]));
+            eo0 = __ddiv_rn(__dadd_rn(M[0][2], M[2][0]), h); eo1 = __ddiv_rn(__dadd_rn(M[1][2], M[2][1]), h); eo2 = h;
+            if (dz < 0.0) { eo0 = -eo0; eo1 = -eo1; eo2 = -eo2; }
+        }
+        const double ep = __dsub_rn(pd, t[3]);  // e_p[r]
+        const double ex = __shfl_sync(IKB_FULL_MASK, ep, 0, 4), ey = __shfl_sync(IKB_FULL_MASK, ep, 1, 4);
+        const double ez = __shfl_sync(IKB_FULL_MASK, ep, 2, 4);
+        const double sp = __dadd_rn(__dadd_rn(__dmul_rn(a.w[0], __dmul_rn(ex, ex)), __dmul_rn(a.w[1], __dmul_rn(ey, ey))),
+                                    __dmul_rn(a.w[2], __dmul_rn(ez, ez)));
+        const double so = __dadd_rn(__dadd_rn(__dmul_rn(a.w[3], __dmul_rn(eo0, eo0)), __dmul_rn(a.w[4], __dmul_rn(eo1, eo1))),
+                                    __dmul_rn(a.w[5], __dmul_rn(eo2, eo2)));
+        const double err = __dsqrt_rn(__dadd_rn(sp, so));
+        // A = J^T W J (upper triangle) and b = J^T W e at full warp width, since the quad sums shuffle (a row that
+        // stops below does not use them).  g = w_r J_r, ga = w_{3+r} J_{3+r}: this lane's weighted task rows
+        const double eor = r == 0 ? eo0 : r == 1 ? eo1 : eo2;
+        double g[4], ga[4];
+#pragma unroll
+        for (int m = 0; m < 4; ++m) {
+            g[m] = __dmul_rn(w_lin, lin[m]);
+            ga[m] = __dmul_rn(w_ang, zs[m]);
+        }
+        double A[4][4], b[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+#pragma unroll
+            for (int j = i; j < 4; ++j)
+                A[i][j] = ikb_quad_sum(task ? __dadd_rn(__dmul_rn(g[i], lin[j]), __dmul_rn(ga[i], zs[j])) : 0.0);
+            b[i] = ikb_quad_sum(task ? __dadd_rn(__dmul_rn(g[i], ep), __dmul_rn(ga[i], eor)) : 0.0);
+        }
+        if (live && (err <= a.tol || k >= a.max_iter)) {  // quad-uniform: every lane holds the same err and k
+            reinterpret_cast<Real *>(a.angles_out)[4 * row + r] = (Real)th;
+            if (r == 0) {
+                if (a.iters)
+                    a.iters[row] = k;
+                if (a.err_out)
+                    reinterpret_cast<Real *>(a.err_out)[row] = (Real)err;
+                ++n_solved;
+                sum_k += (unsigned)k;
+                capped += err <= a.tol ? 0u : 1u;  // NaN rows included
+                if (isfinite(err)) {
+                    err_sum += err;
+                    ++n_err;
+                }
+            }
+            live = false;
+        }
+        if (live) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                A[i][i] = __dadd_rn(A[i][i], a.lam2);
+            // A y = b by LDL^T (no square root)
+            const double l10 = __ddiv_rn(A[0][1], A[0][0]), l20 = __ddiv_rn(A[0][2], A[0][0]);
+            const double l30 = __ddiv_rn(A[0][3], A[0][0]);
+            const double d1 = __dsub_rn(A[1][1], __dmul_rn(l10, A[0][1]));
+            const double t21 = __dsub_rn(A[1][2], __dmul_rn(l20, A[0][1]));
+            const double t31 = __dsub_rn(A[1][3], __dmul_rn(l30, A[0][1]));
+            const double l21 = __ddiv_rn(t21, d1), l31 = __ddiv_rn(t31, d1);
+            const double d2 = __dsub_rn(__dsub_rn(A[2][2], __dmul_rn(l20, A[0][2])), __dmul_rn(l21, t21));
+            const double t32 = __dsub_rn(__dsub_rn(A[2][3], __dmul_rn(l30, A[0][2])), __dmul_rn(l31, t21));
+            const double l32 = __ddiv_rn(t32, d2);
+            const double d3 = __dsub_rn(__dsub_rn(__dsub_rn(A[3][3], __dmul_rn(l30, A[0][3])), __dmul_rn(l31, t31)),
+                                        __dmul_rn(l32, t32));
+            const double z1 = __dsub_rn(b[1], __dmul_rn(l10, b[0]));
+            const double z2 = __dsub_rn(__dsub_rn(b[2], __dmul_rn(l20, b[0])), __dmul_rn(l21, z1));
+            const double z3 = __dsub_rn(__dsub_rn(__dsub_rn(b[3], __dmul_rn(l30, b[0])), __dmul_rn(l31, z1)),
+                                        __dmul_rn(l32, z2));
+            const double y3 = __ddiv_rn(z3, d3);
+            const double y2 = __dsub_rn(__ddiv_rn(z2, d2), __dmul_rn(l32, y3));
+            const double y1 = __dsub_rn(__dsub_rn(__ddiv_rn(z1, d1), __dmul_rn(l21, y2)), __dmul_rn(l31, y3));
+            const double y0 = __dsub_rn(__dsub_rn(__dsub_rn(__ddiv_rn(b[0], A[0][0]), __dmul_rn(l10, y1)),
+                                                  __dmul_rn(l20, y2)),
+                                        __dmul_rn(l30, y3));
+            th = __dadd_rn(th, r == 0 ? y0 : r == 1 ? y1 : r == 2 ? y2 : y3);
+            if (fabs(th) > PI)
+                th = remainder(th, TWO_PI);  // exact: the angle stays inside the FK guard
+            ++k;
+        }
+    }
+    n_solved = ikb_warp_sum(n_solved);
+    sum_k = ikb_warp_sum(sum_k);
+    capped = ikb_warp_sum(capped);
+    n_err = ikb_warp_sum(n_err);
+    err_sum = ikb_warp_sum(err_sum);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        first_limits = min(first_limits, __shfl_xor_sync(IKB_FULL_MASK, first_limits, o));
+        first_range = min(first_range, __shfl_xor_sync(IKB_FULL_MASK, first_range, o));
+    }
+    if (lane == 0 && n_solved != 0) {
+        atomicAdd(&a.stats->n_solved, n_solved);
+        atomicAdd(&a.stats->sum_iterations, sum_k);
+        if (capped)
+            atomicAdd(&a.stats->n_iter_capped, capped);
+        if (n_err) {
+            atomicAdd(&a.stats->sum_fk_error, err_sum);
+            atomicAdd(&a.stats->n_fk_error, n_err);
+        }
+        if (first_limits != IKB_I64_MAX)
+            atomicMin(&a.stats->first_out_of_limits, first_limits);
+        if (first_range != IKB_I64_MAX)
+            atomicMin(&a.stats->first_fk_angle_range, first_range);
+    }
+}
+
 struct LimitsArgs {
     const void *xyz;
     int xyz_f64;
@@ -965,6 +1209,39 @@ cudaError_t ikb_launch_dls_refine(const void *xyz, int xyz_f64, const void *seed
     if (err != cudaSuccess)
         return err;
     // persistent grid: resident CTAs per SM x SM count, trimmed for small batches (one quad per row)
+    const long long want = (n + DLS_THREADS / 4 - 1) / (DLS_THREADS / 4), cap = (long long)num_sms * bps;
+    kern<<<(unsigned)(want < cap ? want : cap), DLS_THREADS, 0, stream>>>(a);
+    return cudaGetLastError();
+}
+
+// damped-least-squares refinement onto poses (ikb_dls_pose_refine_*); work_counter as for ikb_launch_dls_refine
+cudaError_t ikb_launch_dls_pose_refine(const void *poses, int pose_f64, const void *seed, long long n_seed,
+                                       void *angles_out, int angles_f64, int *iters, void *err_out, long long n,
+                                       long long index_base, const double weights[6], double damping, double tol,
+                                       int max_iter, IkbDeviceStats *stats, unsigned long long *work_counter,
+                                       const IkbRobot &rc, int num_sms, cudaStream_t stream)
+{
+    if (n <= 0)
+        return cudaSuccess;
+    DlsPoseArgs a;
+    a.poses = poses; a.pose_f64 = pose_f64; a.seed = seed; a.n_seed = n_seed; a.angles_out = angles_out;
+    a.iters = iters; a.err_out = err_out; a.n = n; a.index_base = index_base;
+    for (int i = 0; i < 6; ++i)
+        a.w[i] = weights[i];
+    a.lam2 = damping * damping; a.tol = tol; a.max_iter = max_iter;
+    a.stats = stats; a.work_counter = work_counter; a.rc = rc;
+    void (*kern)(DlsPoseArgs) = angles_f64 ? dls_pose_refine_kernel<double> : dls_pose_refine_kernel<float>;
+    static int blocks_per_sm[2] = {};
+    int &bps = blocks_per_sm[angles_f64 ? 1 : 0];
+    if (bps == 0) {
+        cudaError_t err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, DLS_THREADS, 0);
+        if (err != cudaSuccess)
+            return err;
+        bps = bps > 0 ? bps : 1;
+    }
+    cudaError_t err = cudaMemsetAsync(work_counter, 0, sizeof(unsigned long long), stream);
+    if (err != cudaSuccess)
+        return err;
     const long long want = (n + DLS_THREADS / 4 - 1) / (DLS_THREADS / 4), cap = (long long)num_sms * bps;
     kern<<<(unsigned)(want < cap ? want : cap), DLS_THREADS, 0, stream>>>(a);
     return cudaGetLastError();

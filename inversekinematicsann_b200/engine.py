@@ -347,10 +347,14 @@ class IkEngine:
     def _dls_args(xyz, seed, out):
         """The checks of `dls_refine` that need no device -> (xyz, seed (n_seed, 4), n_seed, out)."""
         xyz = IkEngine._rows(xyz, 3, "points")
-        n = xyz.shape[0]
+        return (xyz,) + IkEngine._seed_args(xyz.shape[0], seed, out)
+
+    @staticmethod
+    def _seed_args(n, seed, out):
+        """Seeds and result buffer of the DLS refinements for n rows -> (seed (n_seed, 4), n_seed, out)."""
         if out is not None and out is seed:  # in place: the seeds must already be the buffer the library writes
             IkEngine._check_out(out, n, 4, (np.float32, np.float64), "out")
-            return xyz, seed, n, out
+            return seed, n, out
         seed = np.asarray(seed)
         if seed.ndim == 1:
             seed = seed.reshape(1, -1)
@@ -360,7 +364,41 @@ class IkEngine:
         if out is None:
             out = np.empty((n, 4), dtype=seed.dtype)
         IkEngine._check_out(out, n, 4, (seed.dtype,), "out")
-        return xyz, seed, seed.shape[0], out
+        return seed, seed.shape[0], out
+
+    def dls_pose_refine(self, poses, seed, weights=None, damping=None, tol=None, max_iter=None, out=None,
+                        return_iters=False, return_error=False):
+        """Damped-least-squares refinement of joint angles onto (n, 4, 4) effector poses (include/ikb200.h
+        ikb_dls_pose_refine_*): rows 0-2 of each pose hold [R | p], the layout of fk_transforms' matrices, so
+        ``fk_transforms(theta)[0][:, 3]`` is a valid input.  weights: 6 values (x, y, z, then the orientation axes),
+        each >= 0.  Seeds, out and the returns are those of `dls_refine`, the error being the weighted one.  Defaults:
+        POSE_WEIGHTS, POSE_DAMPING, POSE_TOL, POSE_MAX_ITER."""
+        poses, seed, n_seed, out = self._pose_args(poses, seed, out)
+        n = poses.shape[0]
+        w, damping, tol, max_iter = _pose_params(weights, damping, tol, max_iter)
+        iters = np.empty(n, dtype=np.int32) if return_iters else None
+        err = np.empty(n, dtype=out.dtype) if return_error else None
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_dls_pose_refine_host(
+            self._handle, poses.ctypes.data, _np_dtype_code(poses), n, seed.ctypes.data, n_seed, out.ctypes.data,
+            _np_dtype_code(out), w, damping, tol, max_iter, iters.ctypes.data if return_iters else None,
+            err.ctypes.data if return_error else None, ctypes.byref(s)), "ikb_dls_pose_refine_host")
+        res = (out, IkStats.from_c(s))
+        if return_iters:
+            res += (iters,)
+        if return_error:
+            res += (err,)
+        return res
+
+    @staticmethod
+    def _pose_args(poses, seed, out):
+        """The checks of `dls_pose_refine` that need no device -> (poses (n, 4, 4) contiguous, seed, n_seed, out)."""
+        poses = np.ascontiguousarray(poses)
+        if poses.dtype not in (np.float32, np.float64):
+            poses = poses.astype(np.float64)
+        if poses.ndim != 3 or poses.shape[1:] != (4, 4):
+            raise ValueError(f"poses must have shape (n, 4, 4), got {poses.shape}")
+        return (poses,) + IkEngine._seed_args(poses.shape[0], seed, out)
 
     def mlp_load(self, weights, biases, mean_x, scale_x, mean_y, scale_y):
         """reference ann.py:78-85: upload Keras Dense kernels (in, out) + biases and both scalers."""
@@ -607,6 +645,41 @@ class IkEngine:
             _torch_dtype_code(out), damping, tol, max_iter, iters.data_ptr() if iters is not None else None,
             err.data_ptr() if err is not None else None, _torch_stream_ptr(self.device)), "ikb_dls_refine_device")
 
+    def dls_pose_refine_device(self, poses, seed, out, iters=None, err=None, weights=None, damping=None, tol=None,
+                               max_iter=None):
+        """dls_pose_refine on CUDA tensors of this engine's device, enqueued on torch's current stream (no
+        synchronisation): poses a contiguous (n, 4, 4) tensor; seed, out, iters and err as for dls_refine_device.  The
+        guards and statistics accumulate in the engine's block (stats_fetch_torch)."""
+        if not _is_torch_tensor(poses) or not poses.is_cuda:
+            raise TypeError("poses must be a CUDA torch tensor")
+        if poses.device.index != self.device:
+            raise ValueError(f"poses lives on cuda:{poses.device.index}, the engine on cuda:{self.device}")
+        if poses.dim() != 3 or tuple(poses.shape[1:]) != (4, 4) or not poses.is_contiguous():
+            raise ValueError("poses must be a contiguous (n, 4, 4) tensor")
+        n = poses.shape[0]
+        if _is_torch_tensor(seed) and seed.dim() == 1:
+            seed = seed.view(1, -1)
+        seed = self._dev_rows(seed, 4, "seed")
+        if seed.shape[0] not in (1, n):
+            raise ValueError(f"seed must have 1 or {n} rows, got {seed.shape[0]}")
+        _torch_dtype_code(seed)
+        out = self._dev_rows(out, 4, "angles")
+        self._same_rows(poses, out, "angles")
+        if out.dtype != seed.dtype:
+            raise TypeError(f"angles must have the seeds' dtype {seed.dtype}, got {out.dtype}")
+        if iters is not None:
+            self._dev_vec(iters, n, "torch.int32", "iters")
+        if err is not None:
+            self._dev_vec(err, n, str(seed.dtype), "err")
+        w, damping, tol, max_iter = _pose_params(weights, damping, tol, max_iter)
+        if n == 0:  # nothing to do, and an empty tensor's data_ptr() may be NULL
+            return
+        self._check(self._lib.ikb_dls_pose_refine_device(
+            self._handle, poses.data_ptr(), _torch_dtype_code(poses), n, seed.data_ptr(), seed.shape[0],
+            out.data_ptr(), _torch_dtype_code(out), w, damping, tol, max_iter,
+            iters.data_ptr() if iters is not None else None, err.data_ptr() if err is not None else None,
+            _torch_stream_ptr(self.device)), "ikb_dls_pose_refine_device")
+
     def check_limits_device(self, xyz):
         xyz = self._dev_rows(xyz, 3, "points")
         self._check(self._lib.ikb_check_limits_device(self._handle, xyz.data_ptr(), _torch_dtype_code(xyz),
@@ -678,6 +751,30 @@ def _dls_params(damping, tol, max_iter):
     """None -> the defaults; the library checks the values (each refusal has its own message)."""
     return (float(DLS_DAMPING if damping is None else damping), float(DLS_TOL if tol is None else tol),
             int(DLS_MAX_ITER if max_iter is None else max_iter))
+
+
+# defaults of the damped-least-squares refinement onto poses, chosen from the damping sweep of
+# profiles/r07_pose_bench.json (DESIGN.md §5): from 0.5 down to 0.002 every seed kind converges on more rows in fewer
+# steps, and at 0.002 every seed kind converges on at most 0.1 percentage points fewer rows than at the best measured
+# damping (0.001).  Of the rows that converge within 256 steps at 0.002, 99.6 % (FABRIK seeds) and 99.9 % (the DH
+# seed row) do so within 128.  Poses no angles produce always take max_iter steps, so it is not larger.
+POSE_WEIGHTS = (1.0, 1.0, 1.0, 1.0, 1.0, 1.0)  # x, y, z in metres, then the orientation axes (2 sin(theta/2) u)
+POSE_DAMPING = 0.002  # lambda, joint space
+POSE_TOL = 1e-9       # on the weighted error
+POSE_MAX_ITER = 128
+
+
+def _pose_params(weights, damping, tol, max_iter):
+    """None -> the defaults, weights as 6 C doubles; the library checks the values."""
+    w = POSE_WEIGHTS if weights is None else weights
+    try:
+        w = [float(v) for v in w]
+    except TypeError:
+        raise TypeError(f"weights must be 6 numbers, got {weights!r}") from None
+    if len(w) != 6:
+        raise ValueError(f"weights must be 6 numbers (x, y, z, then the orientation axes), got {len(w)}")
+    return ((ctypes.c_double * 6)(*w), float(POSE_DAMPING if damping is None else damping),
+            float(POSE_TOL if tol is None else tol), int(POSE_MAX_ITER if max_iter is None else max_iter))
 
 
 def _choice(table, key, what):

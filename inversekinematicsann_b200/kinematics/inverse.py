@@ -16,11 +16,43 @@ from abc import ABC, abstractmethod
 
 import numpy as np
 
-from ..engine import DLS_DAMPING, DLS_MAX_ITER, DLS_TOL
+from ..engine import DLS_DAMPING, DLS_MAX_ITER, DLS_TOL, POSE_DAMPING, POSE_MAX_ITER, POSE_TOL, POSE_WEIGHTS
 from ..robot.robot import OutOfRobotReachException
 from ._shared import get_engine, points_to_array
 from .ann import ANN
 from .forward import _ANGLE_MSG, ForwardKinematics
+
+
+def poses_to_array(dest_poses):
+    """(n, 4, 4) poses -- an array such as fkine_batch(angles)[0], or nested lists -> contiguous float array (float32
+    arrays stay float32, everything else becomes float64)."""
+    if isinstance(dest_poses, np.ndarray) and dest_poses.dtype in (np.float32, np.float64):
+        arr = dest_poses
+    else:
+        arr = np.asarray(dest_poses, dtype=np.float64)
+    if arr.size == 0:
+        return np.zeros((0, 4, 4), dtype=np.float64)
+    if arr.ndim != 3 or arr.shape[1:] != (4, 4):
+        raise ValueError(f'destination poses must have shape (n, 4, 4), not {arr.shape}')
+    return np.ascontiguousarray(arr)
+
+
+class _PosePositions:
+    """Stands in for the destination points in the exception messages: item i is pose i's position [x, y, z]."""
+
+    def __init__(self, poses):
+        self._poses = poses
+
+    def __getitem__(self, i):
+        return self._poses[i, :3, 3].tolist()
+
+
+def _empty_result(dtype, as_array, return_iterations, return_fk_error):
+    empty = np.zeros((0, 4), dtype=dtype)
+    empty = empty if as_array else []
+    extras = ((np.zeros(0, np.int32),) if return_iterations else ()) + \
+             ((np.zeros(0, dtype),) if return_fk_error else ())
+    return (empty,) + extras if extras else empty
 
 
 class InverseKinematics(ABC):
@@ -117,6 +149,77 @@ class InverseKinematics(ABC):
         self._engine().dls_refine_device(points, angles, out, iters, fk_err, damping, tol, max_iter)
         return out
 
+    def _raise_pose_errors(self, poses, stats):
+        if stats.first_out_of_limits >= 0:
+            raise self._limits_error(_PosePositions(poses), stats.first_out_of_limits)
+        if stats.first_fk_angle_range >= 0:
+            raise OutOfRobotReachException(_ANGLE_MSG)
+
+    def refine_pose(self, dest_poses, angles, weights=POSE_WEIGHTS, damping=POSE_DAMPING, tol=POSE_TOL,
+                    max_iter=POSE_MAX_ITER, as_array=False, return_iterations=False, return_fk_error=False):
+        """Refine joint angles onto full effector poses (position and orientation) by weighted damped least squares on
+        the GPU.  dest_poses: (n, 4, 4) homogeneous transforms, e.g. ``self.fkine.fkine_batch(theta)[0]``; rows 0-2
+        are read.  From `angles` (one row per pose, or one row for all), each row repeats
+        Delta theta = (J^T W J + damping^2 I)^-1 J^T W e over the 6 x 4 geometric Jacobian J, with e = (position error,
+        2 x the vector part of the rotation error's quaternion) and W = diag(weights), until
+        sqrt(sum w_i e_i^2) <= tol or `max_iter` steps (include/ikb200.h ikb_dls_pose_refine_* states the arithmetic).
+        The arm has four joints: a pose that no angles produce stops at max_iter, matched as the weights ask.
+
+        Dtypes, return shapes and exceptions follow `refine`: a pose whose position is outside the workspace box
+        raises OutOfRobotReachException with `ikine`'s message naming that position [x, y, z] (checked first), a seed
+        angle outside [-2pi, 2pi] the forward-kinematics one.  `return_fk_error` gives the weighted error."""
+        poses = poses_to_array(dest_poses)
+        seed = angles if isinstance(angles, np.ndarray) and angles.dtype in (np.float32, np.float64) else \
+            np.asarray(angles, dtype=np.float64)
+        if poses.shape[0] == 0:
+            return _empty_result(seed.dtype, as_array, return_iterations, return_fk_error)
+        res = self._engine().dls_pose_refine(poses, seed, weights, damping, tol, max_iter,
+                                             return_iters=return_iterations, return_error=return_fk_error)
+        out, stats = res[0], res[1]
+        self.last_stats = stats
+        self._raise_pose_errors(poses, stats)
+        out = out if as_array else out.tolist()
+        return (out,) + tuple(res[2:]) if len(res) > 2 else out
+
+    def refine_pose_device(self, poses, angles, out=None, iters=None, fk_err=None, weights=POSE_WEIGHTS,
+                           damping=POSE_DAMPING, tol=POSE_TOL, max_iter=POSE_MAX_ITER):
+        """`refine_pose` on CUDA tensors, enqueued on torch's current stream without a synchronisation: poses a
+        contiguous (n, 4, 4) tensor, angles (n, 4) or one row for all poses, float32 or float64; out, iters and fk_err
+        as for `refine_device` (out may be `angles`: in place).  Returns out.  The guards set first_out_of_limits /
+        first_fk_angle_range of the engine's statistics (``stats_fetch_torch``) instead of raising."""
+        import torch
+        if out is None:
+            out = torch.empty((poses.shape[0], 4), dtype=angles.dtype, device=angles.device)
+        self._engine().dls_pose_refine_device(poses, angles, out, iters, fk_err, weights, damping, tol, max_iter)
+        return out
+
+    def _ikine_pose(self, dest_poses, seed_on_device, weights, damping, tol, max_iter, as_array, return_iterations,
+                    return_fk_error):
+        """Upload the poses once, seed with `seed_on_device(xyz) -> (engine, float64 seeds)` on the position columns,
+        raise what `ikine` raises, refine onto the poses in place and download once."""
+        import torch
+        poses = poses_to_array(dest_poses)
+        n = poses.shape[0]
+        if n == 0:
+            return _empty_result(np.float64, as_array, return_iterations, return_fk_error)
+        eng = self._engine()
+        d_poses = torch.from_numpy(poses).to(torch.device("cuda", eng.device))
+        solver, seed = seed_on_device(d_poses[:, :3, 3].contiguous())
+        stats = solver.stats_fetch_torch()
+        self.last_stats = stats
+        self._raise_from_stats(_PosePositions(poses), stats)
+        eng.stats_reset_torch()
+        iters = torch.empty(n, dtype=torch.int32, device=seed.device) if return_iterations else None
+        err = torch.empty(n, dtype=seed.dtype, device=seed.device) if return_fk_error else None
+        eng.dls_pose_refine_device(d_poses, seed, seed, iters, err, weights, damping, tol, max_iter)
+        out = seed.cpu().numpy()
+        extras = tuple(t.cpu().numpy() for t in (iters, err) if t is not None)
+        stats = eng.stats_fetch_torch()
+        self.last_stats = stats
+        self._raise_pose_errors(poses, stats)
+        out = out if as_array else out.tolist()
+        return (out,) + extras if extras else out
+
 
 class FabrikInverseKinematics(InverseKinematics):
     """Reaching inverse kinematics using the FABRIK method (reference inverse.py:45-139)."""
@@ -153,6 +256,22 @@ class FabrikInverseKinematics(InverseKinematics):
         out = angles if as_array else angles.tolist()
         return (out,) + tuple(res[2:]) if len(res) > 2 else out
 
+    def ikine_pose(self, dest_poses, weights=POSE_WEIGHTS, damping=POSE_DAMPING, tol=POSE_TOL, max_iter=POSE_MAX_ITER,
+                   as_array=False, return_iterations=False, return_fk_error=False):
+        """Joint angles that put the effector on each (4, 4) pose: FABRIK on the pose's position column, then
+        `refine_pose` from there, all on the GPU (one upload of the poses, one download of the float64 angles).
+        Raises what `ikine` raises for those positions, then what `refine_pose` raises; returns as `refine_pose`."""
+        import torch
+
+        def seed(xyz):
+            eng = self._engine()
+            angles = torch.empty((xyz.shape[0], 4), dtype=torch.float64, device=xyz.device)
+            eng.stats_reset_torch()
+            eng.fabrik_solve_device(xyz, angles, precision=self.precision)
+            return eng, angles
+        return self._ikine_pose(dest_poses, seed, weights, damping, tol, max_iter, as_array, return_iterations,
+                                return_fk_error)
+
 
 class AnnInverseKinematics(InverseKinematics):
     """Reaching inverse kinematics using the neural network (reference inverse.py:142-155)."""
@@ -180,3 +299,20 @@ class AnnInverseKinematics(InverseKinematics):
         self._raise_from_stats(dest_points, stats)
         angles = angles if as_array else angles.tolist()
         return (angles, res[2]) if return_fk_error else angles
+
+    def ikine_pose(self, dest_poses, weights=POSE_WEIGHTS, damping=POSE_DAMPING, tol=POSE_TOL, max_iter=POSE_MAX_ITER,
+                   as_array=False, return_iterations=False, return_fk_error=False):
+        """Joint angles that put the effector on each (4, 4) pose: the network's prediction for the pose's position
+        column, widened to float64, then `refine_pose` from there, all on the GPU (one upload of the poses, one
+        download of the angles).  Raises what `ikine` raises for those positions, then what `refine_pose` raises;
+        returns as `refine_pose`."""
+        import torch
+
+        def seed(xyz):
+            eng = self.ann._ensure_uploaded()
+            pred = torch.empty((xyz.shape[0], 4), dtype=torch.float32, device=xyz.device)
+            eng.stats_reset_torch()
+            eng.ann_solve_device(xyz, pred, mode=self.ann.mode)
+            return eng, pred.double()
+        return self._ikine_pose(dest_poses, seed, weights, damping, tol, max_iter, as_array, return_iterations,
+                                return_fk_error)
