@@ -340,11 +340,10 @@ __device__ __noinline__ double fused_fk_error_f64(double t0, double t1, double t
 // Bits riding in a chain's iteration counter (the count itself is below 2^28).
 #define IKB_K_MASK 0x0fffffff
 #define IKB_CAPPED_BIT 0x40000000  // the chain stopped on max_iter, not on the tolerance
-#define IKB_UXZERO_BIT 0x20000000  // the target's x is exactly 0: C.x * D.x of inverse.py:82 is 0, never negative
 
 // Finish one solved chain: derive the effector, extract the four angles as reference inverse.py:54-112 does, write
 // the outputs, raise the per-row flags.  Everything it needs about the target travels with the parked chain (Tr, Tz,
-// theta_1 of the target's plane, the x == 0 flag): no second read of the input (round 1 re-read the row here).
+// theta_1 of the target's plane): no second read of the input (round 1 re-read the row here).
 // CONST_LINKS: the chain was iterated in fp64, so its segments have their link lengths to the last place (see below);
 // an fp32-iterated chain is only good to 1e-7 there and takes the general form with computed lengths.
 // ZERO_ITER: the reference's loop never runs (tol >= 1 or max_iter <= 0) and every chain is the seed chain -- a separate
@@ -403,8 +402,9 @@ __device__ __forceinline__ void fabrik_epilogue(const FabrikArgs &a, int idx, in
     const bool flip = r3 < 0.0;  // theta_1 = atan2(E.y, E.x) with E = r3 (ux, uy) (inverse.py:60): only the sign of r3 matters
     // t4_point_bt = PB(C, E, |CE| / 2) (inverse.py:102): (|CE|/2)/|CE| is exactly 0.5
     const double mr = fma(0.5, r3 - r1, r1), mz = fma(0.5, z3 - z1, z1);
-    // C.x * D.x < 0 (:82) with C.x = r1 ux, D.x = r2 ux: the sign of r1 r2 unless the plane has no x component
-    const bool elbow_neg = !(k_raw & IKB_UXZERO_BIT) & (r1 * r2 < 0);
+    // C.x * D.x < 0 (:82) with C.x = r1 ux, D.x = r2 ux: the sign of r1 r2.  On the plane x = 0 the reference's product
+    // is seed noise (DESIGN 1); the in-plane sign is the limit x -> 0+ of its own rule
+    const bool elbow_neg = r1 * r2 < 0;
     const bool wrist_neg = n_bd > dist2d_sq(R0, Z0, mr, mz);                // :103
     // Rare rows, classified out of line (a branch that is almost never taken):
     //  * a zero-length segment (ZeroDivisionError upstream, point.py:40) -- a length of 0, or a chain that is no longer
@@ -590,19 +590,18 @@ __device__ __forceinline__ void fabrik_warp_loop(const FabrikArgs &a, WarpQueues
             t1 = (Th1)atan2_unit_f32(uy, ux);
         else
             t1 = (Th1)atan2_unit(uy, ux);
-        const int k0 = ux == 0.0 ? IKB_UXZERO_BIT : 0;
         const bool far = valid && a.far_thr2 > 0.0 && is_far(px, py, pz, rc.seed_r[0], rc.seed_z[0], a.far_thr2);
         const bool near = valid && !far;
         const unsigned keep_n = __ballot_sync(IKB_FULL_MASK, near), keep_f = __ballot_sync(IKB_FULL_MASK, far);
         if (near) {
             const int slot = (in_head + in_cnt + __popc(keep_n & lt)) & (IKB_Q - 1);
-            q.in_ik[slot] = make_int2((int)pf_row, k0);
+            q.in_ik[slot] = make_int2((int)pf_row, 0);
             q.in_t[slot] = Real2{tr, (Real)pz};
             q.in_th1[slot] = t1;
         }
         if (far) {
             const int slot = far_cnt + __popc(keep_f & lt);
-            q.far_ik[slot] = make_int2((int)pf_row, k0);
+            q.far_ik[slot] = make_int2((int)pf_row, 0);
             q.far_t[slot] = Real2{tr, (Real)pz};
             q.far_th1[slot] = t1;
         }
@@ -667,7 +666,7 @@ __device__ __forceinline__ void fabrik_warp_loop(const FabrikArgs &a, WarpQueues
                 const int e = u * 32 + lane;
                 const int slot = (out_head + out_cnt + lane) & (IKB_OUT_Q - 1);
                 const int2 fik = q.far_ik[e];
-                q.out_ik[slot] = make_int2(fik.x, max_iter | IKB_CAPPED_BIT | fik.y);
+                q.out_ik[slot] = make_int2(fik.x, max_iter | IKB_CAPPED_BIT);
                 q.out_j1[slot] = Real2{fc[u].r1, fc[u].z1};
                 q.out_j2[slot] = Real2{fc[u].r2, fc[u].z2};
                 q.out_t[slot] = Real2{fTr[u], fTz[u]};
