@@ -318,6 +318,59 @@ int ikb_dls_pose_refine_host(ikb_engine *e, const void *poses, int pose_dtype, i
                              double damping, double tol, int32_t max_iter, int32_t *iters_out /* nullable */,
                              void *err_out /* nullable, angles_dtype */, ikb_stats *stats);
 
+/* Closed-form inverse kinematics: every solution branch of n effector poses, or of n positions at a given approach
+ * (pitch) angle, for arms with a turning base and three parallel joints.  That family is: alpha_2 = alpha_3 =
+ * alpha_4 = 0, |cos alpha_1| <= 1e-12 (treated as 0; s = sign(sin alpha_1)), a_2 > 0 and a_3 > 0; a_1, a_4 and every
+ * epsilon are free, d = (eps_2 + eps_3) + eps_4 is the lateral offset.  (Indices count joints from 1 here, as the
+ * DH table's columns: a_1 = dh[2][0].)  The reference's arm is in it.  Any other table is refused with
+ * IKB_ERR_UNSUPPORTED: the damped-least-squares entries (ikb_dls_pose_refine_*) serve it.
+ * The arithmetic is fp64 (float32 inputs are widened exactly, a float32 output is the fp64 result rounded once); every
+ * input element is read as x + 0, so -0 and +0 give the same bits.  Every angle leaving [-pi, pi] is wrapped with the
+ * exact IEEE remainder(theta, 2pi), as in ikb_dls_refine_*, so every answer is inside the FK guard and valid as a seed.
+ *   Two-link triangle, from in-plane coordinates (u, v) of the effector and phi = theta_2 + theta_3 + theta_4:
+ *     uw = u - a_4 cos phi;  vw = v - a_4 sin phi;  r = sqrt(uw^2 + vw^2)
+ *     num = ((a_2 + a_3) - r)((a_2 + a_3) + r);  den = (r - (a_2 - a_3))(r + (a_2 - a_3))
+ *     t = 2 atan2(sqrt(num > 0 ? num : 0), sqrt(den > 0 ? den : 0))   (half-angle form: exact near the folded arm)
+ *     beta = atan2(vw, uw);  g = atan2(a_3 sin t, a_2 + a_3 cos t)
+ *     elbow +: theta_3 = t,      theta_2 = beta - g
+ *     elbow -: theta_3 = 0 - t,  theta_2 = beta - (0 - g)    (identical bits to elbow + at t = 0)
+ *     theta_4 = (phi - theta_2) - theta_3, with the unwrapped theta_2.
+ *   IKB_AIK_POSE: in = n x 4 x 4 poses of in_dtype, row-major (the layout of ikb_fk_transforms_*, rows 0-2 read), with
+ *   x = column 0, z = column 2, p = column 3:
+ *     theta_1 = atan2(s z_x, -s z_y);  phi = atan2(s x_z, c_1 x_x + s_1 x_y)
+ *     u = (c_1 p_x + s_1 p_y) - a_1;  v = s (p_z - eps_1)
+ *     2 branches per row, ordered [elbow +, elbow -].  A pose that no angles produce is projected onto the arm's plane
+ *     by the same formulas: its angles are defined, and a refinement takes them on to what its weights ask for.
+ *   IKB_AIK_POSITION_PITCH: in = n x 3 targets; pitch = n_pitch values (1 or n) of in_dtype, the angle of the tool axis
+ *   x_4 above the horizontal:
+ *     rho2 = p_x^2 + p_y^2;  q = sqrt(rho2 < d^2 ? 0 : rho2 - d^2)
+ *     front: q' = q, phi = pitch;  back (reaching over the base): q' = -q, phi = pi - pitch
+ *     theta_1 = atan2(p_y, p_x) - atan2(-s d + 0, q');  u = q' - a_1;  v = s (p_z - eps_1)
+ *     4 branches per row, ordered [front +, front -, back +, back -].  With d = 0 all four give the same tool axis
+ *     x_4 = (cos(pitch) r^, s sin(pitch)).  A target on the base axis (p_x = p_y = 0, either sign) with d = 0 gets
+ *     theta_1 = 0 on the front branches and -pi on the back ones.
+ * status_out (nullable, n int32): bit b is set when branch b does not reach -- num < 0 (the arm is stretched toward
+ * the wrist, t = 0), den < 0 (folded toward it, t = pi), or rho2 < d^2 (position kind; q = 0 is used).  num = 0 counts
+ * as reached.  A row with a non-finite input element (or pitch) gets NaN angles and every bit set.
+ * Guard: a position (column 3 of a pose) outside the workspace box sets stats.first_out_of_limits (the inclusive test of
+ * ikb_check_limits_*, NaN passes); the rows are still written.  n_solved counts the rows.
+ * Refused with IKB_ERR_INVALID before the engine is looked at, each with its own message (read with
+ * ikb_last_error(NULL) when e == NULL): NULL input or angles_out (n > 0), an unknown kind or dtype, negative n, a NULL
+ * pitch for the position kind (n > 0) or a pitch for the pose kind, n_pitch not 1 or n (position kind), a buffer not
+ * aligned to its element size (pitch: in_dtype, status_out: 4 bytes), then a NULL engine; then a table outside the
+ * family with IKB_ERR_UNSUPPORTED.  Nothing is launched for a refused call or for n = 0.
+ * _device: DEVICE pointers, enqueued on `stream`, one launch; the guard accumulates in the engine's block.  _host:
+ * HOST pointers, staged through the engine's pipeline with no per-call allocation, `stats` filled (nullable).  A host
+ * chunk, one launch, holds S / 4 rows, S the rows of a staging slot. */
+#define IKB_AIK_POSE 0
+#define IKB_AIK_POSITION_PITCH 1
+int ikb_analytic_ik_device(ikb_engine *e, int kind, const void *in, int in_dtype, int64_t n, const void *pitch,
+                           int64_t n_pitch, void *angles_out /* n x B x 4 */, int angles_dtype,
+                           int32_t *status_out /* nullable */, void *stream);
+int ikb_analytic_ik_host(ikb_engine *e, int kind, const void *in, int in_dtype, int64_t n, const void *pitch,
+                         int64_t n_pitch, void *angles_out /* n x B x 4 */, int angles_dtype,
+                         int32_t *status_out /* nullable */, ikb_stats *stats);
+
 /* ---- ANN (ann.py:70-85, inverse.py:142-155)-------------------------------------------------- */
 /* replaces ANN.load_model (ann.py:78-85): upload the Keras Sequential's Dense kernels/biases and the
  * two StandardScalers.  dims[n_layers+1] = {3, 500, ..., 500, 4}; weights[l] is row-major

@@ -17,6 +17,7 @@ IKB_MLP_FP32_SIMT, IKB_MLP_FP16X3_TC, IKB_MLP_FP16X3_TS = 0, 1, 2
 IKB_CHAIN_MAX_POINTS = 256
 IKB_FK_MATRICES, IKB_FK_JOINTS = 0, 1
 IKB_JAC_GEOMETRIC, IKB_JAC_POSITION = 0, 1
+IKB_AIK_POSE, IKB_AIK_POSITION_PITCH = 0, 1
 
 # every symbol include/ikb200.h declares (tests check that the built library exports them all)
 EXPORTED_SYMBOLS = [
@@ -27,7 +28,7 @@ EXPORTED_SYMBOLS = [
     "ikb_fabrik_chain_device", "ikb_fabrik_chain_host",
     "ikb_fk_device", "ikb_fk_host", "ikb_fk_chain_host", "ikb_fk_transforms_device", "ikb_fk_transforms_host",
     "ikb_jacobian_device", "ikb_jacobian_host", "ikb_dls_refine_device", "ikb_dls_refine_host",
-    "ikb_dls_pose_refine_device", "ikb_dls_pose_refine_host",
+    "ikb_dls_pose_refine_device", "ikb_dls_pose_refine_host", "ikb_analytic_ik_device", "ikb_analytic_ik_host",
     "ikb_mlp_load", "ikb_ann_solve_device", "ikb_ann_solve_host",
     "ikb_generate_device", "ikb_microbench_fma", "ikb_launch_count",
     "ikb_host_alloc", "ikb_host_free", "ikb_host_register", "ikb_host_unregister",
@@ -104,6 +105,8 @@ def load():
                                              vp, vp, vp]),
         "ikb_dls_pose_refine_host": (i32, [engine, vp, i32, i64, vp, i64, vp, i32, dbl_p, dbl, dbl, ctypes.c_int32, vp,
                                            vp, stats_p]),
+        "ikb_analytic_ik_device": (i32, [engine, i32, vp, i32, i64, vp, i64, vp, i32, vp, vp]),
+        "ikb_analytic_ik_host": (i32, [engine, i32, vp, i32, i64, vp, i64, vp, i32, vp, stats_p]),
         "ikb_mlp_load": (i32, [engine, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
                                ctypes.POINTER(vp), ctypes.POINTER(vp), vp, vp, vp, vp]),
         "ikb_ann_solve_device": (i32, [engine, vp, i32, i64, vp, vp, i32, i32, vp]),

@@ -43,6 +43,10 @@ cudaError_t ikb_launch_dls_pose_refine(const void *poses, int pose_f64, const vo
                                        long long index_base, const double weights[6], double damping, double tol,
                                        int max_iter, IkbDeviceStats *stats, unsigned long long *work_counter,
                                        const IkbRobot &rc, int num_sms, cudaStream_t stream);
+cudaError_t ikb_launch_analytic_ik(int kind, const void *in, int in_f64, long long n, long long index_base,
+                                   const void *pitch, int per_row_pitch, void *angles_out, int angles_f64,
+                                   int *status, IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
+                                   cudaStream_t stream);
 cudaError_t ikb_launch_check_limits(const void *xyz, int xyz_f64, long long n, long long index_base,
                                     IkbDeviceStats *stats, const IkbRobot &rc, int num_sms,
                                     cudaStream_t stream);
@@ -98,6 +102,7 @@ struct ikb_engine {
     IkbMlp mlp;
     std::string err;
     long long launches = 0;
+    bool analytic_family = false;  // the DH table has the closed-form inverse kinematics of ikb_analytic_ik_*
 };
 
 namespace {
@@ -335,6 +340,8 @@ int ikb_engine_create(const ikb_config *cfg, ikb_engine **out)
         }
         if (status)
             rc.planar = 0;
+        e->analytic_family = rc.fk_planar_tail && std::fabs(rc.cos_alpha[0]) <= 1e-12 && rc.a[1] > 0.0 &&
+                             rc.a[2] > 0.0;
         rc.seed_ab = std::sqrt(rc.seed_r[0] * rc.seed_r[0] + rc.seed_z[0] * rc.seed_z[0]);
         rc.seed_ab2 = rc.seed_ab * rc.seed_ab;
         rc.half_inv_ab = 0.5 / rc.seed_ab;
@@ -980,6 +987,107 @@ int ikb_dls_pose_refine_host(ikb_engine *e, const void *poses, int pose_dtype, i
             IKB_CUDA(e, cudaMemcpyAsync(iters_out + lo, s.d_aux, m * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
         if (err_out)
             IKB_CUDA(e, cudaMemcpyAsync((char *)err_out + lo * e_row, d_err, m * e_row, cudaMemcpyDeviceToHost, s.stream));
+    }
+    return host_end(e, stats);
+}
+
+// ---- closed-form inverse kinematics ---------------------------------------------------------------------------------
+// what is wrong with the arguments, or nullptr; the engine is checked last, the DH family after it
+static const char *analytic_bad_args(const ikb_engine *e, int kind, const void *in, int in_dtype, int64_t n,
+                                     const void *pitch, int64_t n_pitch, const void *angles_out, int angles_dtype,
+                                     const int32_t *status_out)
+{
+    if (n > 0 && !in)
+        return "NULL input";
+    if (n > 0 && !angles_out)
+        return "NULL angles_out";
+    if (kind != IKB_AIK_POSE && kind != IKB_AIK_POSITION_PITCH)
+        return "unknown kind";
+    if (bad_dtype(in_dtype) || bad_dtype(angles_dtype))
+        return "unknown dtype";
+    if (n < 0)
+        return "negative n";
+    if (kind == IKB_AIK_POSITION_PITCH && n > 0 && !pitch)
+        return "NULL pitch: the position kind needs one pitch or one per row";
+    if (kind == IKB_AIK_POSE && pitch)
+        return "pitch given for the pose kind, which takes none";
+    if (kind == IKB_AIK_POSITION_PITCH && n_pitch != 1 && n_pitch != n)
+        return "n_pitch must be 1 or n";
+    const uintptr_t i_align = esize(in_dtype) - 1;
+    if ((((uintptr_t)in | (uintptr_t)pitch) & i_align) || ((uintptr_t)angles_out & (esize(angles_dtype) - 1)) ||
+        ((uintptr_t)status_out & 3))
+        return "buffers must be aligned to their element size";
+    if (!e)
+        return "NULL engine";
+    return nullptr;
+}
+
+static int analytic_refusal(ikb_engine *e, const char *name, int kind, const void *in, int in_dtype, int64_t n,
+                            const void *pitch, int64_t n_pitch, const void *angles_out, int angles_dtype,
+                            const int32_t *status_out)
+{
+    if (const char *why = analytic_bad_args(e, kind, in, in_dtype, n, pitch, n_pitch, angles_out, angles_dtype,
+                                            status_out))
+        return fail(e, IKB_ERR_INVALID, std::string(name) + ": " + why);
+    if (!e->analytic_family)
+        return fail(e, IKB_ERR_UNSUPPORTED,
+                    std::string(name) + ": the DH table is outside the closed form's family (alpha_2 = alpha_3 = "
+                    "alpha_4 = 0, |cos alpha_1| <= 1e-12, a_2 > 0, a_3 > 0); use ikine_pose / refine_pose for it");
+    return IKB_OK;
+}
+
+int ikb_analytic_ik_device(ikb_engine *e, int kind, const void *in, int in_dtype, int64_t n, const void *pitch,
+                           int64_t n_pitch, void *angles_out, int angles_dtype, int32_t *status_out, void *stream)
+{
+    if (int rc = analytic_refusal(e, "ikb_analytic_ik_device", kind, in, in_dtype, n, pitch, n_pitch, angles_out,
+                                  angles_dtype, status_out))
+        return rc;
+    if (n == 0)
+        return IKB_OK;
+    IKB_CUDA(e, cudaSetDevice(e->device));
+    IKB_CUDA(e, ikb_launch_analytic_ik(kind, in, in_dtype == IKB_F64, n, 0, pitch, n_pitch != 1, angles_out,
+                                       angles_dtype == IKB_F64, status_out, e->d_stats, e->rc, e->num_sms,
+                                       (cudaStream_t)stream));
+    e->launches++;
+    return IKB_OK;
+}
+
+// Chunks of the host pipeline, S / 4 rows each (S the rows of a slot): poses (128 B per fp64 row) or positions in
+// d_in, per-row pitches in d_in2 (a single pitch is copied to d_in2 of every slot once), angles (up to 128 B per fp64
+// row) in d_out, status in d_aux.
+int ikb_analytic_ik_host(ikb_engine *e, int kind, const void *in, int in_dtype, int64_t n, const void *pitch,
+                         int64_t n_pitch, void *angles_out, int angles_dtype, int32_t *status_out, ikb_stats *stats)
+{
+    if (int rc = analytic_refusal(e, "ikb_analytic_ik_host", kind, in, in_dtype, n, pitch, n_pitch, angles_out,
+                                  angles_dtype, status_out))
+        return rc;
+    int rc = host_begin(e, n);
+    if (rc)
+        return rc;
+    const bool pose = kind == IKB_AIK_POSE, per_row_pitch = !pose && n_pitch != 1;
+    const size_t i_row = (pose ? 16 : 3) * esize(in_dtype), p_row = esize(in_dtype);
+    const size_t a_row = (pose ? 2 : 4) * 4 * esize(angles_dtype);
+    const long long m_max = e->slot_rows / 4;
+    if (n > 0 && !pose && !per_row_pitch)
+        for (int i = 0; i < kSlots; ++i)
+            IKB_CUDA(e, cudaMemcpyAsync(e->slots[i].d_in2, pitch, p_row, cudaMemcpyHostToDevice, e->slots[i].stream));
+    int it = 0;
+    for (long long lo = 0, m = 0; lo < n; lo += m, ++it) {
+        Slot &s = e->slots[it % kSlots];
+        m = std::min(m_max, n - lo);
+        IKB_CUDA(e, cudaMemcpyAsync(s.d_in, (const char *)in + lo * i_row, m * i_row, cudaMemcpyHostToDevice, s.stream));
+        if (per_row_pitch)
+            IKB_CUDA(e, cudaMemcpyAsync(s.d_in2, (const char *)pitch + lo * p_row, m * p_row, cudaMemcpyHostToDevice,
+                                        s.stream));
+        IKB_CUDA(e, ikb_launch_analytic_ik(kind, s.d_in, in_dtype == IKB_F64, m, lo, pose ? nullptr : s.d_in2,
+                                           per_row_pitch, s.d_out, angles_dtype == IKB_F64,
+                                           status_out ? s.d_aux : nullptr, e->d_stats, e->rc, e->num_sms, s.stream));
+        e->launches++;
+        IKB_CUDA(e, cudaMemcpyAsync((char *)angles_out + lo * a_row, s.d_out, m * a_row, cudaMemcpyDeviceToHost,
+                                    s.stream));
+        if (status_out)
+            IKB_CUDA(e, cudaMemcpyAsync(status_out + lo, s.d_aux, m * sizeof(int32_t), cudaMemcpyDeviceToHost,
+                                        s.stream));
     }
     return host_end(e, stats);
 }

@@ -400,6 +400,46 @@ class IkEngine:
             raise ValueError(f"poses must have shape (n, 4, 4), got {poses.shape}")
         return (poses,) + IkEngine._seed_args(poses.shape[0], seed, out)
 
+    def analytic_ik(self, x, pitch=None, out_dtype=np.float64):
+        """Every closed-form inverse-kinematics branch (include/ikb200.h ikb_analytic_ik_*) for an arm with a turning
+        base and three parallel joints: x is (n, 4, 4) poses (pitch None; 2 branches [theta3 >= 0, theta3 <= 0]) or
+        (n, 3) positions with `pitch`, the tool axis' angle above the horizontal, one value or n (4 branches [front +,
+        front -, back +, back -]), float32 or float64.  Returns (angles (n, B, 4) of out_dtype, status int32 (n,): bit b
+        set when branch b does not reach, stats); stats.first_out_of_limits >= 0 marks the lowest position outside the
+        workspace box.  A DH table outside the family raises RuntimeError."""
+        x, kind, pitch, branches = self._analytic_args(x, pitch)
+        n = x.shape[0]
+        if np.dtype(out_dtype) not in (np.float32, np.float64):
+            raise TypeError(f"out_dtype must be float32 or float64, got {np.dtype(out_dtype)}")
+        out = np.empty((n, branches, 4), dtype=out_dtype)
+        status = np.empty(n, dtype=np.int32)
+        s = _native.IkbStats()
+        self._check(self._lib.ikb_analytic_ik_host(
+            self._handle, kind, x.ctypes.data, _np_dtype_code(x), n, pitch.ctypes.data if pitch is not None else None,
+            pitch.shape[0] if pitch is not None else 0, out.ctypes.data, _np_dtype_code(out), status.ctypes.data,
+            ctypes.byref(s)), "ikb_analytic_ik_host")
+        return out, status, IkStats.from_c(s)
+
+    @staticmethod
+    def _analytic_args(x, pitch):
+        """The checks of `analytic_ik` that need no device -> (x contiguous, kind, pitch in x's dtype or None,
+        branches per row)."""
+        x = np.ascontiguousarray(x)
+        if x.dtype not in (np.float32, np.float64):
+            x = x.astype(np.float64)
+        if x.ndim == 3 and x.shape[1:] == (4, 4):
+            if pitch is not None:
+                raise ValueError("poses take no pitch: the pose's tool axis fixes it")
+            return x, _native.IKB_AIK_POSE, None, 2
+        if x.ndim != 2 or x.shape[1] != 3:
+            raise ValueError(f"x must be (n, 4, 4) poses or (n, 3) positions, got shape {x.shape}")
+        if pitch is None:
+            raise ValueError("positions need a pitch (one value, or one per row)")
+        pitch = np.ascontiguousarray(pitch, dtype=x.dtype).reshape(-1)
+        if pitch.shape[0] not in (1, x.shape[0]):
+            raise ValueError(f"pitch must have 1 or {x.shape[0]} values, got {pitch.shape[0]}")
+        return x, _native.IKB_AIK_POSITION_PITCH, pitch, 4
+
     def mlp_load(self, weights, biases, mean_x, scale_x, mean_y, scale_y):
         """reference ann.py:78-85: upload Keras Dense kernels (in, out) + biases and both scalers."""
         ws = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
@@ -679,6 +719,48 @@ class IkEngine:
             out.data_ptr(), _torch_dtype_code(out), w, damping, tol, max_iter,
             iters.data_ptr() if iters is not None else None, err.data_ptr() if err is not None else None,
             _torch_stream_ptr(self.device)), "ikb_dls_pose_refine_device")
+
+    def analytic_ik_device(self, x, pitch, out, status=None):
+        """analytic_ik on CUDA tensors of this engine's device, enqueued on torch's current stream (no
+        synchronisation): x a contiguous (n, 4, 4) pose tensor (pitch None) or (n, 3) positions with pitch, a
+        contiguous tensor of x's dtype with 1 or n elements; out (n, B, 4) float32 or float64 with B = 2 for poses and 4
+        for positions; status int32 (n,) or None.  The box guard accumulates in the engine's statistics
+        (stats_fetch_torch)."""
+        if not _is_torch_tensor(x) or not x.is_cuda:
+            raise TypeError("x must be a CUDA torch tensor")
+        if x.device.index != self.device:
+            raise ValueError(f"x lives on cuda:{x.device.index}, the engine on cuda:{self.device}")
+        code = _torch_dtype_code(x)
+        if x.dim() == 3 and tuple(x.shape[1:]) == (4, 4):
+            kind, branches = _native.IKB_AIK_POSE, 2
+            if pitch is not None:
+                raise ValueError("poses take no pitch: the pose's tool axis fixes it")
+        elif x.dim() == 2 and x.shape[1] == 3:
+            kind, branches = _native.IKB_AIK_POSITION_PITCH, 4
+            if pitch is None:
+                raise ValueError("positions need a pitch (one value, or one per row)")
+        else:
+            raise ValueError(f"x must be (n, 4, 4) poses or (n, 3) positions, got shape {tuple(x.shape)}")
+        if not x.is_contiguous():
+            raise ValueError("x must be contiguous")
+        n = x.shape[0]
+        if pitch is not None:
+            self._dev_vec(pitch, pitch.numel() if _is_torch_tensor(pitch) else -1, str(x.dtype), "pitch")
+            if pitch.numel() not in (1, n):
+                raise ValueError(f"pitch must have 1 or {n} elements, got {pitch.numel()}")
+        self._dev_vec(out, out.numel() if _is_torch_tensor(out) else -1, str(out.dtype), "out")
+        out_code = _torch_dtype_code(out)
+        if tuple(out.shape) != (n, branches, 4):
+            raise ValueError(f"out must have shape {(n, branches, 4)}, got {tuple(out.shape)}")
+        if status is not None:
+            self._dev_vec(status, n, "torch.int32", "status")
+        if n == 0:  # nothing to do, and an empty tensor's data_ptr() may be NULL
+            return
+        self._check(self._lib.ikb_analytic_ik_device(
+            self._handle, kind, x.data_ptr(), code, n, pitch.data_ptr() if pitch is not None else None,
+            pitch.numel() if pitch is not None else 0, out.data_ptr(), out_code,
+            status.data_ptr() if status is not None else None, _torch_stream_ptr(self.device)),
+            "ikb_analytic_ik_device")
 
     def check_limits_device(self, xyz):
         xyz = self._dev_rows(xyz, 3, "points")

@@ -195,8 +195,8 @@ class InverseKinematics(ABC):
 
     def _ikine_pose(self, dest_poses, seed_on_device, weights, damping, tol, max_iter, as_array, return_iterations,
                     return_fk_error):
-        """Upload the poses once, seed with `seed_on_device(xyz) -> (engine, float64 seeds)` on the position columns,
-        raise what `ikine` raises, refine onto the poses in place and download once."""
+        """Upload the poses once, seed with `seed_on_device(poses) -> (engine, float64 seeds)` from the device poses
+        (n, 4, 4), raise what `ikine` raises, refine onto the poses in place and download once."""
         import torch
         poses = poses_to_array(dest_poses)
         n = poses.shape[0]
@@ -204,7 +204,7 @@ class InverseKinematics(ABC):
             return _empty_result(np.float64, as_array, return_iterations, return_fk_error)
         eng = self._engine()
         d_poses = torch.from_numpy(poses).to(torch.device("cuda", eng.device))
-        solver, seed = seed_on_device(d_poses[:, :3, 3].contiguous())
+        solver, seed = seed_on_device(d_poses)
         stats = solver.stats_fetch_torch()
         self.last_stats = stats
         self._raise_from_stats(_PosePositions(poses), stats)
@@ -263,8 +263,9 @@ class FabrikInverseKinematics(InverseKinematics):
         Raises what `ikine` raises for those positions, then what `refine_pose` raises; returns as `refine_pose`."""
         import torch
 
-        def seed(xyz):
+        def seed(poses):
             eng = self._engine()
+            xyz = poses[:, :3, 3].contiguous()
             angles = torch.empty((xyz.shape[0], 4), dtype=torch.float64, device=xyz.device)
             eng.stats_reset_torch()
             eng.fabrik_solve_device(xyz, angles, precision=self.precision)
@@ -308,11 +309,119 @@ class AnnInverseKinematics(InverseKinematics):
         returns as `refine_pose`."""
         import torch
 
-        def seed(xyz):
+        def seed(poses):
             eng = self.ann._ensure_uploaded()
+            xyz = poses[:, :3, 3].contiguous()
             pred = torch.empty((xyz.shape[0], 4), dtype=torch.float32, device=xyz.device)
             eng.stats_reset_torch()
             eng.ann_solve_device(xyz, pred, mode=self.ann.mode)
             return eng, pred.double()
         return self._ikine_pose(dest_poses, seed, weights, damping, tol, max_iter, as_array, return_iterations,
                                 return_fk_error)
+
+
+_BASES = {"front": 0, "back": 2}
+_ELBOWS = {1: 0, -1: 1}
+
+
+def _branch(elbow, base="front"):
+    """The branch index of ikb_analytic_ik_*: elbow 1 (theta3 >= 0) or -1 (theta3 <= 0), base 'front' (reaching
+    toward the target) or 'back' (over the base)."""
+    if elbow not in _ELBOWS:
+        raise ValueError(f"elbow must be 1 (theta3 >= 0) or -1 (theta3 <= 0), got {elbow!r}")
+    if base not in _BASES:
+        raise ValueError(f"base must be 'front' or 'back', got {base!r}")
+    return _BASES[base] + _ELBOWS[elbow]
+
+
+class AnalyticInverseKinematics(InverseKinematics):
+    """Closed-form inverse kinematics for arms with a turning base and three parallel joints (alpha_2..4 = 0,
+    |cos alpha_1| <= 1e-12, a_2, a_3 > 0; the reference's arm is one): every solution branch, computed exactly
+    rather than searched for.  A pose has two (one per elbow sign); a position with the tool axis' pitch above the
+    horizontal (e.g. -pi/2: pointing down) has four: reaching toward the target or back over the base, times the elbow
+    signs.  include/ikb200.h ikb_analytic_ik_* states the arithmetic.  Other DH tables raise RuntimeError on the
+    first solve; `ikine_pose` of the other solvers serves them."""
+
+    def __init__(self, dh_matrix, joints_distances, workspace_limits, device=None):
+        super().__init__(dh_matrix, joints_distances, workspace_limits, device=device)
+        self.last_stats = None
+
+    def _solve(self, x, pitch, dest):
+        angles, status, stats = self._engine().analytic_ik(x, pitch)
+        self.last_stats = stats
+        if stats.first_out_of_limits >= 0:
+            raise self._limits_error(dest, stats.first_out_of_limits)
+        return angles, status
+
+    def ikine_branches(self, dest_points, pitch):
+        """All four branches for (n, 3) points at `pitch` (one value or one per point): (angles (n, 4, 4) float64,
+        ordered [front +, front -, back +, back -], status int32 (n,), bit b set when branch b does not reach -- the
+        arm then points stretched or folded toward the wrist).  A point outside the workspace box raises
+        OutOfRobotReachException with `ikine`'s message."""
+        arr = points_to_array(dest_points)
+        if arr.shape[0] == 0:
+            return np.zeros((0, 4, 4)), np.zeros(0, np.int32)
+        return self._solve(arr, np.asarray(pitch, dtype=np.float64), dest_points)
+
+    def ikine(self, dest_points, pitch, elbow=1, base="front", as_array=False, return_status=False):
+        """Joint angles [theta1..theta4] for every destination point with the tool axis at `pitch` above the
+        horizontal: the branch with `elbow` 1 (theta3 >= 0) or -1 (theta3 <= 0), reaching toward the point
+        (base='front') or back over the base (base='back').  Returns a list of rows, or an (n, 4) float64 array with
+        `as_array`; `return_status` appends an int32 array, 1 where that branch does not reach (the angles then point
+        the arm toward the point, stretched or folded).  Raises what `ikine_branches` raises."""
+        b = _branch(elbow, base)
+        angles, status = self.ikine_branches(dest_points, pitch)
+        out = np.ascontiguousarray(angles[:, b])
+        out = out if as_array else out.tolist()
+        return (out, (status >> b) & 1) if return_status else out
+
+    def ikine_device(self, points, pitch, out=None, status=None):
+        """All four branches on CUDA tensors, enqueued on torch's current stream without a synchronisation: points
+        (n, 3), pitch a tensor of the points' dtype with 1 or n elements, or a number; out (n, 4, 4) float32 or float64
+        is allocated (float64) when None; status int32 (n,) or None.  Returns out.  The box guard sets
+        first_out_of_limits of the engine's statistics (``stats_fetch_torch``) instead of raising."""
+        import torch
+        if not torch.is_tensor(pitch):
+            pitch = torch.tensor([float(pitch)], dtype=points.dtype, device=points.device)
+        if out is None:
+            out = torch.empty((points.shape[0], 4, 4), dtype=torch.float64, device=points.device)
+        self._engine().analytic_ik_device(points, pitch, out, status)
+        return out
+
+    def ikine_pose_branches(self, dest_poses):
+        """Both branches for (n, 4, 4) poses: (angles (n, 2, 4) float64, ordered [theta3 >= 0, theta3 <= 0], status
+        int32 (n,), bit b set when branch b does not reach).  theta1 comes from the pose's joint axis, so it is always
+        on the side the pose reaches.  A pose that no angles produce is projected onto the arm's plane.  A position
+        outside the workspace box raises OutOfRobotReachException with `ikine`'s message naming it."""
+        poses = poses_to_array(dest_poses)
+        if poses.shape[0] == 0:
+            return np.zeros((0, 2, 4)), np.zeros(0, np.int32)
+        return self._solve(poses, None, _PosePositions(poses))
+
+    def ikine_pose_device(self, poses, out=None, status=None):
+        """Both branches of (n, 4, 4) CUDA poses, enqueued on torch's current stream without a synchronisation; out
+        (n, 2, 4) float32 or float64 is allocated (float64) when None; status int32 (n,) or None.  Returns out.  The
+        box guard sets first_out_of_limits of the engine's statistics (``stats_fetch_torch``) instead of raising."""
+        import torch
+        if out is None:
+            out = torch.empty((poses.shape[0], 2, 4), dtype=torch.float64, device=poses.device)
+        self._engine().analytic_ik_device(poses, None, out, status)
+        return out
+
+    def ikine_pose(self, dest_poses, elbow=1, refine=True, weights=POSE_WEIGHTS, damping=POSE_DAMPING, tol=POSE_TOL,
+                   max_iter=POSE_MAX_ITER, as_array=False, return_iterations=False, return_fk_error=False):
+        """Joint angles that put the effector on each (4, 4) pose: the closed-form branch of `elbow` (1: theta3 >= 0,
+        -1: theta3 <= 0), then `refine_pose` from there in place (refine=False: no steps, the closed form with its
+        weighted error), all on the GPU (one upload of the poses, one download of the float64 angles).  Returns and
+        raises as the other solvers' `ikine_pose`."""
+        import torch
+        b = _branch(elbow)
+
+        def seed(poses):
+            eng = self._engine()
+            branches = torch.empty((poses.shape[0], 2, 4), dtype=torch.float64, device=poses.device)
+            eng.stats_reset_torch()
+            eng.analytic_ik_device(poses, None, branches)
+            return eng, branches[:, b].contiguous()
+        return self._ikine_pose(dest_poses, seed, weights, damping, tol, max_iter if refine else 0, as_array,
+                                return_iterations, return_fk_error)
